@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the rollout-and-update hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one training epoch of the reference's loop (pipelines/pipeline.py:163-164):
 `buffer.sample()` (policy-in-the-loop rollout of every env for the full horizon) followed by
@@ -26,6 +26,14 @@ slot-steps/s and the valid fraction are printed beside it.
 Extra keys: K1/K2/K3 times, rooflines, GRPO updates/s, `other_configs` (BASELINE configs[1], Pendulum),
 `rank_weights_identical` (all ranks hold bit-identical weights after the timed epochs), the CPU baseline
 measured on this box, clocks under load.
+
+`--dump-outputs DIR` writes what the last timed epoch of the device-resident arm computed, as rank 0 holds it,
+to DIR/<name>.npy (float32 / float64, under 64 MB): the policy parameters after the update, the mean return,
+the episode length of every env and the full trajectories of a fixed, seeded sample of envs.  Initial states,
+noise seeds and start weights are seeded, so two builds run with the same arguments can be compared array by
+array.  With several GPUs everything but the weights (identical on every rank) covers rank 0's envs only: the mean
+return, the valid env-step count, the lengths and the sample are those of its shard, so compare dumps taken with
+the same --gpus.
 """
 import argparse
 import json
@@ -261,8 +269,36 @@ class Dist:
             self.dist.destroy_process_group()
 
 
-def measure(D, w, steps, warmup, full, args):
-    """One workload on this rank's GPU.  full=False: device-resident arm only (the `other_configs` lines)."""
+DUMP_SAMPLE_ENVS = 256      # trajectories of 256 envs: at most 27 MB (QuadPole, T = 1000); lengths of 1M envs: 8 MB
+
+
+def dump_outputs(path, policy, rollout, mean_return, valid_env_steps):
+    """What a caller of the timed epoch holds afterwards: the updated weights (`policy.flat_parameters()`) and,
+    unless the epoch was streamed, the buffer's rollout (`Rollout_Buffer.device_rollout`)."""
+    import torch
+    arrays = {"policy_params": policy.flat_parameters(), "mean_return": mean_return,
+              "valid_env_steps": valid_env_steps}
+    if rollout is not None:
+        r = rollout
+        idx = np.sort(np.random.default_rng(0).choice(r.N, size=min(r.N, DUMP_SAMPLE_ENVS), replace=False))
+        sel = torch.from_numpy(idx).to(r.len.device)
+        arrays.update({
+            "lengths": r.len, "sample_env_index": idx,
+            "sample_observations": r.obs.index_select(2, sel).permute(2, 0, 1),     # [envs, T, O]
+            "sample_actions": r.act.index_select(2, sel).permute(2, 0, 1),          # [envs, T, A]
+            "sample_rewards": r.rew.index_select(1, sel).t(),                       # [envs, T]
+            "sample_log_probs": r.logp.index_select(1, sel).t(),                    # [envs, T]
+        })
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a.detach().cpu() if torch.is_tensor(a) else a)
+        # integers (lengths, counts, indices) as float64: exact, where float32 is not above 2^24
+        np.save(os.path.join(path, name + ".npy"), a.astype(np.float32 if a.dtype == np.float32 else np.float64))
+
+
+def measure(D, w, steps, warmup, full, args, dump=None):
+    """One workload on this rank's GPU.  full=False: device-resident arm only (the `other_configs` lines).
+    dump: directory for dump_outputs() of the last timed device-resident epoch."""
     import torch
     import trajopt_grpo_b200 as tg
     from trajopt_grpo_b200 import engine
@@ -314,6 +350,7 @@ def measure(D, w, steps, warmup, full, args):
     inits = [host_init().to(dev) for _ in range(total)]
     phase = {"rollout": [], "update": []}
     lens_sum = torch.zeros((), dtype=torch.int64, device=dev)
+    last_valid = {}
 
     def one_step_device(i, timed):
         e = [ev() for _ in range(3)]
@@ -321,13 +358,14 @@ def measure(D, w, steps, warmup, full, args):
         if chunked:
             n_valid = algo.learn_streamed(mgr, init_state=inits[i], chunk_groups=w["chunk_groups"])
             e[1].record(); e[2].record()
-            lens_sum.add_(n_valid)
         else:
             buf.sample(init_state=inits[i], sync_metrics=False)
             e[1].record()
             algo.learn(buf)
             e[2].record()
-            lens_sum.add_(buf.device_rollout.len.sum())
+            n_valid = buf.device_rollout.len.sum()
+        lens_sum.add_(n_valid)
+        last_valid["n"] = n_valid
         if timed:
             phase["rollout"].append((e[0], e[1]))
             phase["update"].append((e[1], e[2]))
@@ -353,6 +391,10 @@ def measure(D, w, steps, warmup, full, args):
     value = valid_steps / (ms_total * 1e-3)
     roll_ms = float(np.mean([a.elapsed_time(b) for a, b in phase["rollout"]]))
     upd_ms = float(np.mean([a.elapsed_time(b) for a, b in phase["update"]]))
+    if dump and rank == 0:
+        # before the per-kernel timing below: with reuse_buffers its rollouts overwrite the trajectory buffers
+        dump_outputs(dump, policy, None if chunked else buf.device_rollout,
+                     algo.last_mean_return if chunked else buf.avg_reward[-1], last_valid["n"])
     valid_per_step_rank = valid_rank / steps
     slots_per_step = float(N * T)
 
@@ -537,7 +579,7 @@ def run_ours(args, w):
         w["desc"] = (f"3D QuadPole GRPO sweep point: {w['G'] * w['E']:,} envs per GPU x 1000 steps in "
                      f"{-(-w['G'] // w['chunk_groups'])} streamed chunks, group 64, MLP 256x256")
     full = not args.device_only
-    out, kern, e2e = measure(D, w, args.steps, args.warmup, full, args)
+    out, kern, e2e = measure(D, w, args.steps, args.warmup, full, args, dump=args.dump_outputs)
     peaks = {}
     try:
         peaks = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))
@@ -616,8 +658,13 @@ def main():
     ap.add_argument("--sweep-envs-per-gpu", type=int, default=0, help="quadpole_sweep: envs per GPU (multiple of 64)")
     ap.add_argument("--precision", default="f32", choices=["f32", "f64"],
                     help="env-state arithmetic of the rollout kernel: f32 (throughput mode, default) or f64 (the reference's)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed epoch to DIR/<name>.npy (see the module docstring); "
+                         "with several GPUs all but the weights cover rank 0's envs only")
     args = ap.parse_args()
     w = WORKLOADS[args.workload]
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         run_reference(args, w)
     else:
