@@ -1,8 +1,8 @@
-// Context, error reporting, MLP staging layout and the weight pack kernel.
+// Context, error reporting, Gaussian constants, the staging layouts and their weight pack kernels.
+#include <math.h>
 #include <stdarg.h>
-#include <stdlib.h>
 
-#include "tg_common.cuh"
+#include "tg_umma.cuh"
 
 static thread_local char g_err[512] = "";
 
@@ -42,10 +42,6 @@ extern "C" int tg_ctx_create(int device, tg_ctx **out) {
     c->packed_tc = nullptr;
     c->packed_tc_cap = 0;
     c->math_mode = TG_MATH_AUTO;
-    {
-        const char *e = getenv("TG_ROLLOUT_TC2");     // diagnostics only (A/B of the two width-64 rollout kernels)
-        c->rollout_tc2 = (e && e[0] == '1') ? 1 : 0;
-    }
     c->scratch = nullptr;
     c->scratch_cap = 0;
     c->order_buf = nullptr;
@@ -145,32 +141,20 @@ __global__ void pack_tc_kernel(tg_tc_layout lay, const float *__restrict__ param
                 if (i >= lay.bias[l] && i < lay.bias[l] + TCW) v = Wf[(int64_t)TCW * TCW + (i - lay.bias[l])];
                 const bool hi = i >= lay.whi[l] && i < lay.whi[l] + TCW * TCW;
                 const bool lo = i >= lay.wlo[l] && i < lay.wlo[l] + TCW * TCW;
-                if (hi || lo) {
-                    // invert the core-matrix layout of tg_umma.cuh: byte offset -> (row n, col k)
-                    const uint32_t b = (uint32_t)(i - (hi ? lay.whi[l] : lay.wlo[l])) * 4u;
-                    const uint32_t group = (TCW / 4) * 128u;
-                    const uint32_t r = b % group;
-                    const int n = (int)(b / group) * 8 + (int)((r % 128u) >> 4);
-                    const int k = (int)(r / 128u) * 4 + (int)((r & 15u) >> 2);
+                if (hi || lo) {                             // K-major core-matrix layout, rows n, cols k
+                    int n, k;
+                    core_invert(TCW, i - (hi ? lay.whi[l] : lay.wlo[l]), &n, &k);
                     const float w = Wf[(int64_t)n * TCW + k];
-                    uint32_t hb;
-                    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(hb) : "f"(w));
-                    const float whi = __uint_as_float(hb & 0xffffe000u);
+                    const float whi = tf32_hi(w);
                     v = hi ? whi : (w - whi);
                 }
                 const bool bhi = lay.wbhi[l] >= 0 && i >= lay.wbhi[l] && i < lay.wbhi[l] + TCW * TCW;
                 const bool blo = lay.wblo[l] >= 0 && i >= lay.wblo[l] && i < lay.wblo[l] + TCW * TCW;
-                if (bhi || blo) {
-                    // invert mn32_offset (tg_umma.cuh) of the stored [R = TCW rows n][cols k] matrix
-                    const uint32_t b = (uint32_t)(i - (bhi ? lay.wbhi[l] : lay.wblo[l])) * 4u;
-                    const uint32_t blk = b / (TCW * 128u), r = b % (TCW * 128u);
-                    const int n = (int)(r / 128u);
-                    const int chunk = (int)((r % 128u) >> 5) ^ (n & 3);
-                    const int k = (int)blk * 32 + chunk * 8 + (int)((r & 31u) >> 2);
+                if (bhi || blo) {                           // MN-major SW128_32B layout, rows n, cols k
+                    int n, k;
+                    mn32_invert(TCW, i - (bhi ? lay.wbhi[l] : lay.wblo[l]), &n, &k);
                     const float w = Wf[(int64_t)n * TCW + k];
-                    uint32_t hb;
-                    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(hb) : "f"(w));
-                    const float whi = __uint_as_float(hb & 0xffffe000u);
+                    const float whi = tf32_hi(w);
                     v = bhi ? whi : (w - whi);
                 }
             }
@@ -180,18 +164,8 @@ __global__ void pack_tc_kernel(tg_tc_layout lay, const float *__restrict__ param
 }
 
 int tg_pack_weights_tc(tg_ctx *ctx, const tg_tc_layout &lay, const float *params, cudaStream_t st) {
-    const size_t bytes = (size_t)lay.total * sizeof(float);
-    if (bytes > ctx->packed_tc_cap) {
-        TG_CUDA(cudaSetDevice(ctx->device));
-        if (ctx->packed_tc) {
-            TG_CUDA(cudaDeviceSynchronize());
-            TG_CUDA(cudaFree(ctx->packed_tc));
-            ctx->packed_tc = nullptr;
-            ctx->packed_tc_cap = 0;
-        }
-        TG_CUDA(cudaMalloc(&ctx->packed_tc, bytes));
-        ctx->packed_tc_cap = bytes;
-    }
+    int rc = tg_ctx_grow(ctx, (void **)&ctx->packed_tc, &ctx->packed_tc_cap, (size_t)lay.total * sizeof(float));
+    if (rc) return rc;
     int64_t blocks = (lay.total + 255) / 256;
     if (blocks > 1024) blocks = 1024;
     pack_tc_kernel<<<(unsigned)blocks, 256, 0, st>>>(lay, params, ctx->packed_tc);
@@ -199,19 +173,118 @@ int tg_pack_weights_tc(tg_ctx *ctx, const tg_tc_layout &lay, const float *params
     return TG_OK;
 }
 
+// ---------------------------------------------------------------------------
+// wide tensor-core staging (TcwLayout, tg_common.cuh)
+// ---------------------------------------------------------------------------
+void tg_build_tcw_layout(const tg_mlp_cfg *mlp, TcwLayout *L, bool with_backward) {
+    memset(L, 0, sizeof(*L));
+    L->O = mlp->dims[0];
+    L->OKP = (L->O + 1 + 7) / 8 * 8;
+    L->A = mlp->dims[3];
+    L->act = mlp->activation;
+    L->W = mlp->dims[1];
+    const int W = L->W;
+    int64_t off = 0;
+    L->w0hi = off; off += (int64_t)W * L->OKP;
+    L->w0lo = off; off += (int64_t)W * L->OKP;
+    L->b1 = off; off += W;
+    L->wo = off; off += (int64_t)L->A * W;
+    L->bo = off; off += 4;
+    L->resident = (off + 255) / 256 * 256;
+    L->chunk_floats = (int64_t)W * 32;
+    L->chunks_f = L->resident;
+    L->chunks_b = L->chunks_f + (int64_t)(2 * W / 32) * L->chunk_floats;
+    L->total = with_backward ? L->chunks_b + (int64_t)(2 * W / 32) * L->chunk_floats : L->chunks_b;
+    int64_t flat = 0;
+    for (int l = 0; l < 3; ++l) {
+        L->flat_w[l] = flat;
+        flat += (int64_t)mlp->dims[l] * mlp->dims[l + 1] + mlp->dims[l + 1];
+    }
+    L->n_params = flat;
+}
+
+__global__ void pack_tcw_kernel(TcwLayout L, const float *__restrict__ params, float *__restrict__ packed) {
+    const int W = L.W;
+    const float *W0 = params + L.flat_w[0], *b0 = W0 + (int64_t)W * L.O;
+    const float *W1 = params + L.flat_w[1], *b1 = W1 + (int64_t)W * W;
+    const float *Wo = params + L.flat_w[2], *bo = Wo + (int64_t)L.A * W;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < L.total; i += (int64_t)gridDim.x * blockDim.x) {
+        float v = 0.0f;
+        if (i < L.b1) {
+            const bool lo = i >= L.w0lo;
+            int n, c;
+            core_invert(L.OKP, i - (lo ? L.w0lo : L.w0hi), &n, &c);
+            const float w = c < L.O ? W0[(int64_t)n * L.O + c] : (c == L.O ? b0[n] : 0.0f);
+            const float h = tf32_hi(w);
+            v = lo ? (w - h) : h;
+        } else if (i < L.wo) {
+            v = b1[i - L.b1];
+        } else if (i < L.bo) {
+            v = Wo[i - L.wo];
+        } else if (i < L.bo + L.A) {
+            v = bo[i - L.bo];
+        } else if (i >= L.chunks_f && i < L.chunks_b) {
+            // forward: chunk = (K-chunk kc, hi/lo); [W rows n][32 k] K-major core-matrix layout
+            const int64_t j = i - L.chunks_f;
+            const int chunk = (int)(j / L.chunk_floats);
+            const bool lo = (chunk & 1) != 0;
+            const int kc = chunk >> 1;
+            int n, kk;
+            core_invert(32, j % L.chunk_floats, &n, &kk);
+            const float w = W1[(int64_t)n * W + kc * 32 + kk];
+            const float h = tf32_hi(w);
+            v = lo ? (w - h) : h;
+        } else if (i >= L.chunks_b) {
+            // backward: chunk = (32 out-rows kc, hi/lo); [32 rows out][W cols in] MN-major SW128_32B layout
+            const int64_t j = i - L.chunks_b;
+            const int chunk = (int)(j / L.chunk_floats);
+            const bool lo = (chunk & 1) != 0;
+            const int kc = chunk >> 1;
+            int r, c;
+            mn32_invert(32, j % L.chunk_floats, &r, &c);
+            const float w = W1[(int64_t)(kc * 32 + r) * W + c];
+            const float h = tf32_hi(w);
+            v = lo ? (w - h) : h;
+        }
+        packed[i] = v;
+    }
+}
+
+int tg_pack_weights_tcw(tg_ctx *ctx, const TcwLayout &lay, const float *params, cudaStream_t st) {
+    int rc = tg_ctx_grow(ctx, (void **)&ctx->packed_tc, &ctx->packed_tc_cap, (size_t)lay.total * sizeof(float));
+    if (rc) return rc;
+    pack_tcw_kernel<<<296, 256, 0, st>>>(lay, params, ctx->packed_tc);
+    TG_CUDA(cudaGetLastError());
+    return TG_OK;
+}
+
 extern "C" int tg_ctx_sm_count(const tg_ctx *ctx) { return ctx ? ctx->sm_count : 0; }
 
-int tg_ctx_reserve_packed(tg_ctx *ctx, size_t bytes) {
-    if (bytes <= ctx->packed_cap) return TG_OK;
+int tg_ctx_grow(tg_ctx *ctx, void **buf, size_t *cap, size_t bytes) {
+    if (bytes <= *cap) return TG_OK;
     TG_CUDA(cudaSetDevice(ctx->device));
-    if (ctx->packed) {
+    if (*buf) {
         TG_CUDA(cudaDeviceSynchronize());
-        TG_CUDA(cudaFree(ctx->packed));
-        ctx->packed = nullptr;
-        ctx->packed_cap = 0;
+        TG_CUDA(cudaFree(*buf));
+        *buf = nullptr;
+        *cap = 0;
     }
-    TG_CUDA(cudaMalloc(&ctx->packed, bytes));
-    ctx->packed_cap = bytes;
+    TG_CUDA(cudaMalloc(buf, bytes));
+    *cap = bytes;
+    return TG_OK;
+}
+
+int tg_gauss_consts(const float *cov_diag, int A, float *sd, float *inv_sd, float *inv_var, float *log_norm) {
+    double ln = 0.5 * A * log(2.0 * M_PI);
+    for (int j = 0; j < A; ++j) {
+        TG_REQUIRE(cov_diag[j] > 0.0f, TG_ERR_ARG, "cov_diag[%d] must be positive", j);
+        const float s = sqrtf(cov_diag[j]);
+        if (sd) sd[j] = s;
+        if (inv_sd) inv_sd[j] = 1.0f / s;
+        if (inv_var) inv_var[j] = 1.0f / (s * s);
+        ln += (double)logf(s);
+    }
+    *log_norm = (float)ln;
     return TG_OK;
 }
 
@@ -382,7 +455,7 @@ __global__ void pack_kernel(tg_mlp_layout lay, const float *__restrict__ params,
 }
 
 int tg_pack_weights(tg_ctx *ctx, const tg_mlp_layout &lay, const float *params, cudaStream_t st) {
-    int rc = tg_ctx_reserve_packed(ctx, (size_t)lay.total * sizeof(float));
+    int rc = tg_ctx_grow(ctx, (void **)&ctx->packed, &ctx->packed_cap, (size_t)lay.total * sizeof(float));
     if (rc) return rc;
     const int threads = 256;
     int64_t blocks = (lay.total + threads - 1) / threads;

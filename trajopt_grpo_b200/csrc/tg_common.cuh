@@ -41,20 +41,20 @@ struct TgRange {
 struct TgRange { explicit TgRange(const char *) {} };
 #endif
 
+// Device buffers owned by the ctx are grown with tg_ctx_grow and freed by tg_ctx_destroy.
 struct tg_ctx {
     int device;
     int sm_count;
     int smem_optin;  // max dynamic shared memory per block (bytes)
     float *packed;   // staged (transposed / padded) policy weights, device
     size_t packed_cap;
-    float *packed_tc;  // staged tensor-core operands (hi/lo split, SWIZZLE_128B), device
+    float *packed_tc;  // staged tensor-core operands (hi/lo split, core-matrix / SW128_32B layouts), device
     size_t packed_tc_cap;
     int math_mode;     // TG_MATH_*
-    int rollout_tc2;   // diagnostics: route width-64 rollouts to the two-threads-per-env kernel too
-    // length order of the rollout being updated (tg_order.cu): env indices sorted by episode length,
-    // longest first, and the number of live envs per step; device, owned by the ctx
     void *scratch;     // HBM scratch of the wide tensor-core update (tg_update_tcw.cu), device
     size_t scratch_cap;
+    // length order of the rollout being updated (tg_order.cu): env indices sorted by episode length,
+    // longest first, and the number of live envs per step; device, in order_buf
     void *order_buf;
     size_t order_cap;
     int32_t *perm, *cnt;
@@ -66,7 +66,13 @@ struct tg_ctx {
 };
 // fills ctx->perm [N] and ctx->cnt [T] for `len` (asynchronous on `st`)
 int tg_len_order(tg_ctx *ctx, int64_t N, int T, const int32_t *len, cudaStream_t st);
-int tg_ctx_reserve_packed(tg_ctx *ctx, size_t bytes);
+// makes *buf (capacity *cap, a device buffer of ctx) hold at least `bytes`; a smaller buffer is freed after a
+// device synchronise (kernels in flight may still read it) and replaced, its contents are not kept
+int tg_ctx_grow(tg_ctx *ctx, void **buf, size_t *cap, size_t bytes);
+// constants of the diagonal Gaussian policy N(mu, diag(cov_diag)) over A actions: sd = sqrtf(cov_diag) (fp32, as
+// torch's cholesky of diag(c)), inv_sd = 1 / sd, inv_var = 1 / sd^2, log_norm = A/2 log(2 pi) + sum log sd
+// (summed in double).  Null outputs are skipped; TG_ERR_ARG unless every cov_diag[j] > 0.
+int tg_gauss_consts(const float *cov_diag, int A, float *sd, float *inv_sd, float *inv_var, float *log_norm);
 
 // ---- MLP tile configurations --------------------------------------------------
 // A CTA advances B environments (rollout) / B samples (update) at a time with NT
@@ -135,6 +141,26 @@ struct tg_tc_layout {
 bool tg_tc_eligible(const tg_mlp_cfg *mlp);
 int tg_build_tc_layout(const tg_mlp_cfg *mlp, tg_tc_layout *out, bool with_backward = false);
 int tg_pack_weights_tc(tg_ctx *ctx, const tg_tc_layout &lay, const float *params, cudaStream_t st);
+
+// Wide staging (obs -> W -> W -> act, W = 128 or 256): the 256-wide rollout (tg_rollout_tc256.cu) and the wide
+// update (tg_update_tcw.cu).  The hidden [W x W] weight does not fit in shared memory next to the rest; it is
+// streamed from L2 in chunks of 32 reduction columns (32 KB at W = 256).  Staged buffer (floats):
+//   resident block, copied once into shared memory (multiple of 256 floats):
+//     w0hi, w0lo [W x OKP]  first Linear rows (W0[n][:], b0[n], 0..), core-matrix layout, OKP = roundup(O + 1, 8)
+//     b1 [W], wo [A][W], bo [4]
+//   chunks_f: forward chunks hi(0), lo(0), hi(1), .. of W1 [W rows out][32 cols in], K-major core-matrix layout
+//   chunks_b: backward chunks (update only) of W1 [32 rows out][W cols in], MN-major SW128_32B layout
+struct TcwLayout {
+    int O, OKP, A, act, W;
+    int64_t w0hi, w0lo, b1, wo, bo;      // offsets (floats) in the resident block
+    int64_t resident;                     // floats, multiple of 256
+    int64_t chunks_f, chunks_b;           // forward (K-major) / backward (MN-major) chunk streams
+    int64_t chunk_floats;                 // W * 32
+    int64_t total;                        // floats; = chunks_b without the backward chunks
+    int64_t flat_w[3], n_params;
+};
+void tg_build_tcw_layout(const tg_mlp_cfg *mlp, TcwLayout *out, bool with_backward);
+int tg_pack_weights_tcw(tg_ctx *ctx, const TcwLayout &lay, const float *params, cudaStream_t st);
 // wide (128 / 256) tensor-core update, two streamed kernels per batch of tiles (tg_update_tcw.cu)
 bool tg_update_tcw_shape_built(const tg_mlp_cfg *mlp);
 int tg_policy_grad_tcw(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N, int T, const float *obs, const float *act,

@@ -35,19 +35,6 @@ __global__ void order_count_kernel(int64_t N, int T, const uint32_t *__restrict_
     cnt[t] = (int32_t)lo;
 }
 
-static int reserve(void **p, size_t *cap, size_t bytes) {
-    if (bytes <= *cap) return TG_OK;
-    if (*p) {
-        TG_CUDA(cudaDeviceSynchronize());
-        TG_CUDA(cudaFree(*p));
-        *p = nullptr;
-        *cap = 0;
-    }
-    TG_CUDA(cudaMalloc(p, bytes));
-    *cap = bytes;
-    return TG_OK;
-}
-
 extern "C" int tg_len_order_hold(tg_ctx *ctx, int64_t N, int T, const int32_t *len, void *stream) {
     TG_REQUIRE(ctx && len, TG_ERR_ARG, "tg_len_order_hold: null argument");
     TG_CUDA(cudaSetDevice(ctx->device));
@@ -74,7 +61,7 @@ int tg_len_order(tg_ctx *ctx, int64_t N, int T, const int32_t *len, cudaStream_t
                                             (const int32_t *)nullptr, (int32_t *)nullptr, (int)N, 0, bits, st));
     const size_t nb = ((size_t)N * 4 + 255) / 256 * 256, tb = ((size_t)T * 4 + 255) / 256 * 256;
     // [perm | cnt | key_in | key_out | idx_in | cub temp]
-    int rc = reserve((void **)&ctx->order_buf, &ctx->order_cap, 4 * nb + tb + temp + 256);
+    int rc = tg_ctx_grow(ctx, &ctx->order_buf, &ctx->order_cap, 4 * nb + tb + temp + 256);
     if (rc) return rc;
     char *base = (char *)ctx->order_buf;
     ctx->perm = (int32_t *)base;

@@ -23,9 +23,9 @@
 // tg_rollout_tc256.cu
 bool tg_tc256_eligible(const tg_mlp_cfg *mlp);
 int tg_rollout_tc256(tg_ctx *ctx, const tg_env_cfg *env, const EnvParams &ep, const tg_mlp_cfg *mlp, int precision,
-                     int64_t N, const void *init_state, const float *params, const float *cov_diag, const float *noise,
-                     uint64_t seed, int64_t env_offset, float *out_obs, float *out_act, float *out_rew, float *out_logp,
-                     int32_t *out_len, float *out_ret, cudaStream_t st);
+                     int64_t N, const void *init_state, const float *params, const float *sd, float log_norm,
+                     const float *noise, uint64_t seed, int64_t env_offset, float *out_obs, float *out_act, float *out_rew,
+                     float *out_logp, int32_t *out_len, float *out_ret, cudaStream_t st);
 
 struct RolloutArgs {
     EnvParams env;
@@ -389,8 +389,8 @@ __global__ void __launch_bounds__(128) rollout_tc_kernel(const __grid_constant__
 }
 
 // ---------------------------------------------------------------------------
-// Tensor-core variant with TWO threads per env (256 threads per 128-env tile) for hidden widths
-// 64 and 128: env e = TMEM lane e is served by warps q and q+4 of lane quadrant q, each owning one
+// Tensor-core variant with TWO threads per env (256 threads per 128-env tile) for hidden width
+// 128: env e = TMEM lane e is served by warps q and q+4 of lane quadrant q, each owning one
 // half (HW = W/2 columns) of every activation row, so a 128-wide row costs 64 registers per thread.
 // The hidden activation goes to the tensor core as the A operand straight from registers through
 // tensor memory (tcgen05.st, hi/lo split; tcgen05.mma with A in TMEM), the [W x W] weight (hi/lo,
@@ -404,7 +404,7 @@ __global__ void __launch_bounds__(256, 1) rollout_tc2_kernel(const __grid_consta
     using E = Env<KIND>;
     constexpr int S = E::S, A = E::A, HW = W / 2, O4 = (S + 1 + 3) / 4 * 4;
     constexpr uint32_t TM_D = 0u, TM_AHI = (uint32_t)W, TM_ALO = 2u * (uint32_t)W;
-    constexpr uint32_t TM_COLS = W == 64 ? 256u : 512u;
+    constexpr uint32_t TM_COLS = 512u;
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     __shared__ __align__(8) uint64_t wbar, mbar;
     __shared__ uint32_t tmem_slot;
@@ -672,12 +672,14 @@ extern "C" int tg_rollout(tg_ctx *ctx, const tg_env_cfg *env, const tg_mlp_cfg *
                mlp->n_layers, TG_MAX_LAYERS);
     TG_REQUIRE(mlp->dims[0] == O && mlp->dims[mlp->n_layers] == A, TG_ERR_SHAPE,
                "policy dims (%d -> %d) do not match env obs/act dims (%d/%d)", mlp->dims[0], mlp->dims[mlp->n_layers], O, A);
+    rc = tg_gauss_consts(cov_diag, A, a.sd, nullptr, nullptr, &a.log_norm);
+    if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     TG_CUDA(cudaSetDevice(ctx->device));
     // ---- tensor-core paths (3xTF32 tcgen05) for eligible policies
     if (tg_tc256_eligible(mlp) && ctx->math_mode != TG_MATH_FP32)      // 256-wide: weights streamed from L2
-        return tg_rollout_tc256(ctx, env, a.env, mlp, precision, N, init_state, params, cov_diag, noise, seed, env_offset,
-                                out_obs, out_act, out_rew, out_logp, out_len, out_ret, st);
+        return tg_rollout_tc256(ctx, env, a.env, mlp, precision, N, init_state, params, a.sd, a.log_norm, noise, seed,
+                                env_offset, out_obs, out_act, out_rew, out_logp, out_len, out_ret, st);
     const bool tc_ok = tg_tc_eligible(mlp);
     TG_REQUIRE(ctx->math_mode != TG_MATH_3XTF32 || tc_ok, TG_ERR_UNSUPPORTED,
                "TG_MATH_3XTF32 requested but the policy shape is not eligible (>= 2 hidden layers of equal width 64 or 128)");
@@ -691,30 +693,17 @@ extern "C" int tg_rollout(tg_ctx *ctx, const tg_env_cfg *env, const tg_mlp_cfg *
         if (rc) return rc;
         b.N = N; b.init_state = init_state; b.packed = ctx->packed_tc; b.noise = noise; b.seed = seed;
         b.env_offset = env_offset;
-        double lnb = 0.5 * A * log(2.0 * M_PI);
-        for (int j = 0; j < A; ++j) {
-            TG_REQUIRE(cov_diag[j] > 0.0f, TG_ERR_ARG, "cov_diag[%d] must be positive", j);
-            b.sd[j] = sqrtf(cov_diag[j]);
-            lnb += (double)logf(b.sd[j]);
-        }
-        b.log_norm = (float)lnb;
+        memcpy(b.sd, a.sd, sizeof(b.sd));
+        b.log_norm = a.log_norm;
         b.obs = out_obs; b.act = out_act; b.rew = out_rew; b.logp = out_logp; b.len = out_len; b.ret = out_ret;
         TG_REQUIRE(((size_t)b.lay.total * 4 + 1023) / 1024 * 1024 + 4096 <= (size_t)ctx->smem_optin, TG_ERR_UNSUPPORTED,
                    "staged tensor-core weights need %zu B of shared memory", (size_t)b.lay.total * 4);
-        if (b.lay.W == 128 || ctx->rollout_tc2) {
-            if (b.lay.W == 128) {
-                switch (env->kind) {
-                    case TG_ENV_CARTPOLE: return launch_rollout_tc2<TG_ENV_CARTPOLE, 128>(precision, b, st);
-                    case TG_ENV_PENDULUM: return launch_rollout_tc2<TG_ENV_PENDULUM, 128>(precision, b, st);
-                    case TG_ENV_QUADPOLE2D: return launch_rollout_tc2<TG_ENV_QUADPOLE2D, 128>(precision, b, st);
-                    default: return launch_rollout_tc2<TG_ENV_QUADPOLE, 128>(precision, b, st);
-                }
-            }
+        if (b.lay.W == 128) {
             switch (env->kind) {
-                case TG_ENV_CARTPOLE: return launch_rollout_tc2<TG_ENV_CARTPOLE, 64>(precision, b, st);
-                case TG_ENV_PENDULUM: return launch_rollout_tc2<TG_ENV_PENDULUM, 64>(precision, b, st);
-                case TG_ENV_QUADPOLE2D: return launch_rollout_tc2<TG_ENV_QUADPOLE2D, 64>(precision, b, st);
-                default: return launch_rollout_tc2<TG_ENV_QUADPOLE, 64>(precision, b, st);
+                case TG_ENV_CARTPOLE: return launch_rollout_tc2<TG_ENV_CARTPOLE, 128>(precision, b, st);
+                case TG_ENV_PENDULUM: return launch_rollout_tc2<TG_ENV_PENDULUM, 128>(precision, b, st);
+                case TG_ENV_QUADPOLE2D: return launch_rollout_tc2<TG_ENV_QUADPOLE2D, 128>(precision, b, st);
+                default: return launch_rollout_tc2<TG_ENV_QUADPOLE, 128>(precision, b, st);
             }
         }
         switch (env->kind) {
@@ -734,13 +723,6 @@ extern "C" int tg_rollout(tg_ctx *ctx, const tg_env_cfg *env, const tg_mlp_cfg *
     a.noise = noise;
     a.seed = seed;
     a.env_offset = env_offset;
-    double ln = 0.5 * A * log(2.0 * M_PI);
-    for (int j = 0; j < A; ++j) {
-        TG_REQUIRE(cov_diag[j] > 0.0f, TG_ERR_ARG, "cov_diag[%d] must be positive", j);
-        a.sd[j] = sqrtf(cov_diag[j]);                      // cholesky(diag(c)) = diag(sqrt(c)), fp32 as torch
-        ln += (double)logf(a.sd[j]);
-    }
-    a.log_norm = (float)ln;
     a.obs = out_obs; a.act = out_act; a.rew = out_rew; a.logp = out_logp; a.len = out_len; a.ret = out_ret;
     const int B = a.lay.B, NT = a.lay.NT;
     const size_t act_bytes = (2 * (size_t)a.lay.kmax * (B + 4) + (size_t)(NT / B) * TG_MAX_ACT * B) * sizeof(float);

@@ -33,18 +33,9 @@
 #define CHUNK_FLOATS (W256 * CHUNK_K)           // 8192 floats = 32 KB
 #define N_CHUNKS (2 * W256 / CHUNK_K)           // 16: (hi, lo) x 8 K-chunks
 
-struct Tc256Layout {
-    int O, OKP, A, act;
-    int64_t w0hi, w0lo, b1, wo, bo;             // offsets (floats) inside the resident block
-    int64_t resident;                            // floats, multiple of 256
-    int64_t chunks;                              // offset of chunk 0; chunk i at chunks + i*CHUNK_FLOATS, order hi(0),lo(0),hi(1),..
-    int64_t total;
-    int64_t flat_w[3];
-};
-
 struct RolloutTc256Args {
     EnvParams env;
-    Tc256Layout lay;
+    TcwLayout lay;                               // built without the backward chunks
     int64_t N;
     const void *init_state;
     const float *packed;
@@ -62,82 +53,9 @@ bool tg_tc256_eligible(const tg_mlp_cfg *mlp) {
            mlp->activation <= 2;
 }
 
-static void build_tc256_layout(const tg_mlp_cfg *mlp, Tc256Layout *L) {
-    memset(L, 0, sizeof(*L));
-    L->O = mlp->dims[0];
-    L->OKP = (L->O + 1 + 7) / 8 * 8;
-    L->A = mlp->dims[3];
-    L->act = mlp->activation;
-    int64_t off = 0;
-    L->w0hi = off; off += (int64_t)W256 * L->OKP;
-    L->w0lo = off; off += (int64_t)W256 * L->OKP;
-    L->b1 = off; off += W256;
-    L->wo = off; off += (int64_t)L->A * W256;
-    L->bo = off; off += 4;
-    L->resident = (off + 255) / 256 * 256;
-    L->chunks = L->resident;
-    L->total = L->resident + (int64_t)N_CHUNKS * CHUNK_FLOATS;
-    int64_t flat = 0;
-    for (int l = 0; l < 3; ++l) {
-        L->flat_w[l] = flat;
-        flat += (int64_t)mlp->dims[l] * mlp->dims[l + 1] + mlp->dims[l + 1];
-    }
-}
-
-TG_D float tf32_hi_of(float w) {
-    uint32_t hb;
-    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(hb) : "f"(w));
-    return __uint_as_float(hb & 0xffffe000u);
-}
-
-// invert the K-major core-matrix layout of a stored [R][C] matrix: float index -> (row, col)
-TG_D void core_invert(int C, int64_t idx, int *r, int *c) {
-    const uint32_t b = (uint32_t)idx * 4u;
-    const uint32_t group = (uint32_t)(C >> 2) * 128u;
-    const uint32_t rr = b % group;
-    *r = (int)(b / group) * 8 + (int)((rr % 128u) >> 4);
-    *c = (int)(rr / 128u) * 4 + (int)((rr & 15u) >> 2);
-}
-
-__global__ void pack_tc256_kernel(Tc256Layout L, const float *__restrict__ params, float *__restrict__ packed) {
-    const float *W0 = params + L.flat_w[0], *b0 = W0 + (int64_t)W256 * L.O;
-    const float *W1 = params + L.flat_w[1], *b1 = W1 + (int64_t)W256 * W256;
-    const float *Wo = params + L.flat_w[2], *bo = Wo + (int64_t)L.A * W256;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < L.total; i += (int64_t)gridDim.x * blockDim.x) {
-        float v = 0.0f;
-        if (i < L.b1) {                          // first Linear, rows (W0[n][:], b0[n], 0..), hi then lo
-            const bool lo = i >= L.w0lo;
-            int n, c;
-            core_invert(L.OKP, i - (lo ? L.w0lo : L.w0hi), &n, &c);
-            const float w = c < L.O ? W0[(int64_t)n * L.O + c] : (c == L.O ? b0[n] : 0.0f);
-            const float h = tf32_hi_of(w);
-            v = lo ? (w - h) : h;
-        } else if (i < L.wo) {
-            v = b1[i - L.b1];
-        } else if (i < L.bo) {
-            v = Wo[i - L.wo];
-        } else if (i < L.bo + L.A) {
-            v = bo[i - L.bo];
-        } else if (i >= L.chunks) {
-            const int64_t j = i - L.chunks;
-            const int chunk = (int)(j / CHUNK_FLOATS);
-            const bool lo = (chunk & 1) != 0;
-            const int kc = chunk >> 1;
-            int n, kk;
-            core_invert(CHUNK_K, j % CHUNK_FLOATS, &n, &kk);
-            const float w = W1[(int64_t)n * W256 + kc * CHUNK_K + kk];     // torch [out][in] = K-major B operand
-            const float h = tf32_hi_of(w);
-            v = lo ? (w - h) : h;
-        }
-        packed[i] = v;
-    }
-}
-
 #define BAR_L1 5
 #define BAR_K0 6
 #define BAR_K1 7
-TG_D void nb_arrive(int id, int count) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(count) : "memory"); }
-TG_D void nb_sync(int id, int count) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(count) : "memory"); }
 
 template <int KIND, typename R, bool RELU>
 __global__ void __launch_bounds__(576, 1) rollout_tc256_kernel(const __grid_constant__ RolloutTc256Args a) {
@@ -182,7 +100,7 @@ __global__ void __launch_bounds__(576, 1) rollout_tc256_kernel(const __grid_cons
     if (warp == 16) {
         // ===== TMA producer: streams the 16 weight chunks of every step through the ring =====
         uint32_t gi = 0;
-        const float *src = a.packed + a.lay.chunks;
+        const float *src = a.packed + a.lay.chunks_f;
         for (int t = 0; t < T; ++t) {
             if (lane == 0) {
                 for (int i = 0; i < N_CHUNKS; ++i, ++gi) {
@@ -205,7 +123,7 @@ __global__ void __launch_bounds__(576, 1) rollout_tc256_kernel(const __grid_cons
         uint32_t gi = 0;
         for (int t = 0; t < T; ++t) {
             // ---- first Linear: D = [obs, 1] . [W0, b0]^T  (3xTF32, both operands K-major in smem)
-            nb_sync(BAR_L1, 544);
+            named_sync(BAR_L1, 544);
             tc_fence_after();
             if (lane == 0) {
                 uint32_t acc = 0;
@@ -224,8 +142,8 @@ __global__ void __launch_bounds__(576, 1) rollout_tc256_kernel(const __grid_cons
             __syncwarp();
             // ---- second Linear, two K halves; each (hi, lo) chunk pair: A_hi.B_hi, A_lo.B_hi, A_hi.B_lo
             for (int half = 0; half < 2; ++half) {
-                if (half == 0) nb_sync(BAR_K0, 544);
-                else nb_sync(BAR_K1, 288);
+                if (half == 0) named_sync(BAR_K0, 544);
+                else named_sync(BAR_K1, 288);
                 tc_fence_after();
                 if (lane == 0) {
                     for (int c = 0; c < 4; ++c) {
@@ -298,7 +216,7 @@ __global__ void __launch_bounds__(576, 1) rollout_tc256_kernel(const __grid_cons
             }
             fence_proxy_async();
             tc_fence_before();
-            nb_arrive(BAR_L1, 544);
+            named_arrive(BAR_L1, 544);
             mbar_wait(&bar_d, ph_d);
             ph_d ^= 1u;
             tc_fence_after();
@@ -313,7 +231,7 @@ __global__ void __launch_bounds__(576, 1) rollout_tc256_kernel(const __grid_cons
             }
             tc_fence_before();
             if (part >= 2) {
-                nb_arrive(BAR_K0, 544);               // this thread has read D; its K half waits for half 0
+                named_arrive(BAR_K0, 544);               // this thread has read D; its K half waits for half 0
                 mbar_wait(&bar_k0, ph_k0);
                 tc_fence_after();
             }
@@ -334,8 +252,8 @@ __global__ void __launch_bounds__(576, 1) rollout_tc256_kernel(const __grid_cons
                 tmem_st_wait();
                 tc_fence_before();
             }
-            if (part >= 2) nb_arrive(BAR_K1, 288);
-            else nb_arrive(BAR_K0, 544);
+            if (part >= 2) named_arrive(BAR_K1, 288);
+            else named_arrive(BAR_K0, 544);
             mbar_wait(&bar_d, ph_d);
             ph_d ^= 1u;
             tc_fence_after();
@@ -363,7 +281,7 @@ __global__ void __launch_bounds__(576, 1) rollout_tc256_kernel(const __grid_cons
             tc_fence_before();
 #pragma unroll
             for (int j = 0; j < A; ++j) muS[part][j][e] = pm[j];
-            nb_sync(q + 1, 128);                      // the four warps of this lane quadrant
+            named_sync(q + 1, 128);                      // the four warps of this lane quadrant
             if (part == 0) {
                 float mu[A];
 #pragma unroll
@@ -437,37 +355,19 @@ static int launch_tc256(int precision, const RolloutTc256Args &a, size_t smem, c
 
 // Called by tg_rollout (tg_rollout.cu) for eligible 256-wide policies.
 int tg_rollout_tc256(tg_ctx *ctx, const tg_env_cfg *env, const EnvParams &ep, const tg_mlp_cfg *mlp, int precision,
-                     int64_t N, const void *init_state, const float *params, const float *cov_diag, const float *noise,
-                     uint64_t seed, int64_t env_offset, float *out_obs, float *out_act, float *out_rew, float *out_logp,
-                     int32_t *out_len, float *out_ret, cudaStream_t st) {
+                     int64_t N, const void *init_state, const float *params, const float *sd, float log_norm,
+                     const float *noise, uint64_t seed, int64_t env_offset, float *out_obs, float *out_act, float *out_rew,
+                     float *out_logp, int32_t *out_len, float *out_ret, cudaStream_t st) {
     RolloutTc256Args a;
     memset(&a, 0, sizeof(a));
     a.env = ep;
-    build_tc256_layout(mlp, &a.lay);
-    // staged weights live in the ctx's tensor-core staging buffer
-    const size_t bytes = (size_t)a.lay.total * sizeof(float);
-    if (bytes > ctx->packed_tc_cap) {
-        if (ctx->packed_tc) {
-            TG_CUDA(cudaDeviceSynchronize());
-            TG_CUDA(cudaFree(ctx->packed_tc));
-            ctx->packed_tc = nullptr;
-            ctx->packed_tc_cap = 0;
-        }
-        TG_CUDA(cudaMalloc(&ctx->packed_tc, bytes));
-        ctx->packed_tc_cap = bytes;
-    }
-    pack_tc256_kernel<<<296, 256, 0, st>>>(a.lay, params, ctx->packed_tc);
-    TG_CUDA(cudaGetLastError());
+    tg_build_tcw_layout(mlp, &a.lay, false);
+    int rc = tg_pack_weights_tcw(ctx, a.lay, params, st);
+    if (rc) return rc;
     a.N = N; a.init_state = init_state; a.packed = ctx->packed_tc; a.noise = noise; a.seed = seed;
     a.env_offset = env_offset;
-    const int A = a.lay.A;
-    double lnb = 0.5 * A * log(2.0 * M_PI);
-    for (int j = 0; j < A; ++j) {
-        TG_REQUIRE(cov_diag[j] > 0.0f, TG_ERR_ARG, "cov_diag[%d] must be positive", j);
-        a.sd[j] = sqrtf(cov_diag[j]);
-        lnb += (double)logf(a.sd[j]);
-    }
-    a.log_norm = (float)lnb;
+    memcpy(a.sd, sd, sizeof(a.sd));
+    a.log_norm = log_norm;
     a.obs = out_obs; a.act = out_act; a.rew = out_rew; a.logp = out_logp; a.len = out_len; a.ret = out_ret;
     const size_t smem = (size_t)RING_STAGES * CHUNK_FLOATS * 4 + (size_t)a.lay.resident * 4 + 2 * (size_t)128 * a.lay.OKP * 4;
     TG_REQUIRE(smem + 12 * 1024 <= (size_t)ctx->smem_optin, TG_ERR_UNSUPPORTED, "tc256 rollout needs %zu B of shared memory", smem);

@@ -32,11 +32,21 @@ TG_D float tf32_hi(float x) {
     asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
     return __uint_as_float(r & 0xffffe000u);
 }
+// the value the tensor core uses for a raw fp32 operand of kind::tf32: the low 13 mantissa bits dropped
+TG_D float tf32_trunc(float x) { return __uint_as_float(__float_as_uint(x) & 0xffffe000u); }
 
 // byte offset of element (r, c) of a stored [R][C] fp32 matrix in the core-matrix layout
 TG_HD uint32_t core_offset(int C, int r, int c) {
     return (uint32_t)(r >> 3) * (uint32_t)(C >> 2) * 128u + (uint32_t)(c >> 2) * 128u + (uint32_t)(r & 7) * 16u +
            (uint32_t)(c & 3) * 4u;
+}
+// inverse of core_offset: float index `idx` of a stored [R][C] matrix -> (row, col)
+TG_HD void core_invert(int C, int64_t idx, int *r, int *c) {
+    const uint32_t b = (uint32_t)idx * 4u;
+    const uint32_t group = (uint32_t)(C >> 2) * 128u;
+    const uint32_t rr = b % group;
+    *r = (int)(b / group) * 8 + (int)((rr % 128u) >> 4);
+    *c = (int)(rr / 128u) * 4 + (int)((rr & 15u) >> 2);
 }
 
 TG_D uint64_t umma_desc_raw(uint32_t smem_addr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
@@ -52,6 +62,13 @@ TG_D uint64_t umma_desc_raw(uint32_t smem_addr, uint32_t lbo_bytes, uint32_t sbo
 TG_HD uint32_t mn32_offset(int R, int r, int c) {
     return (uint32_t)(c >> 5) * (uint32_t)R * 128u + (uint32_t)r * 128u + (uint32_t)((((c & 31) >> 3) ^ (r & 3)) << 5) +
            (uint32_t)(c & 7) * 4u;
+}
+// inverse of mn32_offset: float index `idx` of a stored [R][C] matrix -> (row, col)
+TG_HD void mn32_invert(int R, int64_t idx, int *r, int *c) {
+    const uint32_t b = (uint32_t)idx * 4u;
+    const uint32_t blk = b / ((uint32_t)R * 128u), rr = b % ((uint32_t)R * 128u);
+    *r = (int)(rr / 128u);
+    *c = (int)blk * 32 + (((int)((rr % 128u) >> 5) ^ (*r & 3)) << 3) + (int)((rr & 31u) >> 2);
 }
 // layout type 1 = SWIZZLE_128B_BASE32B; LBO = next 32-element M/N block, SBO = next 4-row group
 TG_D uint64_t umma_desc_mn32(uint32_t smem_addr, uint32_t mn_block_bytes) {
@@ -83,6 +100,9 @@ TG_D void tmem_alloc(uint32_t *dst_smem, uint32_t ncols) {   // one full warp; n
 TG_D void tmem_dealloc(uint32_t taddr, uint32_t ncols) {     // same warp that allocated
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
 }
+// named barriers: bar.arrive does not wait, bar.sync waits until `count` threads have arrived at barrier `id`
+TG_D void named_arrive(int id, int count) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(count) : "memory"); }
+TG_D void named_sync(int id, int count) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(count) : "memory"); }
 TG_D void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 TG_D void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 // generic-proxy shared-memory writes -> visible to the async proxy (UMMA operand reads)

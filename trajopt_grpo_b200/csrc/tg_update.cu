@@ -13,7 +13,6 @@
 // kernel sums the private copies in a fixed order: the result is deterministic
 // and has the flat torch layout the NCCL allreduce and Adam consume.
 #include <math.h>
-#include <stdlib.h>
 
 #include "tg_mlp.cuh"
 
@@ -377,16 +376,21 @@ extern "C" int64_t tg_policy_grad_workspace_bytes(const tg_ctx *ctx, const tg_ml
     return grid * lay.n_params * (int64_t)sizeof(float) + grid * 4 * (int64_t)sizeof(double) + 256;
 }
 
-static int fill_gauss(UpdArgs &a, const float *cov_diag, int A) {
-    double ln = 0.5 * A * log(2.0 * M_PI);
-    for (int j = 0; j < A; ++j) {
-        TG_REQUIRE(cov_diag[j] > 0.0f, TG_ERR_ARG, "cov_diag[%d] must be positive", j);
-        const float sd = sqrtf(cov_diag[j]);
-        a.inv_sd[j] = 1.0f / sd;
-        a.inv_var[j] = 1.0f / (sd * sd);
-        ln += (double)logf(sd);
-    }
-    a.log_norm = (float)ln;
+// The gradient of every update path: the workspace holds one partial gradient per CTA, gpart [grid][n_params], and
+// the statistics spart [grid][4] (256-byte aligned); both are zeroed, `update(gpart, spart)` launches the kernels
+// that fill them, and grad_reduce_kernel sums the copies in a fixed order into out_grad / out_stats.
+template <typename Update>
+static int grad_via_partials(int grid, int64_t n_params, void *workspace, float *out_grad, float *out_stats,
+                             cudaStream_t st, Update update) {
+    const size_t gbytes = ((size_t)grid * n_params * sizeof(float) + 255) / 256 * 256;
+    float *gpart = reinterpret_cast<float *>(workspace);
+    double *spart = reinterpret_cast<double *>(reinterpret_cast<char *>(workspace) + gbytes);
+    TG_CUDA(cudaMemsetAsync(workspace, 0, gbytes + (size_t)grid * 4 * sizeof(double), st));
+    int rc = update(gpart, spart);
+    if (rc) return rc;
+    grad_reduce_kernel<<<(unsigned)((n_params + 255) / 256), 256, 0, st>>>(grid, n_params, gpart, spart, out_grad,
+                                                                          out_stats);
+    TG_CUDA(cudaGetLastError());
     return TG_OK;
 }
 
@@ -403,17 +407,11 @@ static int run_grad(tg_ctx *ctx, UpdArgs &a, const float *params, float *out_gra
         a.cnt = ctx->cnt;
     }
     const int grid = update_grid(ctx, a.lay);
-    const size_t gbytes = (size_t)grid * a.lay.n_params * sizeof(float);
-    a.gpart = reinterpret_cast<float *>(workspace);
-    a.spart = reinterpret_cast<double *>(reinterpret_cast<char *>(workspace) + ((gbytes + 255) / 256) * 256);
-    TG_CUDA(cudaMemsetAsync(a.gpart, 0, gbytes, st));
-    rc = dispatch_update(ctx, a, grid, st);
-    if (rc) return rc;
-    const int threads = 256;
-    grad_reduce_kernel<<<(unsigned)((a.lay.n_params + threads - 1) / threads), threads, 0, st>>>(
-        grid, a.lay.n_params, a.gpart, a.spart, out_grad, out_stats);
-    TG_CUDA(cudaGetLastError());
-    return TG_OK;
+    return grad_via_partials(grid, a.lay.n_params, workspace, out_grad, out_stats, st, [&](float *gpart, double *spart) {
+        a.gpart = gpart;
+        a.spart = spart;
+        return dispatch_update(ctx, a, grid, st);
+    });
 }
 
 extern "C" int tg_policy_grad(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N, int T, const float *obs, const float *act,
@@ -428,7 +426,7 @@ extern "C" int tg_policy_grad(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N, int
     memset(&a, 0, sizeof(a));
     int rc = tg_build_layout(mlp, true, &a.lay, ctx->smem_optin);
     if (rc) return rc;
-    rc = fill_gauss(a, cov_diag, a.lay.A);
+    rc = tg_gauss_consts(cov_diag, a.lay.A, nullptr, a.inv_sd, a.inv_var, &a.log_norm);
     if (rc) return rc;
     a.N = N; a.T = T; a.head = HEAD_POLICY;
     a.obs = obs; a.act = act; a.adv = adv; a.oldlp = old_logp; a.len = len;
@@ -438,17 +436,10 @@ extern "C" int tg_policy_grad(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N, int
         cudaStream_t st = (cudaStream_t)stream;
         TG_CUDA(cudaSetDevice(ctx->device));
         const int grid = ctx->sm_count;
-        const size_t gbytes = (size_t)grid * a.lay.n_params * sizeof(float);
-        float *gpart = reinterpret_cast<float *>(workspace);
-        double *spart = reinterpret_cast<double *>(reinterpret_cast<char *>(workspace) + ((gbytes + 255) / 256) * 256);
-        TG_CUDA(cudaMemsetAsync(gpart, 0, ((gbytes + 255) / 256) * 256 + (size_t)grid * 4 * sizeof(double), st));
-        rc = tg_policy_grad_tcw(ctx, mlp, N, T, obs, act, adv, old_logp, nullptr, len, params, a.inv_sd, a.inv_var, a.log_norm,
-                                eps_clip, scale, kl_coef, gpart, spart, grid, st);
-        if (rc) return rc;
-        grad_reduce_kernel<<<(unsigned)((a.lay.n_params + 255) / 256), 256, 0, st>>>(grid, a.lay.n_params, gpart, spart,
-                                                                                     out_grad, out_stats);
-        TG_CUDA(cudaGetLastError());
-        return TG_OK;
+        return grad_via_partials(grid, a.lay.n_params, workspace, out_grad, out_stats, st, [&](float *gpart, double *spart) {
+            return tg_policy_grad_tcw(ctx, mlp, N, T, obs, act, adv, old_logp, nullptr, len, params, a.inv_sd, a.inv_var,
+                                      a.log_norm, eps_clip, scale, kl_coef, gpart, spart, grid, st);
+        });
     }
     const bool tc_ok = tg_update_tc_eligible(mlp);
     TG_REQUIRE(ctx->math_mode != TG_MATH_3XTF32 || tc_ok, TG_ERR_UNSUPPORTED,
@@ -458,17 +449,10 @@ extern "C" int tg_policy_grad(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N, int
         cudaStream_t st = (cudaStream_t)stream;
         TG_CUDA(cudaSetDevice(ctx->device));
         const int grid = tg_update_tc_grid(ctx);
-        const size_t gbytes = (size_t)grid * a.lay.n_params * sizeof(float);
-        float *gpart = reinterpret_cast<float *>(workspace);
-        double *spart = reinterpret_cast<double *>(reinterpret_cast<char *>(workspace) + ((gbytes + 255) / 256) * 256);
-        TG_CUDA(cudaMemsetAsync(gpart, 0, gbytes, st));
-        rc = tg_policy_grad_tc(ctx, mlp, N, T, obs, act, adv, old_logp, len, params, a.inv_sd, a.inv_var, a.log_norm,
-                               eps_clip, scale, kl_coef, gpart, spart, grid, st);
-        if (rc) return rc;
-        grad_reduce_kernel<<<(unsigned)((a.lay.n_params + 255) / 256), 256, 0, st>>>(grid, a.lay.n_params, gpart, spart,
-                                                                                     out_grad, out_stats);
-        TG_CUDA(cudaGetLastError());
-        return TG_OK;
+        return grad_via_partials(grid, a.lay.n_params, workspace, out_grad, out_stats, st, [&](float *gpart, double *spart) {
+            return tg_policy_grad_tc(ctx, mlp, N, T, obs, act, adv, old_logp, len, params, a.inv_sd, a.inv_var, a.log_norm,
+                                     eps_clip, scale, kl_coef, gpart, spart, grid, st);
+        });
     }
     return run_grad(ctx, a, params, out_grad, out_stats, workspace, (cudaStream_t)stream);
 }
@@ -487,7 +471,7 @@ extern "C" int tg_policy_grad_batch(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t 
     memset(&a, 0, sizeof(a));
     int rc = tg_build_layout(mlp, true, &a.lay, ctx->smem_optin);
     if (rc) return rc;
-    rc = fill_gauss(a, cov_diag, a.lay.A);
+    rc = tg_gauss_consts(cov_diag, a.lay.A, nullptr, a.inv_sd, a.inv_var, &a.log_norm);
     if (rc) return rc;
     a.N = N; a.T = T; a.head = HEAD_POLICY;
     a.obs = obs; a.act = act; a.adv = adv; a.oldlp = old_logp;
@@ -532,17 +516,10 @@ extern "C" int tg_value_grad(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N, int 
         cudaStream_t st = (cudaStream_t)stream;
         TG_CUDA(cudaSetDevice(ctx->device));
         const int grid = ctx->sm_count;
-        const size_t gbytes = (size_t)grid * a.lay.n_params * sizeof(float);
-        float *gpart = reinterpret_cast<float *>(workspace);
-        double *spart = reinterpret_cast<double *>(reinterpret_cast<char *>(workspace) + ((gbytes + 255) / 256) * 256);
-        TG_CUDA(cudaMemsetAsync(gpart, 0, ((gbytes + 255) / 256) * 256 + (size_t)grid * 4 * sizeof(double), st));
-        rc = tg_policy_grad_tcw(ctx, mlp, N, T, obs, nullptr, nullptr, nullptr, target, len, params, nullptr, nullptr, 0.0f,
-                                0.0f, scale, 0.0f, gpart, spart, grid, st);
-        if (rc) return rc;
-        grad_reduce_kernel<<<(unsigned)((a.lay.n_params + 255) / 256), 256, 0, st>>>(grid, a.lay.n_params, gpart, spart,
-                                                                                     out_grad, out_stats);
-        TG_CUDA(cudaGetLastError());
-        return TG_OK;
+        return grad_via_partials(grid, a.lay.n_params, workspace, out_grad, out_stats, st, [&](float *gpart, double *spart) {
+            return tg_policy_grad_tcw(ctx, mlp, N, T, obs, nullptr, nullptr, nullptr, target, len, params, nullptr, nullptr,
+                                      0.0f, 0.0f, scale, 0.0f, gpart, spart, grid, st);
+        });
     }
     return run_grad(ctx, a, params, out_grad, out_stats, workspace, (cudaStream_t)stream);
 }
@@ -559,7 +536,7 @@ extern "C" int tg_policy_forward(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t M, 
     int rc = tg_build_layout(mlp, false, &a.lay, ctx->smem_optin);
     if (rc) return rc;
     if (cov_diag) {
-        rc = fill_gauss(a, cov_diag, a.lay.A);
+        rc = tg_gauss_consts(cov_diag, a.lay.A, nullptr, a.inv_sd, a.inv_var, &a.log_norm);
         if (rc) return rc;
     } else {
         for (int j = 0; j < TG_MAX_ACT; ++j) a.inv_sd[j] = a.inv_var[j] = 1.0f;
@@ -590,7 +567,7 @@ extern "C" int tg_policy_forward_traj(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_
     int rc = tg_build_layout(mlp, false, &a.lay, ctx->smem_optin);
     if (rc) return rc;
     if (cov_diag) {
-        rc = fill_gauss(a, cov_diag, a.lay.A);
+        rc = tg_gauss_consts(cov_diag, a.lay.A, nullptr, a.inv_sd, a.inv_var, &a.log_norm);
         if (rc) return rc;
     } else {
         for (int j = 0; j < TG_MAX_ACT; ++j) a.inv_sd[j] = a.inv_var[j] = 1.0f;

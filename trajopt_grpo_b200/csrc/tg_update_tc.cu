@@ -31,8 +31,6 @@
 // (tg_update.cu) sums the copies in a fixed order -> deterministic result in flat torch layout.
 #include <math.h>
 
-#include <stdlib.h>
-
 #include "tg_umma.cuh"
 
 struct UpdTcArgs {
@@ -118,8 +116,6 @@ TG_D void split4(const float *v, float4 &hi, float4 &lo) {
 // named barriers between the 8 compute warps (arrive, non-blocking) and the MMA issuer warp (sync)
 #define BAR_FWD 5
 #define BAR_BWD 6
-TG_D void named_arrive(int id, int count) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(count) : "memory"); }
-TG_D void named_sync(int id, int count) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(count) : "memory"); }
 
 // TMEM column map (512 columns allocated)
 #define TM_DF 0u     // forward accumulator  [128 x 64]
@@ -127,8 +123,10 @@ TG_D void named_sync(int id, int count) { asm volatile("bar.sync %0, %1;" ::"r"(
 #define TM_DW 128u   // dW1 [64 x 64], M = 64 layout, PERSISTENT across the CTA's tiles
 #define TM_A0 192u   // A operand buffer 0: hi at +0, lo at +64; buffer 1 at +128
 
-// NPART threads serve one sample (2 or 4): NPART*4 compute warps + the issuer warp
-template <int O, int A, bool RELU, int NPART>
+// NPART threads serve one sample: NPART*4 compute warps + the issuer warp (4 threads per sample measured no faster:
+// the kernel is bound by its instruction count and phase chain, not by warp parallelism; DESIGN.md K3-TC)
+constexpr int NPART = 2;
+template <int O, int A, bool RELU>
 __global__ void __launch_bounds__(NPART * 128 + 32, 1) update_tc_kernel(const __grid_constant__ UpdTcArgs a) {
     constexpr int W = TC_W, HW = TC_W / NPART, O4 = (O + 1 + 3) / 4 * 4;
     constexpr int NCW = NPART * 4, NT = NPART * 128 + 32;
@@ -422,7 +420,7 @@ __global__ void __launch_bounds__(NPART * 128 + 32, 1) update_tc_kernel(const __
             muS[hf][j][s] = acc;
         }
         // only the warps that share this lane quadrant exchange data: named barrier
-        asm volatile("bar.sync %0, %1;" ::"r"(q + 1), "r"(NPART * 32) : "memory");
+        named_sync(q + 1, NPART * 32);
         float mu[A], dmu[A];
 #pragma unroll
         for (int j = 0; j < A; ++j) {
@@ -589,17 +587,9 @@ __global__ void __launch_bounds__(NPART * 128 + 32, 1) update_tc_kernel(const __
 
 template <int O, int A>
 static int launch_update_tc(const UpdTcArgs &a, int grid, size_t smem, cudaStream_t st) {
-    static const int nparts = [] {
-        // 2 threads per sample is the default; 4 (TG_UPDATE_TC_PARTS=4) measured the same 4.35-4.39 ms on
-        // Pendulum: the kernel is bound by its instruction count and phase chain, not by warp parallelism
-        const char *e = getenv("TG_UPDATE_TC_PARTS");
-        return (e && e[0] == '4') ? 4 : 2;
-    }();
-    void (*kern)(const UpdTcArgs);
-    if (nparts == 2) kern = a.lay.act == TG_ACT_RELU ? update_tc_kernel<O, A, true, 2> : update_tc_kernel<O, A, false, 2>;
-    else kern = a.lay.act == TG_ACT_RELU ? update_tc_kernel<O, A, true, 4> : update_tc_kernel<O, A, false, 4>;
+    void (*kern)(const UpdTcArgs) = a.lay.act == TG_ACT_RELU ? update_tc_kernel<O, A, true> : update_tc_kernel<O, A, false>;
     TG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<grid, nparts * 128 + 32, smem, st>>>(a);
+    kern<<<grid, NPART * 128 + 32, smem, st>>>(a);
     TG_CUDA(cudaGetLastError());
     return TG_OK;
 }

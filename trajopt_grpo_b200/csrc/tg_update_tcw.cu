@@ -13,7 +13,7 @@
 //       scratch, in the operand layout of kernel B:  H1, H2, dZ1 as fp32 (MN-major SW128_32B, 8-sample
 //       sub-blocks) and Y = [x, 1, dmu] (fp32, K-major).  No column sums over samples are left in this kernel:
 //       round 1 computed dWo = dmu^T . H2 with register butterflies here (187 us of 847 us per 2656-tile batch at
-//       W = 256); dWo is now one more small GEMM of kernel B.
+//       W = 256); dWo moved to kernel B.
 //   kernel B  (update_tcw_wgrad_kernel)   split-K weight-gradient GEMMs over the batch's samples:
 //       dW1 += dZ2^T . H1   and   [dW0 | db0] += dZ1^T . [x, 1]   on the tensor core (fp32 accumulators persistent in tensor
 //       memory for all tiles of the launch, added to the CTA-private gradient copy at the end);
@@ -39,16 +39,6 @@
 #define TCW_BAR_L1 5
 #define TCW_BAR_K0 6
 #define TCW_BAR_K1 7
-
-struct TcwLayout {
-    int O, OKP, A, act, W;
-    int64_t w0hi, w0lo, b1, wo, bo;      // offsets (floats) in the resident block
-    int64_t resident;                     // floats, multiple of 256
-    int64_t chunks_f, chunks_b;           // forward (K-major) / backward (MN-major) chunk streams
-    int64_t chunk_floats;                 // W * 32
-    int64_t total;
-    int64_t flat_w[3], n_params;
-};
 
 struct TcwScratch {                       // per-tile byte strides / bases inside the HBM scratch
     unsigned char *base;
@@ -87,99 +77,6 @@ bool tg_update_tcw_eligible(const tg_mlp_cfg *mlp) {
     const int W = mlp->dims[1];
     return (W == 128 || W == 256) && mlp->dims[2] == W && mlp->dims[0] >= 1 && mlp->dims[0] <= 23 &&
            (mlp->dims[3] == 1 || mlp->dims[3] == 2 || mlp->dims[3] == 4) && mlp->activation >= 0 && mlp->activation <= 2;
-}
-
-static void build_tcw_layout(const tg_mlp_cfg *mlp, TcwLayout *L) {
-    memset(L, 0, sizeof(*L));
-    L->O = mlp->dims[0];
-    L->OKP = (L->O + 1 + 7) / 8 * 8;
-    L->A = mlp->dims[3];
-    L->act = mlp->activation;
-    L->W = mlp->dims[1];
-    const int W = L->W;
-    int64_t off = 0;
-    L->w0hi = off; off += (int64_t)W * L->OKP;
-    L->w0lo = off; off += (int64_t)W * L->OKP;
-    L->b1 = off; off += W;
-    L->wo = off; off += (int64_t)L->A * W;
-    L->bo = off; off += 4;
-    L->resident = (off + 255) / 256 * 256;
-    L->chunk_floats = (int64_t)W * 32;
-    L->chunks_f = L->resident;
-    L->chunks_b = L->chunks_f + (int64_t)(2 * W / 32) * L->chunk_floats;
-    L->total = L->chunks_b + (int64_t)(2 * W / 32) * L->chunk_floats;
-    int64_t flat = 0;
-    for (int l = 0; l < 3; ++l) {
-        L->flat_w[l] = flat;
-        flat += (int64_t)mlp->dims[l] * mlp->dims[l + 1] + mlp->dims[l + 1];
-    }
-    L->n_params = flat;
-}
-
-// the value the tensor core uses for a raw fp32 operand of kind::tf32: the low 13 mantissa bits dropped
-TG_D float tf32_trunc(float x) { return __uint_as_float(__float_as_uint(x) & 0xffffe000u); }
-
-TG_D float tcw_hi(float w) {
-    uint32_t hb;
-    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(hb) : "f"(w));
-    return __uint_as_float(hb & 0xffffe000u);
-}
-TG_D void tcw_core_invert(int C, int64_t idx, int *r, int *c) {
-    const uint32_t b = (uint32_t)idx * 4u;
-    const uint32_t group = (uint32_t)(C >> 2) * 128u;
-    const uint32_t rr = b % group;
-    *r = (int)(b / group) * 8 + (int)((rr % 128u) >> 4);
-    *c = (int)(rr / 128u) * 4 + (int)((rr & 15u) >> 2);
-}
-
-__global__ void pack_tcw_kernel(TcwLayout L, const float *__restrict__ params, float *__restrict__ packed) {
-    const int W = L.W;
-    const float *W0 = params + L.flat_w[0], *b0 = W0 + (int64_t)W * L.O;
-    const float *W1 = params + L.flat_w[1], *b1 = W1 + (int64_t)W * W;
-    const float *Wo = params + L.flat_w[2], *bo = Wo + (int64_t)L.A * W;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < L.total; i += (int64_t)gridDim.x * blockDim.x) {
-        float v = 0.0f;
-        if (i < L.b1) {
-            const bool lo = i >= L.w0lo;
-            int n, c;
-            tcw_core_invert(L.OKP, i - (lo ? L.w0lo : L.w0hi), &n, &c);
-            const float w = c < L.O ? W0[(int64_t)n * L.O + c] : (c == L.O ? b0[n] : 0.0f);
-            const float h = tcw_hi(w);
-            v = lo ? (w - h) : h;
-        } else if (i < L.wo) {
-            v = b1[i - L.b1];
-        } else if (i < L.bo) {
-            v = Wo[i - L.wo];
-        } else if (i < L.bo + L.A) {
-            v = bo[i - L.bo];
-        } else if (i >= L.chunks_f && i < L.chunks_b) {
-            // forward: chunk = (K-chunk kc, hi/lo); [W rows n][32 k] K-major core-matrix layout
-            const int64_t j = i - L.chunks_f;
-            const int chunk = (int)(j / L.chunk_floats);
-            const bool lo = (chunk & 1) != 0;
-            const int kc = chunk >> 1;
-            int n, kk;
-            tcw_core_invert(32, j % L.chunk_floats, &n, &kk);
-            const float w = W1[(int64_t)n * W + kc * 32 + kk];
-            const float h = tcw_hi(w);
-            v = lo ? (w - h) : h;
-        } else if (i >= L.chunks_b) {
-            // backward: chunk = (32 out-rows kc, hi/lo); [32 rows out][W cols in] MN-major SW128_32B (invert mn32_offset)
-            const int64_t j = i - L.chunks_b;
-            const int chunk = (int)(j / L.chunk_floats);
-            const bool lo = (chunk & 1) != 0;
-            const int kc = chunk >> 1;
-            const uint32_t b = (uint32_t)(j % L.chunk_floats) * 4u;
-            const uint32_t blk = b / (32u * 128u), rr = b % (32u * 128u);
-            const int r = (int)(rr / 128u);
-            const int ch = (int)((rr % 128u) >> 5) ^ (r & 3);
-            const int c = (int)blk * 32 + ch * 8 + (int)((rr & 31u) >> 2);
-            const float w = W1[(int64_t)(kc * 32 + r) * W + c];
-            const float h = tcw_hi(w);
-            v = lo ? (w - h) : h;
-        }
-        packed[i] = v;
-    }
 }
 
 // tstart[t] = number of live tiles of steps < t (tile = 128 sorted positions), tstart[T] = total
@@ -222,34 +119,6 @@ TG_D bool tcw_tile_next(const int64_t *__restrict__ tstart, int T, int64_t k, in
 struct TrueTag { static constexpr bool value = true; };
 struct FalseTag { static constexpr bool value = false; };
 
-TG_D void tcw_arrive(int id, int count) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(count) : "memory"); }
-TG_D void tcw_sync(int id, int count) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(count) : "memory"); }
-
-// butterfly column sum: v[0..32) per lane -> the warp's sum over its 32 lanes of entry `lane`
-template <int HALF, int OFF> TG_D void tcw_colsum_step(float *v, int lane) {
-    const bool up = (lane & OFF) != 0;
-#pragma unroll
-    for (int j = 0; j < HALF; ++j) {
-        const float send = up ? v[j] : v[j + HALF];
-        const float keep = up ? v[j + HALF] : v[j];
-        v[j] = keep + __shfl_xor_sync(0xffffffffu, send, OFF);
-    }
-}
-TG_D float tcw_colsum32(float *v, int lane) {
-    tcw_colsum_step<16, 16>(v, lane);
-    tcw_colsum_step<8, 8>(v, lane);
-    tcw_colsum_step<4, 4>(v, lane);
-    tcw_colsum_step<2, 2>(v, lane);
-    tcw_colsum_step<1, 1>(v, lane);
-    return v[0];
-}
-
-// byte offset of (sample s, column c) inside one MN-major scratch array of a tile (8-sample sub-blocks)
-template <int W> TG_D uint32_t tcw_sc_off(int s, int c) {
-    const int r = s & 7;
-    return (uint32_t)(s >> 3) * (uint32_t)(W / 32 * 1024) + (uint32_t)(c >> 5) * 1024u + (uint32_t)r * 128u +
-           (uint32_t)((((c & 31) >> 3) ^ (r & 3)) << 5) + (uint32_t)(c & 7) * 4u;
-}
 // 256-bit global accesses (sm_100): one lane moves a whole 32-byte sector, so the row-per-thread scratch traffic
 // is made of full sectors instead of 16-byte halves
 TG_D void stg256(void *p, const float *v) {
@@ -264,30 +133,6 @@ TG_D void ldg256(const void *p, float *v) {
                  : "memory");
 }
 
-// 32 consecutive columns (column block cbk) of sample s written as fp32 to a scratch array (MN-major sub-block
-// layout; kernel B splits into tf32 hi/lo after its TMA load, which halves the HBM traffic of both kernels)
-template <int W>
-TG_D void tcw_store32(unsigned char *arr, int s, int cbk, const float *v) {
-    const int r = s & 7;
-    unsigned char *p = arr + (size_t)(s >> 3) * (W / 32 * 1024) + (size_t)cbk * 1024 + (size_t)r * 128;
-#pragma unroll
-    for (int c8 = 0; c8 < 4; ++c8)                    // 32-byte chunk (8 columns) c8 of the 128-byte row
-        stg256(p + (uint32_t)((c8 ^ (r & 3)) << 5), v + 8 * c8);
-}
-// 32 columns hi/lo split into the tensor-memory A operand (hi at tm_hi, lo at tm_lo), 16 columns at a time
-TG_D void tcw_tm32(const float *v, uint32_t tm_hi, uint32_t tm_lo) {
-#pragma unroll
-    for (int hh = 0; hh < 2; ++hh) {
-        float hi[16], lo[16];
-#pragma unroll
-        for (int jj = 0; jj < 16; ++jj) {
-            hi[jj] = tf32_hi(v[hh * 16 + jj]);
-            lo[jj] = v[hh * 16 + jj] - hi[jj];
-        }
-        tmem_st16(tm_hi + (uint32_t)(hh * 16), hi);
-        tmem_st16(tm_lo + (uint32_t)(hh * 16), lo);
-    }
-}
 // 16-column pieces (half hh of the 32-column block): the epilogues of kernel A work at this granularity so that a
 // thread holds 16 accumulator values + their hi/lo split (48 registers) instead of 32 + 32 + 32 -- at 96 registers
 // per thread (18 warps) the 32-column form spilled ~0.7 KB per thread
@@ -430,7 +275,7 @@ __global__ void __launch_bounds__(NP * 128 + 64, 1) update_tcw_fwdbwd_kernel(con
         for (int64_t k = a.k_begin + blockIdx.x; k < k_end; k += gridDim.x) {
             if (!(first_tile ? tcw_tile_of(a.tstart, a.T, k, &t, &blk) : tcw_tile_next(a.tstart, a.T, k, &t, &blk))) break;
             first_tile = false;
-            tcw_sync(TCW_BAR_L1, CNT_ALL);
+            named_sync(TCW_BAR_L1, CNT_ALL);
             tc_fence_after();
             {
                 uint32_t acc = 0;
@@ -449,8 +294,8 @@ __global__ void __launch_bounds__(NP * 128 + 64, 1) update_tcw_fwdbwd_kernel(con
             __syncwarp();
             for (int dir = 0; dir < (a.forward_only ? 1 : 2); ++dir) {   // 0: forward (K-major B), 1: backward-data (MN-major B)
                 for (int half = 0; half < KH; ++half) {
-                    if (half == 0) tcw_sync(TCW_BAR_K0, CNT_ALL);
-                    else tcw_sync(TCW_BAR_K1, CNT_H1);
+                    if (half == 0) named_sync(TCW_BAR_K0, CNT_ALL);
+                    else named_sync(TCW_BAR_K1, CNT_H1);
                     tc_fence_after();
                     {
                         for (int c = 0; c < 4; ++c) {
@@ -519,7 +364,7 @@ __global__ void __launch_bounds__(NP * 128 + 64, 1) update_tcw_fwdbwd_kernel(con
         auto finish_A = [&](const unsigned char *arr, bool dz2) {
             if (deferred) {
                 tc_fence_before();
-                tcw_arrive(TCW_BAR_K0, CNT_ALL);
+                named_arrive(TCW_BAR_K0, CNT_ALL);
                 mbar_wait(&bar_k0, ph_k0);
                 tc_fence_after();
 #pragma unroll
@@ -532,8 +377,8 @@ __global__ void __launch_bounds__(NP * 128 + 64, 1) update_tcw_fwdbwd_kernel(con
             ph_k0 ^= 1u;
             tmem_st_wait();
             tc_fence_before();
-            if (deferred) tcw_arrive(TCW_BAR_K1, CNT_H1);
-            else tcw_arrive(TCW_BAR_K0, CNT_ALL);
+            if (deferred) named_arrive(TCW_BAR_K1, CNT_H1);
+            else named_arrive(TCW_BAR_K0, CNT_ALL);
         };
 
         int t = 0, blk = 0;
@@ -572,7 +417,7 @@ __global__ void __launch_bounds__(NP * 128 + 64, 1) update_tcw_fwdbwd_kernel(con
             }
             if (part == 0) fence_proxy_async();       // only these threads wrote the shared-memory obs operand
             tc_fence_before();
-            tcw_arrive(TCW_BAR_L1, CNT_ALL);
+            named_arrive(TCW_BAR_L1, CNT_ALL);
             mbar_wait(&bar_d, ph_d);
             ph_d ^= 1u;
             tc_fence_after();
@@ -650,7 +495,7 @@ __global__ void __launch_bounds__(NP * 128 + 64, 1) update_tcw_fwdbwd_kernel(con
 #pragma unroll
                 for (int jj = 0; jj < A; ++jj) muS[part][jj][e] = pm[jj];
             }
-            tcw_sync(q + 1, NP * 32);
+            named_sync(q + 1, NP * 32);
             if (part == 0) {
                 float mu[A], dmu[A];
 #pragma unroll
@@ -726,7 +571,7 @@ __global__ void __launch_bounds__(NP * 128 + 64, 1) update_tcw_fwdbwd_kernel(con
                 tc_fence_before();
                 continue;
             }
-            tcw_sync(q + 1, NP * 32);
+            named_sync(q + 1, NP * 32);
             // ---- epilogue 2b: H2 -> scratch (kernel B: dWo, and dZ2 rebuilt from it); dZ2 = (Wo^T dmu) * act'(H2) -> A operand
             {
 #pragma unroll
@@ -1192,19 +1037,6 @@ static int launch_tcw(const TcwArgs &a0, int grid, int64_t total_upper, int64_t 
     return launch_tcw_np<O, A, W, (W == 256 ? 4 : 2)>(a0, grid, total_upper, batch_tiles, st);
 }
 
-static int reserve_bytes(void **p, size_t *cap, size_t bytes) {
-    if (bytes <= *cap) return TG_OK;
-    if (*p) {
-        TG_CUDA(cudaDeviceSynchronize());
-        TG_CUDA(cudaFree(*p));
-        *p = nullptr;
-        *cap = 0;
-    }
-    TG_CUDA(cudaMalloc(p, bytes));
-    *cap = bytes;
-    return TG_OK;
-}
-
 // gpart [sm_count][n_params] and spart [sm_count][4] must be zeroed by the caller.
 int tg_policy_grad_tcw(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N, int T, const float *obs, const float *act,
                        const float *adv, const float *old_logp, const float *target, const int32_t *len, const float *params,
@@ -1213,12 +1045,10 @@ int tg_policy_grad_tcw(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N, int T, con
                        float *out_logp) {
     TcwArgs a;
     memset(&a, 0, sizeof(a));
-    build_tcw_layout(mlp, &a.lay);
+    tg_build_tcw_layout(mlp, &a.lay, true);
     const int W = a.lay.W, O = a.lay.O, A = a.lay.A;
-    int rc = reserve_bytes((void **)&ctx->packed_tc, &ctx->packed_tc_cap, (size_t)a.lay.total * 4);
+    int rc = tg_pack_weights_tcw(ctx, a.lay, params, st);
     if (rc) return rc;
-    pack_tcw_kernel<<<296, 256, 0, st>>>(a.lay, params, ctx->packed_tc);
-    TG_CUDA(cudaGetLastError());
     rc = tg_len_order(ctx, N, T, len, st);
     if (rc) return rc;
     // per-tile scratch; batch = as many tiles as fit the budget (a multiple of the grid)
@@ -1236,7 +1066,7 @@ int tg_policy_grad_tcw(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N, int T, con
     if (batch_tiles < grid) batch_tiles = grid;
     if (batch_tiles > total_upper) batch_tiles = (total_upper + grid - 1) / grid * grid;
     const size_t tstart_bytes = ((size_t)(T + 1) * 8 + 255) / 256 * 256;
-    rc = reserve_bytes(&ctx->scratch, &ctx->scratch_cap, tstart_bytes + (size_t)batch_tiles * a.sc.tile_bytes);
+    rc = tg_ctx_grow(ctx, &ctx->scratch, &ctx->scratch_cap, tstart_bytes + (size_t)batch_tiles * a.sc.tile_bytes);
     if (rc) return rc;
     int64_t *tstart = reinterpret_cast<int64_t *>(ctx->scratch);
     a.sc.base = reinterpret_cast<unsigned char *>(ctx->scratch) + tstart_bytes;
@@ -1267,7 +1097,7 @@ extern "C" int tg_policy_grad_scratch_bytes(const tg_ctx *ctx, const tg_mlp_cfg 
     *bytes_written = *bytes_read = 0;
     if (!tg_update_tcw_shape_built(mlp) || ctx->math_mode == TG_MATH_FP32) return TG_OK;
     TcwLayout L;
-    build_tcw_layout(mlp, &L);
+    tg_build_tcw_layout(mlp, &L, true);
     const int64_t arr = (int64_t)16 * (L.W / 32) * 1024, xb = (int64_t)16 * ((L.O + 1 + L.A + 7) / 8 * 8) * 32;
     *bytes_written = n_tiles * (3 * arr + xb);                           // kernel A: H1, H2, dZ1, [x,1,dmu], all fp32
     // kernel B: H2, H1, dZ1 once each; [x,1,dmu] once per launch (two launches at W = 256: dW1 | dW0)
