@@ -377,13 +377,15 @@ def test_large_rollout_properties(E):
 # shards' sums, normalise with the global statistics, gradients scaled by the global step count --
 # the two ranks of a world-size-2 run emulated one after the other on one GPU (SURVEY 8e)
 # ----------------------------------------------------------------------------
-@pytest.mark.parametrize("mode_name", ["mc", "gae"])
-def test_ppo_sharded_equals_single_rollout(E, mode_name):
+@pytest.mark.parametrize("mode_name,width", [pytest.param("mc", 32, id="mc"), pytest.param("gae", 32, id="gae"),
+                                             pytest.param("mc", 128, id="mc-w128"), pytest.param("gae", 128, id="gae-w128")])
+def test_ppo_sharded_equals_single_rollout(E, mode_name, width):
+    """32 wide: FP32-pipe kernels; 128 wide: the streamed tensor-core critic forward and actor / critic gradients."""
     from trajopt_grpo_b200 import _lib as L
     rng = np.random.default_rng(11)
     G, Eg, T, O, A = 6, 8, 20, 10, 2
     N = G * Eg
-    a_dims, c_dims = [O, 32, 32, A], [O, 32, 32, 1]
+    a_dims, c_dims = [O, width, width, A], [O, width, width, 1]
     mk = lambda dims: dev(_flat([(rng.standard_normal((dims[i + 1], dims[i])) / np.sqrt(dims[i])).astype(np.float32)
                                  for i in range(3)], [(0.1 * rng.standard_normal(dims[i + 1])).astype(np.float32) for i in range(3)]))
     a_flat, c_flat = mk(a_dims), mk(c_dims)

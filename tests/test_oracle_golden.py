@@ -158,6 +158,109 @@ def test_grpo_adam_updates_match_reference(golden_dir, name):
             np.testing.assert_allclose(p, g[f"{key}{i}"], rtol=1e-4, atol=2e-6)
 
 
+PPO_FIXTURES = ["ppo_mc_quadpole2d", "ppo_gae_quadpole2d", "ppo_mc_ragged_quadpole2d", "ppo_gae_ragged_quadpole2d",
+                "ppo_mc_quadpole2d_shipped", "ppo_gae_cartpole_shipped"]
+
+
+def _ppo_setup(g):
+    """Actor / critic weights and the start-of-learn() quantities of PPO.learn (ppo.py:85-143) in float32."""
+    import torch
+    Ws, bs = _weights(g)
+    cWs, cbs = _weights(g, "c")
+    kind = int(g["kind"])
+    cov = np.full(R.ACT_DIM[kind], g["cov"], np.float32)
+    t = lambda x: torch.tensor(np.asarray(x))
+    with torch.no_grad():
+        values = R._torch_mlp(t(g["obs"]), [t(w) for w in cWs], [t(b) for b in cbs], R.ACT_RELU)[..., 0].numpy()
+        old_logp = R._torch_logp(R._torch_mlp(t(g["obs"]), [t(w) for w in Ws], [t(b) for b in bs], R.ACT_RELU),
+                                 t(cov), t(g["act"])).numpy()
+    return Ws, bs, cWs, cbs, cov, values, old_logp
+
+
+def _pairs(flat, shapes):
+    out, off = [], 0
+    for s in shapes:
+        n = int(np.prod(s))
+        out.append(flat[off:off + n].reshape(s))
+        off += n
+    return out
+
+
+@pytest.mark.parametrize("name", PPO_FIXTURES)
+def test_ppo_restatement_matches_reference(golden_dir, name):
+    """R.ppo_advantages + R.ppo_objective_and_grad in float32 against PPO.learn full batch: one SGD(lr=1) update
+    (the gradient) and three Adam updates with the old log-probs fixed at the start of learn() (ppo.py:142-143)."""
+    g = load(golden_dir, f"{name}.npz")
+    Ws, bs, cWs, cbs, cov, values, old_logp = _ppo_setup(g)
+    mask = g["mask"]
+    _, _, adv, ret = R.ppo_advantages(g["rew"], mask, values, float(g["gamma"]), float(g["lam"]),
+                                      bool(g["monte_carlo"]))
+    shapes = [p.shape for wb in zip(Ws, bs) for p in wb] + [p.shape for wb in zip(cWs, cbs) for p in wb]
+    params = [p.copy() for wb in zip(Ws, bs) for p in wb] + [p.copy() for wb in zip(cWs, cbs) for p in wb]
+    na = 2 * len(Ws)
+    m = [np.zeros_like(p) for p in params]
+    v = [np.zeros_like(p) for p in params]
+    for step in range(1, 4):
+        o = R.ppo_objective_and_grad(g["obs"], g["act"], adv, ret, mask, params[0:na:2], params[1:na:2],
+                                     params[na::2], params[na + 1::2], old_logp, cov, float(g["eps_clip"]), 0.5, 0.5,
+                                     dtype="float32")
+        grads = _pairs(np.concatenate([o["actor_grad"], o["critic_grad"]]), shapes)
+        if step == 1:
+            assert o["n"] == int(mask.sum())
+            for i, gr in enumerate(grads):
+                ref = g[f"ppo_grad{i}"]
+                assert np.abs(gr - ref).max() <= 2e-4 * max(np.abs(ref).max(), 1e-6) + 1e-5, (i, np.abs(gr - ref).max())
+        params = R.adam_step(params, grads, m, v, step, 2e-4)
+    for i, p in enumerate(params):
+        np.testing.assert_allclose(p, g[f"ppo_adam3_p{i}"], rtol=1e-4, atol=2e-6, err_msg=str(i))
+
+
+def test_ppo_minibatch_restatement_matches_reference(golden_dir):
+    """batch_size=64: one torch.randperm over the valid rows per epoch, drawn from torch's default generator seeded
+    right before learn() (ppo.py:147-157), the rows in the reference's flattening order (env-major, step-minor), each
+    minibatch's means over its own rows, one Adam step per minibatch."""
+    import torch
+    g = load(golden_dir, "ppo_minibatch_quadpole2d.npz")
+    Ws, bs, cWs, cbs, cov, values, old_logp = _ppo_setup(g)
+    mask = g["mask"]
+    _, _, adv, ret = R.ppo_advantages(g["rew"], mask, values, float(g["gamma"]), float(g["lam"]),
+                                      bool(g["monte_carlo"]))
+    sel = mask > 0
+    rows = {k: np.asarray(x)[sel] for k, x in (("obs", g["obs"]), ("act", g["act"]), ("adv", adv), ("ret", ret),
+                                                ("olp", old_logp))}
+    n, bsz = int(sel.sum()), int(g["batch_size"])
+    shapes = [p.shape for wb in zip(Ws, bs) for p in wb] + [p.shape for wb in zip(cWs, cbs) for p in wb]
+    params = [p.copy() for wb in zip(Ws, bs) for p in wb] + [p.copy() for wb in zip(cWs, cbs) for p in wb]
+    na = 2 * len(Ws)
+    m = [np.zeros_like(p) for p in params]
+    v = [np.zeros_like(p) for p in params]
+    step = 0
+    torch.manual_seed(int(g["torch_seed"]))
+    for _ in range(int(g["updates"])):
+        perm = torch.randperm(n).numpy()
+        for s in range(0, n, bsz):
+            idx = perm[s:s + bsz]
+            o = R.ppo_objective_and_grad(rows["obs"][idx], rows["act"][idx], rows["adv"][idx], rows["ret"][idx],
+                                         np.ones(idx.size), params[0:na:2], params[1:na:2], params[na::2],
+                                         params[na + 1::2], rows["olp"][idx], cov, float(g["eps_clip"]), 0.5, 0.5,
+                                         dtype="float32")
+            step += 1
+            params = R.adam_step(params, _pairs(np.concatenate([o["actor_grad"], o["critic_grad"]]), shapes), m, v,
+                                 step, 2e-4)
+    for i, p in enumerate(params):
+        np.testing.assert_allclose(p, g[f"ppo_mb_adam_p{i}"], rtol=1e-4, atol=2e-6, err_msg=str(i))
+
+
+def test_gae_gamma_lambda_is_one_rounded_scalar():
+    """The GAE recurrence multiplies by fp32(gamma*lam) (the float64 product, ppo.py:123), which for 0.99 / 0.99
+    differs from fp32(0.99)*fp32(0.99): a restatement that rounds the factors separately disagrees in the last bit."""
+    assert np.float32(0.99 * 0.99) != np.float32(0.99) * np.float32(0.99)
+    rew = np.array([[0.0, 0.0, 1.0]], np.float32)
+    adv, _ = R.gae(rew, np.ones_like(rew), np.zeros_like(rew), 0.99, 0.99)
+    f = np.float32(0.99 * 0.99)
+    assert adv[0, 0] == f * (f * np.float32(1.0))
+
+
 def test_rtg_reference_example():
     # the one numeric expectation the reference's tests hold (tests/test_rollout_buffer.py:78-92),
     # evaluated in floating point (its expected array is int-typed, SURVEY section 4)
