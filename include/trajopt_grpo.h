@@ -308,6 +308,24 @@ int tg_value_grad_batch(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N, int T, co
                         const int64_t *sample_ids, int64_t n_samples, const float *params, float scale,
                         float *out_grad, float *out_stats, void *workspace, void *stream);
 
+/* Minibatch plan of one PPO epoch (algorithms/ppo.py:147-157) over a rollout sharded by whole groups.
+ *   perm [n_total] int64 (device): the epoch's torch.randperm over the valid steps of the WHOLE rollout,
+ *        in the reference's flattening order (global env index major, step minor)
+ *   len [N] int32, row0 [N] int64 = exclusive prefix sum of len (as tg_export_trajectory): the shard's local
+ *        valid step row0[n] + t is step t of env n
+ *   base: global index of this shard's first valid step; n_local = sum(len)
+ *   -> out_ids [max_ids] int64: flat slot ids t*N + n of the perm entries in [base, base + n_local), in perm order
+ *      out_offsets [n_batches + 1] int64, n_batches = ceil(n_total / batch_size):
+ *      out_offsets[b] = number of this shard's entries in perm[0 : b*batch_size]
+ *      (minibatch b = out_ids[out_offsets[b] : out_offsets[b+1]]).  No write at or past out_ids[max_ids];
+ *      out_offsets still counts every entry, so the caller detects a perm that is not a permutation.
+ *   workspace: tg_minibatch_plan_workspace_bytes(n_total) bytes of device scratch (8 per perm entry + 8 per 4096)
+ * Deterministic: positions come from per-chunk counts and their prefix sum, never from atomics. */
+int64_t tg_minibatch_plan_workspace_bytes(int64_t n_total);
+int tg_minibatch_plan(tg_ctx *ctx, int64_t N, const int32_t *len, const int64_t *row0, const int64_t *perm,
+                      int64_t n_total, int64_t batch_size, int64_t base, int64_t n_local, int64_t max_ids,
+                      int64_t *out_ids, int64_t *out_offsets, void *workspace, void *stream);
+
 /* ---- Adam --------------------------------------------------------------------
  * torch.optim.Adam defaults as the reference constructs it
  * (pipelines/cartpole_pipeline_grpo.py:65): p -= lr/(1-b1^t) * m/(sqrt(v)/sqrt(1-b2^t)+eps).

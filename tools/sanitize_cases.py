@@ -84,6 +84,35 @@ def case_ppo(N=70, T=9):
     torch.cuda.synchronize()
 
 
+def case_ppo_shard(T=11):
+    """Minibatch plans of a ragged rollout (N = 70, lengths 1..T) split into 1, 2 and 3 emulated ranks of uneven
+    size, then the batch gradients on every planned minibatch of each rank."""
+    rng = np.random.default_rng(2)
+    a_dims, c_dims = [10, 32, 32, 2], [10, 32, 32, 1]
+    pa, pc = policy(rng, a_dims), policy(rng, c_dims)
+    N = 70
+    lens = torch.from_numpy(rng.integers(1, T + 1, N).astype(np.int32)).cuda()
+    obs = torch.randn(T, 10, N, device="cuda")
+    act = torch.randn(T, 2, N, device="cuda")
+    adv, olp, rtg = (torch.randn(T, N, device="cuda") for _ in range(3))
+    n = int(lens.sum())
+    perm = torch.randperm(n, generator=torch.Generator().manual_seed(3)).cuda()
+    for cuts in ((0, N), (0, 33, N), (0, 5, 48, N)):
+        base = 0
+        for e0, e1 in zip(cuts[:-1], cuts[1:]):
+            ln = lens[e0:e1].contiguous()
+            ids, offs = E.minibatch_plan(perm, ln, 37, base)
+            base += int(ln.sum())
+            o, a = obs[..., e0:e1].contiguous(), act[..., e0:e1].contiguous()
+            ad, lp, rt = (x[:, e0:e1].contiguous() for x in (adv, olp, rtg))
+            for b in range(len(offs) - 1):
+                sid = ids[offs[b]:offs[b + 1]]
+                if sid.numel():
+                    E.policy_grad_batch(a_dims, "ReLU", pa, [0.3, 0.3], o, a, ad, lp, sid, 0.2, -1.0 / 37, 0.5 / 37)
+                    E.value_grad_batch(c_dims, "ReLU", pc, o, rt, sid, 0.5 / 37)
+    torch.cuda.synchronize()
+
+
 def case_env():
     for kind in range(4):
         s = init_state(kind, 33).double()
@@ -102,6 +131,7 @@ CASES = {
     "tc128": lambda: case_rollout_update(2, [128, 128], 200, 6, "3xtf32"),
     "tc256": lambda: case_rollout_update(3, [256, 256], 200, 6, "3xtf32"),
     "ppo": case_ppo,
+    "ppo_shard": case_ppo_shard,
     "env": case_env,
 }
 

@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(CSRC, "obj")
 LIB = os.path.join(HERE, "libtrajopt_grpo_b200.so")
-SOURCES = ["tg_api.cu", "tg_rollout.cu", "tg_rollout_tc256.cu", "tg_advantage.cu", "tg_update.cu", "tg_update_tc.cu", "tg_update_tcw.cu", "tg_order.cu", "tg_export.cu", "tg_selftest.cu", "tg_env_dynamics.cu", "tg_comm.cu"]
+SOURCES = ["tg_api.cu", "tg_rollout.cu", "tg_rollout_tc256.cu", "tg_advantage.cu", "tg_update.cu", "tg_update_tc.cu", "tg_update_tcw.cu", "tg_order.cu", "tg_export.cu", "tg_minibatch.cu", "tg_selftest.cu", "tg_env_dynamics.cu", "tg_comm.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr", "-Xptxas", "-v"]
 

@@ -79,6 +79,8 @@ _SIGS = {
                                        C.POINTER(_f), _f, _f, _f, _vp, _vp, _vp, _vp]),
     "tg_value_grad_batch": (C.c_int, [_vp, C.POINTER(MlpCfg), _i64, _i32, _vp, _vp, _vp, _i64, _vp, _f, _vp, _vp, _vp,
                                       _vp]),
+    "tg_minibatch_plan_workspace_bytes": (_i64, [_i64]),
+    "tg_minibatch_plan": (C.c_int, [_vp, _i64, _vp, _vp, _vp, _i64, _i64, _i64, _i64, _i64, _vp, _vp, _vp, _vp]),
     "tg_adam_step": (C.c_int, [_vp, _i64, _vp, _vp, _vp, _vp, _i64, _d, _d, _d, _d, _vp]),
     "tg_comm_handle_bytes": (C.c_int, []),
     "tg_comm_create": (C.c_int, [_vp, _i32, _i32, _i64, C.POINTER(_vp), _vp]),

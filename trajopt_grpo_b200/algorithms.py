@@ -365,8 +365,11 @@ class GRPO(Algorithm):
 
 
 class PPO(Algorithm):
-    """algorithms/ppo.py:8-225: full-batch updates (batch_size=None, the shipped pipelines' setting; shards over
-    GPUs) and randperm minibatches (batch_size=k, single GPU)."""
+    """algorithms/ppo.py:8-225: full-batch updates (batch_size=None, the shipped pipelines' setting) and randperm
+    minibatches (batch_size=k, the constructor's default).  Both shard over GPUs (RolloutManager(rank=, world_size=)):
+    for minibatches, rank 0 draws the epoch's torch.randperm from its default CPU generator and broadcasts it, every
+    rank computes the gradient of its own samples of each minibatch scaled by the global 1/len(batch), and the ranks
+    sum their gradients before each Adam step -- the single-GPU minibatch step up to fp32 summation order."""
 
     def __init__(self, epsilon: float, policy, optimizer, ref_model, updates_per_iter: int, c1: float = 0.5,
                  kl_coeff: float = 0.5, gamma: float = 0.99, lam: float = 0.95, entropy: float = 0.01,
@@ -382,9 +385,6 @@ class PPO(Algorithm):
 
     def learn(self, buffer) -> None:
         world = _dist_world()
-        if self.batch_size is not None and world > 1:
-            # ppo.py:149 draws ONE torch.randperm over all valid steps; it has no sharded equivalent (SURVEY 8e)
-            raise L.EngineError("minibatched PPO (batch_size != None) runs on one GPU; use batch_size=None when sharded")
         r = _rollout_of(buffer)
         pol = self.policy
         flat = pol.flat_parameters()
@@ -408,9 +408,10 @@ class PPO(Algorithm):
         _, old_logp = engine.policy_forward_traj(a_dims, act_name, a_flat, r.obs, cov, r.act, r.len)
         n_valid = int(round(float(sums[4].item())))                 # global valid-step count (the .mean()s)
         grad = torch.empty_like(flat)
-        comm = self._flat_opt.peer_comm(flat) if (world > 1 and self.batch_size is None) else None
+        comm = self._flat_opt.peer_comm(flat) if world > 1 else None
         if self.batch_size is not None:
-            self._learn_minibatched(r, flat, grad, na, a_dims, c_dims, act_name, cov, adv, rtg, old_logp, n_valid)
+            self._learn_minibatched(r, flat, grad, comm, world, na, a_dims, c_dims, act_name, cov, adv, rtg, old_logp,
+                                    n_valid)
             self.old_policy.load_state_dict(self.policy.state_dict())   # ppo.py:186
             return
         with engine.length_order(r.len, r.T):
@@ -433,30 +434,63 @@ class PPO(Algorithm):
                 self.last_stats = stats
         self.old_policy.load_state_dict(self.policy.state_dict())   # ppo.py:186
 
-    def _learn_minibatched(self, r, flat, grad, na, a_dims, c_dims, act_name, cov, adv, rtg, old_logp, n_valid):
+    def _learn_minibatched(self, r, flat, grad, comm, world, na, a_dims, c_dims, act_name, cov, adv, rtg, old_logp,
+                           n_valid):
         """ppo.py:147-183 with batch_size != None: one `torch.randperm(data_size)` per epoch from torch's
         default CPU generator (the reference's call, so a seeded run draws the same permutation), sliced
         into minibatches over the valid steps in the reference's flattening order (env-major, step-minor);
-        one Adam step per minibatch.  Each minibatch is a list of flat slot ids for the *_batch kernels."""
+        one Adam step per minibatch.  tg_minibatch_plan turns the permutation into this rank's flat slot ids
+        for the *_batch kernels, grouped by minibatch.
+
+        Sharded, rank r owns the global valid steps [base_r, base_r + n_r) (whole groups, ranks in order).  Rank 0
+        draws the permutation and broadcasts it; the other ranks leave their generators alone.  Each rank computes
+        the gradient of its own samples of minibatch b with the global 1/m_b (a rank without samples contributes
+        zeros) and the ranks sum their gradients, so every rank takes the same Adam step."""
         a_flat, c_flat = flat[:na], flat[na:]
         dev = flat.device
-        lens = r.len.to(torch.int64)
-        csum = torch.cumsum(lens, 0)
-        row0 = csum - lens
+        bs = self.batch_size
+        if world > 1:
+            import torch.distributed as dist
+            n_loc = r.len.sum(dtype=torch.int64).reshape(1)
+            counts = [torch.empty_like(n_loc) for _ in range(world)]
+            dist.all_gather(counts, n_loc)
+            counts = [int(c.item()) for c in counts]
+            if sum(counts) != n_valid:
+                raise L.EngineError(f"ranks hold {counts} valid steps, {sum(counts)} in all; the advantage sums "
+                                    f"counted {n_valid}")
+            rank = dist.get_rank()
+            base, n_local = sum(counts[:rank]), counts[rank]
+        else:
+            base, n_local = 0, n_valid
         for _ in range(self.updates_per_iter):
-            permutation = torch.randperm(n_valid)                   # ppo.py:149
-            perm_d = permutation.to(dev)
-            n_of = torch.searchsorted(csum, perm_d, right=True)     # valid-step index k -> env n, step t
-            sid_all = ((perm_d - row0[n_of]) * r.N + n_of).contiguous()
-            for start in range(0, n_valid, self.batch_size):        # ppo.py:152-153
-                sid = sid_all[start:start + self.batch_size]
-                m = sid.numel()
-                _, stats = engine.policy_grad_batch(a_dims, act_name, a_flat, cov, r.obs, r.act, adv, old_logp, sid,
-                                                    self.epsilon, -1.0 / m, self.kl_coeff / m, out_grad=grad[:na])
-                engine.value_grad_batch(c_dims, act_name, c_flat, r.obs, rtg, sid, self.c1 / m, out_grad=grad[na:])
-                self._flat_opt.step(flat, grad)
+            if world > 1:
+                perm = torch.randperm(n_valid).to(dev) if rank == 0 else \
+                    torch.empty((n_valid,), dtype=torch.int64, device=dev)
+                dist.broadcast(perm, 0)
+            else:
+                perm = torch.randperm(n_valid).to(dev)              # ppo.py:149
+            ids, offsets = engine.minibatch_plan(perm, r.len, bs, base, n_local=n_local)
+            del perm                                                # 8 bytes per valid step of the whole rollout
+            offsets = offsets.tolist()
+            for b in range(len(offsets) - 1):                       # ppo.py:152-153
+                m = min(bs, n_valid - b * bs)                       # the reference's .mean() over the batch
+                g = comm.grad_slot()[:flat.numel()] if comm is not None else grad
+                if offsets[b + 1] > offsets[b]:
+                    sid = ids[offsets[b]:offsets[b + 1]]
+                    _, stats = engine.policy_grad_batch(a_dims, act_name, a_flat, cov, r.obs, r.act, adv, old_logp,
+                                                        sid, self.epsilon, -1.0 / m, self.kl_coeff / m,
+                                                        out_grad=g[:na])
+                    engine.value_grad_batch(c_dims, act_name, c_flat, r.obs, rtg, sid, self.c1 / m, out_grad=g[na:])
+                    self.last_stats = stats
+                else:
+                    g.zero_()                                       # no samples here: still part of the sum
+                if comm is not None:
+                    self._flat_opt.step_allreduced(flat, comm)
+                else:
+                    if world > 1:
+                        dist.all_reduce(g)
+                    self._flat_opt.step(flat, g)
                 self.policy.bump_param_epoch()
-                self.last_stats = stats
 
     def metadata(self) -> dict:
         return {"algorithm": "PPO", "epsilon": self.epsilon, "c1": self.c1, "kl_coeff": self.kl_coeff,

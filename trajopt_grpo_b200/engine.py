@@ -424,6 +424,45 @@ def value_grad(dims, activation, params, obs, target, length, scale, out_grad=No
     return grad, stats
 
 
+def minibatch_plan(perm, length, batch_size, base, n_local=None):
+    """tg_minibatch_plan: this shard's part of every minibatch of one PPO epoch.
+
+    perm [n_total] int64 (device): the epoch's permutation of the valid steps of the WHOLE rollout (global env index
+    major, step minor); length [N] int32: this shard's episode lengths; base: global index of its first valid step.
+    `n_local` (= length.sum()) may be passed when the caller knows it, which saves a device-to-host copy.
+    Returns (ids [n_local] int64 device: flat slot ids t*N + n in perm order, offsets [n_batches + 1] int64 host):
+    minibatch b of this shard is ids[offsets[b]:offsets[b + 1]].  Raises EngineError unless the plan holds exactly
+    n_local entries (perm is not a permutation of range(n_total))."""
+    lib = L.load()
+    _need(perm, torch.int64, "perm")
+    _need(length, torch.int32, "len")
+    if perm.dim() != 1 or length.dim() != 1 or perm.numel() == 0 or length.numel() == 0:
+        raise L.EngineError("perm and len must be non-empty 1-d tensors")
+    if int(batch_size) <= 0:
+        raise L.EngineError(f"batch_size must be positive, got {batch_size}")
+    dev = perm.device
+    n_total, N = perm.numel(), length.numel()
+    row0 = torch.cumsum(length.to(torch.int64), 0)
+    if n_local is None:
+        n_local = int(row0[-1].item())
+    row0.sub_(length)
+    n_batches = -(-n_total // int(batch_size))
+    ids = torch.empty((int(n_local),), dtype=torch.int64, device=dev)
+    offsets = torch.empty((n_batches + 1,), dtype=torch.int64, device=dev)
+    ws = _workspace("plan", lib.tg_minibatch_plan_workspace_bytes(n_total), dev)
+    with torch.cuda.device(dev):
+        rc = lib.tg_minibatch_plan(L.ctx(dev), N, L.ptr(length), L.ptr(row0), L.ptr(perm), n_total, int(batch_size),
+                                   int(base), int(n_local), ids.numel(), L.ptr(ids), L.ptr(offsets), L.ptr(ws),
+                                   L.stream_ptr())
+    L.check(rc, "tg_minibatch_plan")
+    _count(3)
+    offsets = offsets.cpu()
+    if int(offsets[-1]) != int(n_local):
+        raise L.EngineError(f"tg_minibatch_plan: {int(offsets[-1])} entries of perm fall in this shard's "
+                            f"{int(n_local)} valid steps: perm is not a permutation of range({n_total})")
+    return ids, offsets
+
+
 def adam_step(params, grad, exp_avg, exp_avg_sq, step, lr, beta1=0.9, beta2=0.999, eps=1e-8):
     lib = L.load()
     for t, nm in ((params, "params"), (grad, "grad"), (exp_avg, "exp_avg"), (exp_avg_sq, "exp_avg_sq")):
