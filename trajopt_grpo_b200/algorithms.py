@@ -280,8 +280,6 @@ class GRPO(Algorithm):
         One trajectory buffer of chunk size is reused.  With updates_per_iter == 1 no work is repeated.
         Equal to sample() + learn() on the same seed up to the fp32 summation order of the per-chunk gradients.
         Returns the number of valid env-steps of this rank's rollout as a 0-dim CUDA tensor (no host sync)."""
-        from .rollout import shard_initial_states
-        import numpy as np
         pol = self.policy
         self._resync_after_checkpoint_load()
         flat = pol.flat_parameters()
@@ -293,12 +291,7 @@ class GRPO(Algorithm):
         G_loc = manager.local_workers
         world = _dist_world()
         dev = flat.device
-        if init_state is None:
-            blk = shard_initial_states(env, manager.num_workers, E, manager.restart, manager._rng, manager.rank,
-                                       manager.world_size)
-            init_state = torch.from_numpy(np.ascontiguousarray(blk.T)).to(torch.float32).pin_memory().to(dev, non_blocking=True)
-        seed = (manager._seed + 0x9E3779B97F4A7C15 * (manager._epoch + 1)) & (2 ** 64 - 1)
-        manager._epoch += 1
+        init_state, seed = manager.next_epoch(init_state, dtype=torch.float32)
         scale = (-1.0 if self.maximize else 1.0) / (G_loc * world)
         n_valid = torch.zeros((), dtype=torch.int64, device=dev)
         ret_sum = torch.zeros((), dtype=torch.float64, device=dev)
@@ -491,6 +484,135 @@ class PPO(Algorithm):
                         dist.all_reduce(g)
                     self._flat_opt.step(flat, g)
                 self.policy.bump_param_epoch()
+
+    def learn_streamed(self, manager, init_state=None, chunk_groups: int = 8192):
+        """One whole full-batch epoch -- rollout AND learn -- for more envs than the rollout fits in HBM, with the
+        contract of GRPO.learn_streamed: only the initial states and the Philox seed are kept, the rollout is
+        rematerialised chunk by chunk (`chunk_groups` whole groups) under the weights of the start of the epoch.
+
+        PPO z-scores advantages and returns over the WHOLE rollout before the first gradient (ppo.py:127-139), so the
+        epoch is one statistics pass followed by one pass per update:
+
+            statistics:  per chunk: K1 -> critic values -> raw K2; the five float64 sums added up
+                         [40-byte allreduce]; the global valid-step count read once
+            each update: per chunk: K1 -> critic values -> raw K2 -> z-score with the global sums
+                                    -> old log-probs -> actor + critic K3, accumulated into one gradient
+                         [gradient exchange]  Adam
+
+        The rematerialisations (rollout, values, old log-probs) use a copy of the flat parameters taken at the
+        start; only the gradients see the live weights.  One chunk-sized set of buffers is reused throughout.  An
+        epoch costs updates_per_iter + 1 rollouts and critic forwards, and updates_per_iter actor forwards and
+        gradients.  With one chunk it trains bit-identically to sample() + learn(); with several, up to the fp32
+        order in which the chunks' gradients are summed.  `last_stats` holds the actor statistics of the last update
+        summed over the chunks.  The update passes z-score with the global sums of the statistics pass; the sums
+        that K2 returns with each rematerialised chunk's raw advantages are a by-product and go unused.  Full batch
+        only (batch_size=None): a randperm minibatch draws from every chunk.  `init_state`, when given, is this rank's
+        [S, local envs] float32 / float64 tensor on the policy's device.
+        Returns the number of valid env-steps of this rank's rollout as a 0-dim CUDA tensor (no host sync)."""
+        if self.batch_size is not None:
+            raise L.EngineError(f"PPO.learn_streamed needs batch_size=None (got {self.batch_size}): every minibatch "
+                                "would need the whole rollout rematerialised")
+        if chunk_groups < 1:
+            raise L.EngineError(f"chunk_groups must be positive, got {chunk_groups}")
+        import math
+        world = _dist_world()
+        pol = self.policy
+        flat = pol.flat_parameters()
+        na = pol.actor.n_params()
+        a_flat, c_flat = flat[:na], flat[na:]
+        a_dims, c_dims, act_name, cov = pol.actor.dims, pol.critic.dims, pol.actor.activation_name, pol.cov_diag
+        env, E, G_loc = manager.env, manager.num_episodes_per_worker, manager.local_workers
+        T, O, A = int(env.max_steps), a_dims[0], a_dims[-1]
+        mode = L.ADV_PPO_MC if self.monte_carlo else L.ADV_PPO_GAE
+        dev = flat.device
+        kind = getattr(env, "_tg_kind", -1)
+        if kind < 0:
+            raise L.EngineError(f"{type(env).__name__} has no fused kernel (supported: CartPole, Pendulum, "
+                                "QuadPole2D, QuadPole)")
+        if init_state is not None:                                  # every chunk is a column slice of it
+            want = (engine.OBS_DIM[kind], G_loc * E)
+            if not (isinstance(init_state, torch.Tensor) and init_state.device == dev
+                    and init_state.dtype in (torch.float32, torch.float64) and tuple(init_state.shape) == want):
+                got = (f"{init_state.dtype} {tuple(init_state.shape)} on {init_state.device}"
+                       if isinstance(init_state, torch.Tensor) else type(init_state).__name__)
+                raise L.EngineError(f"init_state must be a float32 or float64 tensor of shape {want} (this rank's "
+                                    f"envs) on {dev}, got {got}")
+        init_state, seed = manager.next_epoch(init_state)
+        frozen = flat.clone()                                       # the actor and critic of the start of learn()
+        fa, fc = frozen[:na], frozen[na:]
+        chunks = [(g0, min(G_loc, g0 + chunk_groups)) for g0 in range(0, G_loc, chunk_groups)]
+
+        def shapes(n):
+            return {"obs": (T, O, n), "act": (T, A, n), "rew": (T, n), "len": (n,), "ret": (n,), "val": (T, 1, n),
+                    "adv": (T, n), "rtg": (T, n), "old_logp": (T, n)}
+
+        n_max = (chunks[0][1] - chunks[0][0]) * E
+        store = {k: torch.empty(math.prod(s), dtype=torch.int32 if k == "len" else torch.float32, device=dev)
+                 for k, s in shapes(n_max).items()}
+
+        def rematerialise(g0, g1):
+            """K1, critic values and raw K2 of local groups [g0, g1) under the frozen weights -> (buffers, sums)."""
+            n0, n = g0 * E, (g1 - g0) * E
+            c = {k: store[k][:math.prod(s)].view(s) for k, s in shapes(n).items()}
+            roll = {k: c[k] for k in ("obs", "act", "rew", "len", "ret")}
+            s0 = init_state[:, n0:n0 + n].contiguous()
+            out = engine.rollout(kind, T, env.timestep, a_dims, act_name, fa, cov, s0, seed=seed,
+                                 env_offset=manager.env_offset + n0, phys=getattr(env, "_tg_phys", None), out=roll)
+            if out is not roll:                                     # the kernels below read the chunk buffers
+                raise L.EngineError("the rollout did not write the chunk buffers")
+            engine.policy_forward_traj(c_dims, act_name, fc, c["obs"], None, None, c["len"], want_mu=True,
+                                       want_logp=False, out_mu=c["val"])
+            _, _, sums = engine.advantage_ppo_raw(mode, g1 - g0, E, T, self.gamma, self.lam, c["rew"], c["len"],
+                                                  c["val"].view(T, n), out_adv=c["adv"], out_rtg=c["rtg"])
+            return c, sums
+
+        # statistics pass (ppo.py:127-139 over the whole rollout)
+        n_valid = torch.zeros((), dtype=torch.int64, device=dev)
+        ret_sum = torch.zeros((), dtype=torch.float64, device=dev)
+        sums = None
+        for g0, g1 in chunks:
+            c, s = rematerialise(g0, g1)
+            sums = s if sums is None else sums.add_(s)
+            n_valid.add_(c["len"].sum())
+            ret_sum.add_(c["ret"].sum(dtype=torch.float64))
+        if world > 1:
+            import torch.distributed as dist
+            dist.all_reduce(sums)
+        n = int(round(float(sums[4].item())))                       # global valid-step count (the .mean()s)
+
+        grad_own = torch.empty_like(flat)
+        grad_part = torch.empty_like(flat) if len(chunks) > 1 else None
+        comm = self._flat_opt.peer_comm(flat) if world > 1 else None
+        for _ in range(self.updates_per_iter):                      # ppo.py:147 (full batch)
+            grad = comm.grad_slot()[:flat.numel()] if comm is not None else grad_own
+            stats = None
+            for g0, g1 in chunks:
+                c, _ = rematerialise(g0, g1)
+                engine.advantage_ppo_normalize(T, c["len"], sums, c["adv"], c["rtg"])
+                g = grad if g0 == 0 else grad_part                  # the first chunk writes the sum's first term
+                with engine.length_order(c["len"], T):              # one length order for the chunk's forward + K3s
+                    engine.policy_forward_traj(a_dims, act_name, fa, c["obs"], cov, c["act"], c["len"],
+                                               out_logp=c["old_logp"])
+                    _, st = engine.policy_grad(a_dims, act_name, a_flat, cov, c["obs"], c["act"], c["adv"],
+                                               c["old_logp"], c["len"], self.epsilon, -1.0 / n, self.kl_coeff / n,
+                                               out_grad=g[:na])
+                    engine.value_grad(c_dims, act_name, c_flat, c["obs"], c["rtg"], c["len"], self.c1 / n,
+                                      out_grad=g[na:])
+                if g0 != 0:
+                    grad.add_(grad_part)
+                stats = st if stats is None else stats.add_(st)
+            if comm is not None:
+                self._flat_opt.step_allreduced(flat, comm)
+            else:
+                if world > 1:
+                    import torch.distributed as dist
+                    dist.all_reduce(grad)
+                self._flat_opt.step(flat, grad)
+            pol.bump_param_epoch()
+            self.last_stats = stats
+        self.old_policy.load_state_dict(self.policy.state_dict())   # ppo.py:186
+        self.last_mean_return = ret_sum / (G_loc * E)
+        return n_valid
 
     def metadata(self) -> dict:
         return {"algorithm": "PPO", "epsilon": self.epsilon, "c1": self.c1, "kl_coeff": self.kl_coeff,

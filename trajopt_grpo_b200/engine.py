@@ -203,9 +203,10 @@ def policy_forward(dims, activation, params, x, cov_diag=None, act=None, want_mu
 
 
 def policy_forward_traj(dims, activation, params, obs, cov_diag=None, act=None, length=None, want_mu=False,
-                        want_logp=True):
+                        want_logp=True, out_mu=None, out_logp=None):
     """tg_policy_forward_traj.  obs [T,O,N] (+ act [T,A,N]) -> (mu [T,A,N] | None, logp [T,N] | None);
-    rows past `length` are left unwritten."""
+    rows past `length` are left unwritten: zero in the tensors allocated here, unchanged in `out_mu` / `out_logp`
+    (given, they are written in place and imply want_mu / want_logp)."""
     lib = L.load()
     _need(obs, torch.float32, "obs")
     T, O, N = obs.shape
@@ -216,8 +217,14 @@ def policy_forward_traj(dims, activation, params, obs, cov_diag=None, act=None, 
         _need(act, torch.float32, "act", (T, A, N))
     if length is not None:
         _need(length, torch.int32, "len", (N,))
-    mu = torch.zeros((T, A, N), dtype=torch.float32, device=dev) if want_mu else None
-    logp = torch.zeros((T, N), dtype=torch.float32, device=dev) if want_logp else None
+    if out_mu is not None:
+        mu = _need(out_mu, torch.float32, "out_mu", (T, A, N))
+    else:
+        mu = torch.zeros((T, A, N), dtype=torch.float32, device=dev) if want_mu else None
+    if out_logp is not None:
+        logp = _need(out_logp, torch.float32, "out_logp", (T, N))
+    else:
+        logp = torch.zeros((T, N), dtype=torch.float32, device=dev) if want_logp else None
     mcfg = L.mlp_cfg(dims, activation)
     cov = L.cov_array(cov_diag) if cov_diag is not None else None
     with torch.cuda.device(dev):
@@ -249,16 +256,18 @@ def advantage(mode, G, E, T, gamma, lam, rew, length, values=None, want_rtg=Fals
     return adv, rtg
 
 
-def advantage_ppo_raw(mode, G, E, T, gamma, lam, rew, length, values):
+def advantage_ppo_raw(mode, G, E, T, gamma, lam, rew, length, values, out_adv=None, out_rtg=None):
     """tg_advantage_ppo_raw -> (raw adv [T,N], raw returns [T,N], sums [5] float64 =
-    (sum adv, sum adv^2, sum ret, sum ret^2, n valid)).  The sums are additive over ranks."""
+    (sum adv, sum adv^2, sum ret, sum ret^2, n valid)).  The sums are additive over ranks (and over chunks of whole
+    groups).  `out_adv` / `out_rtg`, when given, receive the raw values (every row is written)."""
     lib = L.load()
     N = G * E
     _need(rew, torch.float32, "rew", (T, N))
     _need(length, torch.int32, "len", (N,))
     _need(values, torch.float32, "values", (T, N))
     dev = rew.device
-    adv, rtg = torch.empty_like(rew), torch.empty_like(rew)
+    adv = torch.empty_like(rew) if out_adv is None else _need(out_adv, torch.float32, "out_adv", (T, N))
+    rtg = torch.empty_like(rew) if out_rtg is None else _need(out_rtg, torch.float32, "out_rtg", (T, N))
     sums = torch.empty((5,), dtype=torch.float64, device=dev)
     ws = _workspace("adv", lib.tg_advantage_workspace_bytes(N, G), dev)
     with torch.cuda.device(dev):

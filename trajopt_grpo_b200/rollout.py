@@ -179,18 +179,28 @@ class RolloutManager:
     def print_progress(self):  # rollout_manager.py:63-83: nothing to poll, a rollout is one launch
         pass
 
-    def rollout_device(self, init_state=None, noise=None) -> DeviceRollout:
-        """The fast path: launch the fused kernel for this rank's groups and return
-        the struct-of-arrays result without materialising masks."""
-        G, E = self.local_workers, self.num_episodes_per_worker
-        if init_state is None and self.world_size > 1:
-            blk = shard_initial_states(self.env, self.num_workers, E, self.restart, self._rng, self.rank,
-                                       self.world_size)
-            dtype = torch.float64 if self.precision == "f64" else torch.float32
+    def next_epoch(self, init_state=None, dtype=None):
+        """Starts the next epoch: returns (init_state [S, local envs] on the policy's device, Philox seed) and advances
+        the epoch counter.  Without `init_state` this rank's block of the global initial states is drawn from the
+        manager's generator (float64 when precision == "f64", else float32, unless `dtype` says otherwise).  Every
+        rollout of an epoch -- rollout_device() or a streamed epoch -- takes its inputs from here, so the same seed
+        gives the same trajectories either way."""
+        if init_state is None:
+            blk = shard_initial_states(self.env, self.num_workers, self.num_episodes_per_worker, self.restart,
+                                       self._rng, self.rank, self.world_size)
+            if dtype is None:
+                dtype = torch.float64 if self.precision == "f64" else torch.float32
             dev = self.policy.actor.flat_params().device                 # the policy's device, not the current one
             init_state = torch.from_numpy(np.ascontiguousarray(blk.T)).to(dtype).pin_memory().to(dev, non_blocking=True)
         seed = (self._seed + 0x9E3779B97F4A7C15 * (self._epoch + 1)) & (2 ** 64 - 1)
         self._epoch += 1
+        return init_state, seed
+
+    def rollout_device(self, init_state=None, noise=None) -> DeviceRollout:
+        """The fast path: launch the fused kernel for this rank's groups and return
+        the struct-of-arrays result without materialising masks."""
+        G, E = self.local_workers, self.num_episodes_per_worker
+        init_state, seed = self.next_epoch(init_state)
         self.last = _device_rollout(self.env, self.policy, G, E, self.restart, self._rng, seed, self.precision,
                                     init_state=init_state, noise=noise, env_offset=self.env_offset,
                                     out=self._out if self.reuse_buffers else None)
