@@ -274,6 +274,17 @@ int tg_policy_grad(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N, int T,
                    const int32_t *len, const float *params, const float *cov_diag,
                    float eps_clip, float scale, float kl_coef,
                    float *out_grad, float *out_stats, void *workspace, void *stream);
+/* tg_policy_grad with GRPO's KL penalty to a frozen reference policy (Shao et al. 2024, eq. 4; the k3 estimator):
+ * per valid sample, u = ref_logp - lp and D = exp(u) - u - 1 >= 0; the objective gains -ref_coef * sum D, so
+ * d objective / d lp gains ref_coef * expm1(u).  ref_coef = beta * scale.
+ *   ref_logp [T][N]: log-prob of act under the reference policy (its own covariance)
+ *   -> out_stats [5] fp32: {objective (with the KL term), n_valid, sum ratio, n_clipped, sum D}
+ * ref_logp == NULL is tg_policy_grad: no KL term, out_stats [4].  Same workspace as tg_policy_grad. */
+int tg_policy_grad_ref(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N, int T,
+                       const float *obs, const float *act, const float *adv, const float *old_logp,
+                       const float *ref_logp, const int32_t *len, const float *params, const float *cov_diag,
+                       float eps_clip, float scale, float kl_coef, float ref_coef,
+                       float *out_grad, float *out_stats, void *workspace, void *stream);
 
 /* The update kernels walk a ragged rollout in LENGTH ORDER (env indices sorted by episode length, live envs per
  * step), built from `len` at the start of every tg_policy_grad / tg_value_grad / tg_policy_forward_traj call.

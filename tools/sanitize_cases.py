@@ -113,6 +113,28 @@ def case_ppo_shard(T=11):
     torch.cuda.synchronize()
 
 
+def case_grpo_ref(N=200, T=6):
+    """GRPO's KL term: the reference forward and tg_policy_grad_ref on the three K3 families."""
+    rng = np.random.default_rng(4)
+    for kind, hidden, math in ((1, [64, 64], "3xtf32"), (3, [256, 256], "3xtf32"), (1, [40, 24], "fp32")):
+        dims = [OBS[kind]] + hidden + [ACT[kind]]
+        p, pr = policy(rng, dims), policy(rng, [OBS[kind]] + [32, 32] + [ACT[kind]])
+        cov = [0.3] * ACT[kind]
+        E.set_math(math)
+        try:
+            out = E.rollout(kind, T, 0.02 if kind != 1 else 0.05, dims, "ReLU", p, cov, init_state(kind, N), seed=3)
+            G = N // 5
+            adv, _ = E.advantage(0, G, 5, T, 0.99, 0.0, out["rew"], out["len"])
+            _, rlp = E.policy_forward_traj([OBS[kind], 32, 32, ACT[kind]], "Tanh", pr, out["obs"], [0.5] * ACT[kind],
+                                           out["act"], out["len"])
+            g, st = E.policy_grad(dims, "ReLU", p, cov, out["obs"], out["act"], adv, out["logp"], out["len"], 0.2,
+                                  -1.0 / G, ref_logp=rlp, ref_scale=-0.04 / G)
+            torch.cuda.synchronize()
+            assert bool(torch.isfinite(g).all()) and float(st[4]) >= 0
+        finally:
+            E.set_math("auto")
+
+
 def case_env():
     for kind in range(4):
         s = init_state(kind, 33).double()
@@ -132,6 +154,7 @@ CASES = {
     "tc256": lambda: case_rollout_update(3, [256, 256], 200, 6, "3xtf32"),
     "ppo": case_ppo,
     "ppo_shard": case_ppo_shard,
+    "grpo_ref": case_grpo_ref,
     "env": case_env,
 }
 

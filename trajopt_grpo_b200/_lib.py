@@ -74,6 +74,8 @@ _SIGS = {
     "tg_policy_grad_scratch_bytes": (C.c_int, [_vp, C.POINTER(MlpCfg), _i64, C.POINTER(_i64), C.POINTER(_i64)]),
     "tg_policy_grad": (C.c_int, [_vp, C.POINTER(MlpCfg), _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, C.POINTER(_f),
                                  _f, _f, _f, _vp, _vp, _vp, _vp]),
+    "tg_policy_grad_ref": (C.c_int, [_vp, C.POINTER(MlpCfg), _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                     C.POINTER(_f), _f, _f, _f, _f, _vp, _vp, _vp, _vp]),
     "tg_value_grad": (C.c_int, [_vp, C.POINTER(MlpCfg), _i64, _i32, _vp, _vp, _vp, _vp, _f, _vp, _vp, _vp, _vp]),
     "tg_policy_grad_batch": (C.c_int, [_vp, C.POINTER(MlpCfg), _i64, _i32, _vp, _vp, _vp, _vp, _vp, _i64, _vp,
                                        C.POINTER(_f), _f, _f, _f, _vp, _vp, _vp, _vp]),

@@ -7,7 +7,8 @@ attribute as the reference; `learn` is a short sequence of kernel launches:
       tg_advantage(GRPO)                         RTG + per-group z-score
       [tg_policy_forward_traj]                   frozen old-policy log-prob (skipped when
                                                  the rollout's own log-prob is that value)
-      updates_per_iter x { tg_policy_grad  ->  [NCCL allreduce]  ->  tg_adam_step }
+      [tg_policy_forward_traj]                   reference-policy log-prob (ref_model, beta != 0)
+      updates_per_iter x { tg_policy_grad[_ref]  ->  [NCCL allreduce]  ->  tg_adam_step }
 
 The objective keeps the reference's sign: `J.backward(); optimizer.step()` with a
 minimising optimizer descends on J (SURVEY q1) -- pass `maximize=True` to ascend.
@@ -202,8 +203,29 @@ def _rollout_of(buffer):
     return r
 
 
+def _check_ref_model(ref, policy):
+    """GRPO's reference policy: a Gaussian actor (or actor-critic, whose actor is used) of this package on the policy's
+    device, with the policy's obs and action dims and storage of its own.  Its hidden dims, activation and covariance
+    may differ from the policy's."""
+    from .policies import GaussianActor_NeuralNetwork, GaussianActorCritic_NeuralNetwork
+    if not isinstance(ref, (GaussianActor_NeuralNetwork, GaussianActorCritic_NeuralNetwork)):
+        raise L.EngineError(f"ref_model must be a GaussianActor_NeuralNetwork or GaussianActorCritic_NeuralNetwork, "
+                            f"got {type(ref).__name__}")
+    if ref is policy:
+        raise L.EngineError("ref_model is the policy itself: a reference that moves with the updates is no reference")
+    pa, ra = policy.actor.dims, ref.actor.dims
+    if (ra[0], ra[-1]) != (pa[0], pa[-1]):
+        raise L.EngineError(f"ref_model maps {ra[0]} obs to {ra[-1]} actions, the policy {pa[0]} to {pa[-1]}")
+    pflat, rflat = policy.flat_parameters(), ref.actor.flat_params()
+    if rflat.device != pflat.device:
+        raise L.EngineError(f"ref_model is on {rflat.device}, the policy on {pflat.device}")
+    if rflat.untyped_storage().data_ptr() == pflat.untyped_storage().data_ptr():
+        raise L.EngineError("ref_model shares its parameter storage with the policy: it would move with the updates")
+
+
 class GRPO(Algorithm):
-    """algorithms/grpo.py:12-168."""
+    """algorithms/grpo.py:12-168.  With a ref_model and beta != 0 the objective gains the k3 KL penalty
+    -(beta / G) sum_valid (exp(u) - u - 1), u = log pi_ref(a|s) - log pi_theta(a|s) (INTEGRATION.md)."""
 
     def __init__(self, epsilon: float, beta: float, gamma: float, policy, optimizer, ref_model=None,
                  updates_per_iter: int = 10, *, maximize: bool = False):
@@ -211,14 +233,21 @@ class GRPO(Algorithm):
         self.gamma, self.updates_per_iter, self.optimizer = gamma, updates_per_iter, optimizer
         self.maximize = maximize
         if ref_model is not None:
-            # grpo.py:129-132 cannot run in the reference either (SURVEY q5); no oracle for a KL term
-            raise L.EngineError("ref_model is not supported: the reference's KL branch is broken (every config passes None)")
+            _check_ref_model(ref_model, policy)
         self.old_policy = copy.deepcopy(self.policy)                 # grpo.py:48
         self._synced_tag = policy.param_tag()                        # old_policy == policy at this tag ...
         self._old_tag = self.old_policy.param_tag()                  # ... while old_policy itself is untouched
         self._seen_loads = getattr(policy, "checkpoint_loads", 0)
         self._flat_opt = _FlatOptimizer(optimizer, policy)
         self.last_stats = None
+
+    def _ref_actor(self):
+        """(dims, activation, flat params, cov) of the reference actor, or None when the KL term is off
+        (no ref_model, or beta == 0: then no reference forward runs at all)."""
+        if self.ref_model is None or self.beta == 0:
+            return None
+        a = self.ref_model.actor
+        return a.dims, a.activation_name, a.flat_params(), self.ref_model.cov_diag
 
     def learn(self, buffer) -> None:
         r = _rollout_of(buffer)
@@ -242,14 +271,19 @@ class GRPO(Algorithm):
                                                      r.act, r.len)
         scale = (-1.0 if self.maximize else 1.0) / G_global         # grpo.py:140 (J /= group_size)
         comm = self._flat_opt.peer_comm(flat) if world > 1 else None
+        ref = self._ref_actor()
         with engine.length_order(r.len, r.T):                       # lengths are fixed for all updates of this learn()
+            # grpo.py:129: log pi_ref(a|s), once: the reference is frozen, so every update would see the same values
+            ref_logp = None if ref is None else engine.policy_forward_traj(ref[0], ref[1], ref[2], r.obs, ref[3], r.act,
+                                                                           r.len)[1]
             for _ in range(self.updates_per_iter):                  # grpo.py:106
                 # the path's only collective: the gradient summed over ranks.  With the peer-memory window the kernel
                 # writes its gradient into this rank's slot and ONE launch does allreduce + Adam (tg_comm.cu);
                 # otherwise NCCL allreduce + tg_adam_step
                 slot = comm.grad_slot()[:flat.numel()] if comm is not None else None
                 grad, stats = engine.policy_grad(dims, act_name, flat, cov, r.obs, r.act, adv, old_logp, r.len,
-                                                 self.epsilon, scale, out_grad=slot)
+                                                 self.epsilon, scale, out_grad=slot, ref_logp=ref_logp,
+                                                 ref_scale=self.beta * scale)
                 if comm is not None:
                     self._flat_opt.step_allreduced(flat, comm)      # grpo.py:143-145 on the summed gradient
                 else:
@@ -277,7 +311,9 @@ class GRPO(Algorithm):
                 K2 advantages of the chunk         K3 gradient of the chunk under the current weights, accumulated
             [gradient allreduce]  Adam
 
-        One trajectory buffer of chunk size is reused.  With updates_per_iter == 1 no work is repeated.
+        One trajectory buffer of chunk size is reused.  With updates_per_iter == 1 no work is repeated.  With a
+        reference policy (ref_model, beta != 0) each chunk also runs the reference forward into a chunk-sized
+        log-prob buffer, once per chunk and update, because the buffer is reused.
         Equal to sample() + learn() on the same seed up to the fp32 summation order of the per-chunk gradients.
         Returns the number of valid env-steps of this rank's rollout as a 0-dim CUDA tensor (no host sync)."""
         pol = self.policy
@@ -298,6 +334,9 @@ class GRPO(Algorithm):
         out = getattr(self, "_stream_out", None)
         grad_own, grad_part = torch.empty_like(flat), torch.empty_like(flat)
         comm = self._flat_opt.peer_comm(flat) if world > 1 else None
+        ref = self._ref_actor()
+        ref_store = None if ref is None else \
+            torch.empty(env.max_steps * min(G_loc, chunk_groups) * E, dtype=torch.float32, device=dev)
         for u in range(self.updates_per_iter):
             grad_total = comm.grad_slot()[:flat.numel()] if comm is not None else grad_own
             grad_total.zero_()
@@ -309,8 +348,14 @@ class GRPO(Algorithm):
                                      seed=seed, env_offset=manager.env_offset + n0, phys=getattr(env, "_tg_phys", None),
                                      out=out)
                 adv, _ = engine.advantage(L.ADV_GRPO, g1 - g0, E, env.max_steps, self.gamma, 0.0, out["rew"], out["len"])
+                ref_logp = None
+                if ref is not None:
+                    ref_logp = ref_store[:env.max_steps * (n1 - n0)].view(env.max_steps, n1 - n0)
+                    engine.policy_forward_traj(ref[0], ref[1], ref[2], out["obs"], ref[3], out["act"], out["len"],
+                                               out_logp=ref_logp)
                 _, stats = engine.policy_grad(dims, act_name, flat, cov, out["obs"], out["act"], adv, out["logp"],
-                                              out["len"], self.epsilon, scale, out_grad=grad_part)
+                                              out["len"], self.epsilon, scale, out_grad=grad_part, ref_logp=ref_logp,
+                                              ref_scale=self.beta * scale)
                 grad_total.add_(grad_part)
                 if u == 0:
                     n_valid.add_(out["len"].sum())

@@ -161,17 +161,23 @@ struct TcwLayout {
 };
 void tg_build_tcw_layout(const tg_mlp_cfg *mlp, TcwLayout *out, bool with_backward);
 int tg_pack_weights_tcw(tg_ctx *ctx, const TcwLayout &lay, const float *params, cudaStream_t st);
+// statistics each update CTA leaves in its row of spart [grid][TG_SPART_LD]: objective, n_valid, sum ratio, n_clipped,
+// and the sum of GRPO's k3 KL estimator (0 without a reference policy).  The row is padded to 8 doubles: with a
+// stride of 5, ptxas spilled more in the tensor-core kernels without the KL term (W = 256 kernel A 44 -> 72 B).
+#define TG_NSTAT 5
+#define TG_SPART_LD 8
 // wide (128 / 256) tensor-core update, two streamed kernels per batch of tiles (tg_update_tcw.cu)
 bool tg_update_tcw_shape_built(const tg_mlp_cfg *mlp);
 int tg_policy_grad_tcw(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N, int T, const float *obs, const float *act,
                        const float *adv, const float *old_logp, const float *target, const int32_t *len, const float *params,
                        const float *inv_sd, const float *inv_var, float log_norm, float eps_clip, float scale,
                        float kl_scale, float *gpart, double *spart, int grid, cudaStream_t st, float *out_mu = nullptr,
-                       float *out_logp = nullptr);   // out_mu / out_logp non-null: forward only (no gradients)
+                       float *out_logp = nullptr,    // out_mu / out_logp non-null: forward only (no gradients)
+                       const float *ref_logp = nullptr, float ref_coef = 0.0f);   // GRPO's k3 KL term
 // tensor-core update kernel (tg_update_tc.cu)
 bool tg_update_tc_eligible(const tg_mlp_cfg *mlp);
 int tg_update_tc_grid(const tg_ctx *ctx);
 int tg_policy_grad_tc(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N, int T, const float *obs, const float *act,
-                      const float *adv, const float *old_logp, const int32_t *len, const float *params,
-                      const float *inv_sd, const float *inv_var, float log_norm, float eps_clip, float scale,
-                      float kl_scale, float *gpart, double *spart, int grid, cudaStream_t st);
+                      const float *adv, const float *old_logp, const float *ref_logp, const int32_t *len,
+                      const float *params, const float *inv_sd, const float *inv_var, float log_norm, float eps_clip,
+                      float scale, float kl_scale, float ref_coef, float *gpart, double *spart, int grid, cudaStream_t st);

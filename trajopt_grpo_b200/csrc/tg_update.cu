@@ -26,6 +26,7 @@ struct UpdArgs {
     int T;
     int head;
     const float *obs, *act, *adv, *oldlp, *target;
+    const float *reflp;   // log-prob under a frozen reference policy (GRPO's KL term) or null
     const int32_t *len;
     // length order (tg_order.cu) or null: sorted position j of step t is env perm[j], live iff j < cnt[t]
     const int32_t *perm, *cnt;
@@ -35,9 +36,9 @@ struct UpdArgs {
     int64_t n_sidx;
     const float *packed;
     float inv_sd[TG_MAX_ACT], inv_var[TG_MAX_ACT], log_norm;
-    float eps_clip, scale, kl_scale;
+    float eps_clip, scale, kl_scale, ref_coef;
     float *gpart;   // [grid][n_params]
-    double *spart;  // [grid][4]
+    double *spart;  // [grid][TG_SPART_LD]
     float *out_mu, *out_logp;
 };
 
@@ -117,7 +118,7 @@ __global__ void __launch_bounds__(TileCfg<CFG>::NT) update_kernel(const __grid_c
     constexpr int B = TileCfg<CFG>::B, NT = TileCfg<CFG>::NT, NP = TileCfg<CFG>::NP, LDX = B + 4;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ __align__(8) uint64_t wbar;
-    __shared__ double sred[4][NT / 32];
+    __shared__ double sred[TG_NSTAT][NT / 32];
     __shared__ int32_t tile_env[B];      // env index of each sample of the tile, -1 = padding
     __shared__ int32_t tile_t[B];        // its step index (tile-uniform except in minibatch mode)
     const int nl = a.lay.n_layers, nh = nl - 1;
@@ -138,7 +139,7 @@ __global__ void __launch_bounds__(TileCfg<CFG>::NT) update_kernel(const __grid_c
     const int64_t ntiles = a.sidx ? NB : NB * a.T;
     float *gp = a.gpart ? a.gpart + (int64_t)blockIdx.x * a.lay.n_params : nullptr;
     const bool owner = threadIdx.x < B;
-    double s_obj = 0.0, s_cnt = 0.0, s_ratio = 0.0, s_clip = 0.0;
+    double s_obj = 0.0, s_cnt = 0.0, s_ratio = 0.0, s_clip = 0.0, s_kl = 0.0;
     const tg_layer_layout &LO = a.lay.L[nl - 1];
 
     for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
@@ -232,6 +233,13 @@ __global__ void __launch_bounds__(TileCfg<CFG>::NT) update_kernel(const __grid_c
                             s_obj += (double)a.kl_scale * eo * (olp - lp);
                             dlp -= a.kl_scale * eo;
                         }
+                        if (a.reflp) {                              // k3 KL to the reference policy
+                            const float u = a.reflp[row] - lp, em = expm1f(u);
+                            const float d = em - u;
+                            s_obj -= (double)a.ref_coef * d;
+                            s_kl += d;
+                            dlp += a.ref_coef * em;
+                        }
                         s_cnt += 1.0;
                         s_ratio += ratio;
                         s_clip += in_range ? 0.0 : 1.0;
@@ -281,34 +289,34 @@ __global__ void __launch_bounds__(TileCfg<CFG>::NT) update_kernel(const __grid_c
     }
     // ---- statistics: warp shuffle, then a fixed-order sum over the warps
     if (a.spart) {
-        double v[4] = {s_obj, s_cnt, s_ratio, s_clip};
+        double v[TG_NSTAT] = {s_obj, s_cnt, s_ratio, s_clip, s_kl};
 #pragma unroll
-        for (int q = 0; q < 4; ++q) {
+        for (int q = 0; q < TG_NSTAT; ++q) {
             for (int off = 16; off > 0; off >>= 1) v[q] += __shfl_down_sync(0xffffffffu, v[q], off);
             if ((threadIdx.x & 31) == 0) sred[q][threadIdx.x >> 5] = v[q];
         }
         __syncthreads();
-        if (threadIdx.x < 4) {
+        if (threadIdx.x < TG_NSTAT) {
             double s = 0.0;
             for (int w = 0; w < NT / 32; ++w) s += sred[threadIdx.x][w];
-            a.spart[(int64_t)blockIdx.x * 4 + threadIdx.x] = s;
+            a.spart[(int64_t)blockIdx.x * TG_SPART_LD + threadIdx.x] = s;
         }
     }
 }
 
-// sum the CTA-private gradient copies in a fixed order
+// sum the CTA-private gradient copies in a fixed order; the first nstat statistics go to out_stats
 __global__ void grad_reduce_kernel(int grid, int64_t n_params, const float *__restrict__ gpart,
                                    const double *__restrict__ spart, float *__restrict__ out_grad,
-                                   float *__restrict__ out_stats) {
+                                   float *__restrict__ out_stats, int nstat) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n_params) {
         float s = 0.0f;
         for (int c = 0; c < grid; ++c) s += gpart[(int64_t)c * n_params + i];
         out_grad[i] = s;
     }
-    if (out_stats && blockIdx.x == 0 && threadIdx.x < 4) {
+    if (out_stats && blockIdx.x == 0 && threadIdx.x < nstat) {
         double s = 0.0;
-        for (int c = 0; c < grid; ++c) s += spart[(int64_t)c * 4 + threadIdx.x];
+        for (int c = 0; c < grid; ++c) s += spart[(int64_t)c * TG_SPART_LD + threadIdx.x];
         out_stats[threadIdx.x] = (float)s;
     }
 }
@@ -373,29 +381,30 @@ extern "C" int64_t tg_policy_grad_workspace_bytes(const tg_ctx *ctx, const tg_ml
     tg_mlp_layout lay;
     if (tg_build_layout(mlp, true, &lay, ctx->smem_optin)) return -1;
     const int64_t grid = update_grid(ctx, lay);
-    return grid * lay.n_params * (int64_t)sizeof(float) + grid * 4 * (int64_t)sizeof(double) + 256;
+    return grid * lay.n_params * (int64_t)sizeof(float) + grid * TG_SPART_LD * (int64_t)sizeof(double) + 256;
 }
 
 // The gradient of every update path: the workspace holds one partial gradient per CTA, gpart [grid][n_params], and
-// the statistics spart [grid][4] (256-byte aligned); both are zeroed, `update(gpart, spart)` launches the kernels
-// that fill them, and grad_reduce_kernel sums the copies in a fixed order into out_grad / out_stats.
+// the statistics spart [grid][TG_SPART_LD] (256-byte aligned); both are zeroed, `update(gpart, spart)` launches the
+// kernels that fill them, and grad_reduce_kernel sums the copies in a fixed order into out_grad and the first
+// `nstat` statistics into out_stats.
 template <typename Update>
-static int grad_via_partials(int grid, int64_t n_params, void *workspace, float *out_grad, float *out_stats,
+static int grad_via_partials(int grid, int64_t n_params, void *workspace, float *out_grad, float *out_stats, int nstat,
                              cudaStream_t st, Update update) {
     const size_t gbytes = ((size_t)grid * n_params * sizeof(float) + 255) / 256 * 256;
     float *gpart = reinterpret_cast<float *>(workspace);
     double *spart = reinterpret_cast<double *>(reinterpret_cast<char *>(workspace) + gbytes);
-    TG_CUDA(cudaMemsetAsync(workspace, 0, gbytes + (size_t)grid * 4 * sizeof(double), st));
+    TG_CUDA(cudaMemsetAsync(workspace, 0, gbytes + (size_t)grid * TG_SPART_LD * sizeof(double), st));
     int rc = update(gpart, spart);
     if (rc) return rc;
     grad_reduce_kernel<<<(unsigned)((n_params + 255) / 256), 256, 0, st>>>(grid, n_params, gpart, spart, out_grad,
-                                                                          out_stats);
+                                                                          out_stats, nstat);
     TG_CUDA(cudaGetLastError());
     return TG_OK;
 }
 
-static int run_grad(tg_ctx *ctx, UpdArgs &a, const float *params, float *out_grad, float *out_stats, void *workspace,
-                    cudaStream_t st) {
+static int run_grad(tg_ctx *ctx, UpdArgs &a, const float *params, float *out_grad, float *out_stats, int nstat,
+                    void *workspace, cudaStream_t st) {
     TG_CUDA(cudaSetDevice(ctx->device));
     int rc = tg_pack_weights(ctx, a.lay, params, st);
     if (rc) return rc;
@@ -407,21 +416,23 @@ static int run_grad(tg_ctx *ctx, UpdArgs &a, const float *params, float *out_gra
         a.cnt = ctx->cnt;
     }
     const int grid = update_grid(ctx, a.lay);
-    return grad_via_partials(grid, a.lay.n_params, workspace, out_grad, out_stats, st, [&](float *gpart, double *spart) {
+    return grad_via_partials(grid, a.lay.n_params, workspace, out_grad, out_stats, nstat, st, [&](float *gpart, double *spart) {
         a.gpart = gpart;
         a.spart = spart;
         return dispatch_update(ctx, a, grid, st);
     });
 }
 
-extern "C" int tg_policy_grad(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N, int T, const float *obs, const float *act,
-                              const float *adv, const float *old_logp, const int32_t *len, const float *params,
-                              const float *cov_diag, float eps_clip, float scale, float kl_coef, float *out_grad,
-                              float *out_stats, void *workspace, void *stream) {
+// tg_policy_grad and tg_policy_grad_ref: ref_logp == null leaves out the KL term and writes 4 statistics
+static int policy_grad_impl(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N, int T, const float *obs, const float *act,
+                            const float *adv, const float *old_logp, const float *ref_logp, const int32_t *len,
+                            const float *params, const float *cov_diag, float eps_clip, float scale, float kl_coef,
+                            float ref_coef, float *out_grad, float *out_stats, void *workspace, void *stream) {
     TgRange nvtx_range("tg_policy_grad (K3: clipped surrogate + MLP backward)");
     TG_REQUIRE(ctx && mlp && obs && act && adv && old_logp && len && params && cov_diag && out_grad && workspace,
                TG_ERR_ARG, "tg_policy_grad: null argument");
     TG_REQUIRE(N > 0 && T > 0, TG_ERR_SHAPE, "tg_policy_grad: N and T must be positive");
+    const int nstat = ref_logp ? TG_NSTAT : 4;
     UpdArgs a;
     memset(&a, 0, sizeof(a));
     int rc = tg_build_layout(mlp, true, &a.lay, ctx->smem_optin);
@@ -429,16 +440,18 @@ extern "C" int tg_policy_grad(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N, int
     rc = tg_gauss_consts(cov_diag, a.lay.A, nullptr, a.inv_sd, a.inv_var, &a.log_norm);
     if (rc) return rc;
     a.N = N; a.T = T; a.head = HEAD_POLICY;
-    a.obs = obs; a.act = act; a.adv = adv; a.oldlp = old_logp; a.len = len;
-    a.eps_clip = eps_clip; a.scale = scale; a.kl_scale = kl_coef;
+    a.obs = obs; a.act = act; a.adv = adv; a.oldlp = old_logp; a.reflp = ref_logp; a.len = len;
+    a.eps_clip = eps_clip; a.scale = scale; a.kl_scale = kl_coef; a.ref_coef = ref_coef;
     // ---- tensor-core paths (3xTF32 tcgen05) for eligible policies
     if (tg_update_tcw_shape_built(mlp) && ctx->math_mode != TG_MATH_FP32) {      // 128 / 256 wide: streamed, two kernels
         cudaStream_t st = (cudaStream_t)stream;
         TG_CUDA(cudaSetDevice(ctx->device));
         const int grid = ctx->sm_count;
-        return grad_via_partials(grid, a.lay.n_params, workspace, out_grad, out_stats, st, [&](float *gpart, double *spart) {
+        return grad_via_partials(grid, a.lay.n_params, workspace, out_grad, out_stats, nstat, st,
+                                 [&](float *gpart, double *spart) {
             return tg_policy_grad_tcw(ctx, mlp, N, T, obs, act, adv, old_logp, nullptr, len, params, a.inv_sd, a.inv_var,
-                                      a.log_norm, eps_clip, scale, kl_coef, gpart, spart, grid, st);
+                                      a.log_norm, eps_clip, scale, kl_coef, gpart, spart, grid, st, nullptr, nullptr,
+                                      ref_logp, ref_coef);
         });
     }
     const bool tc_ok = tg_update_tc_eligible(mlp);
@@ -449,12 +462,30 @@ extern "C" int tg_policy_grad(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N, int
         cudaStream_t st = (cudaStream_t)stream;
         TG_CUDA(cudaSetDevice(ctx->device));
         const int grid = tg_update_tc_grid(ctx);
-        return grad_via_partials(grid, a.lay.n_params, workspace, out_grad, out_stats, st, [&](float *gpart, double *spart) {
-            return tg_policy_grad_tc(ctx, mlp, N, T, obs, act, adv, old_logp, len, params, a.inv_sd, a.inv_var, a.log_norm,
-                                     eps_clip, scale, kl_coef, gpart, spart, grid, st);
+        return grad_via_partials(grid, a.lay.n_params, workspace, out_grad, out_stats, nstat, st,
+                                 [&](float *gpart, double *spart) {
+            return tg_policy_grad_tc(ctx, mlp, N, T, obs, act, adv, old_logp, ref_logp, len, params, a.inv_sd, a.inv_var,
+                                     a.log_norm, eps_clip, scale, kl_coef, ref_coef, gpart, spart, grid, st);
         });
     }
-    return run_grad(ctx, a, params, out_grad, out_stats, workspace, (cudaStream_t)stream);
+    return run_grad(ctx, a, params, out_grad, out_stats, nstat, workspace, (cudaStream_t)stream);
+}
+
+extern "C" int tg_policy_grad(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N, int T, const float *obs, const float *act,
+                              const float *adv, const float *old_logp, const int32_t *len, const float *params,
+                              const float *cov_diag, float eps_clip, float scale, float kl_coef, float *out_grad,
+                              float *out_stats, void *workspace, void *stream) {
+    return policy_grad_impl(ctx, mlp, N, T, obs, act, adv, old_logp, nullptr, len, params, cov_diag, eps_clip, scale,
+                            kl_coef, 0.0f, out_grad, out_stats, workspace, stream);
+}
+
+extern "C" int tg_policy_grad_ref(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N, int T, const float *obs,
+                                  const float *act, const float *adv, const float *old_logp, const float *ref_logp,
+                                  const int32_t *len, const float *params, const float *cov_diag, float eps_clip,
+                                  float scale, float kl_coef, float ref_coef, float *out_grad, float *out_stats,
+                                  void *workspace, void *stream) {
+    return policy_grad_impl(ctx, mlp, N, T, obs, act, adv, old_logp, ref_logp, len, params, cov_diag, eps_clip, scale,
+                            kl_coef, ref_coef, out_grad, out_stats, workspace, stream);
 }
 
 // Minibatch forms (PPO with batch_size != None, algorithms/ppo.py:147-183): the gradient of the same
@@ -477,7 +508,7 @@ extern "C" int tg_policy_grad_batch(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t 
     a.obs = obs; a.act = act; a.adv = adv; a.oldlp = old_logp;
     a.sidx = sample_ids; a.n_sidx = n_samples;
     a.eps_clip = eps_clip; a.scale = scale; a.kl_scale = kl_coef;
-    return run_grad(ctx, a, params, out_grad, out_stats, workspace, (cudaStream_t)stream);
+    return run_grad(ctx, a, params, out_grad, out_stats, 4, workspace, (cudaStream_t)stream);
 }
 
 extern "C" int tg_value_grad_batch(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N, int T, const float *obs,
@@ -495,7 +526,7 @@ extern "C" int tg_value_grad_batch(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N
     a.N = N; a.T = T; a.head = HEAD_VALUE;
     a.obs = obs; a.target = target; a.scale = scale;
     a.sidx = sample_ids; a.n_sidx = n_samples;
-    return run_grad(ctx, a, params, out_grad, out_stats, workspace, (cudaStream_t)stream);
+    return run_grad(ctx, a, params, out_grad, out_stats, 4, workspace, (cudaStream_t)stream);
 }
 
 extern "C" int tg_value_grad(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N, int T, const float *obs,
@@ -516,12 +547,12 @@ extern "C" int tg_value_grad(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N, int 
         cudaStream_t st = (cudaStream_t)stream;
         TG_CUDA(cudaSetDevice(ctx->device));
         const int grid = ctx->sm_count;
-        return grad_via_partials(grid, a.lay.n_params, workspace, out_grad, out_stats, st, [&](float *gpart, double *spart) {
+        return grad_via_partials(grid, a.lay.n_params, workspace, out_grad, out_stats, 4, st, [&](float *gpart, double *spart) {
             return tg_policy_grad_tcw(ctx, mlp, N, T, obs, nullptr, nullptr, nullptr, target, len, params, nullptr, nullptr,
                                       0.0f, 0.0f, scale, 0.0f, gpart, spart, grid, st);
         });
     }
-    return run_grad(ctx, a, params, out_grad, out_stats, workspace, (cudaStream_t)stream);
+    return run_grad(ctx, a, params, out_grad, out_stats, 4, workspace, (cudaStream_t)stream);
 }
 
 extern "C" int tg_policy_forward(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t M, const float *x, const float *params,

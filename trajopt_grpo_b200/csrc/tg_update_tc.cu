@@ -43,9 +43,12 @@ struct UpdTcArgs {
     float inv_sd[TG_MAX_ACT], inv_var[TG_MAX_ACT], log_norm;
     float eps_clip, scale, kl_scale;
     float *gpart;   // [grid][n_params], zero-initialised
-    double *spart;  // [grid][4]
+    double *spart;  // [grid][TG_SPART_LD]
     // length order of the rollout (tg_order.cu): sorted position j of step t is env perm[j], live iff j < cnt[t]
     const int32_t *perm, *cnt;
+    // GRPO's KL term (REF instances): log-prob under a frozen reference policy and its coefficient beta * scale
+    const float *reflp;
+    float ref_coef;
 };
 
 // butterfly column sums: v[0..32) per lane -> v[0] = sum over the warp's 32 lanes of column `lane`
@@ -126,14 +129,17 @@ TG_D void split4(const float *v, float4 &hi, float4 &lo) {
 // NPART threads serve one sample: NPART*4 compute warps + the issuer warp (4 threads per sample measured no faster:
 // the kernel is bound by its instruction count and phase chain, not by warp parallelism; DESIGN.md K3-TC)
 constexpr int NPART = 2;
-template <int O, int A, bool RELU>
+// REF: with GRPO's KL term to a reference policy (a.reflp).  A template flag, not a branch: the instances without it
+// keep their register allocation and spills (the epilogues are at the 168-register cap)
+template <int O, int A, bool RELU, bool REF>
 __global__ void __launch_bounds__(NPART * 128 + 32, 1) update_tc_kernel(const __grid_constant__ UpdTcArgs a) {
     constexpr int W = TC_W, HW = TC_W / NPART, O4 = (O + 1 + 3) / 4 * 4;
     constexpr int NCW = NPART * 4, NT = NPART * 128 + 32;
+    constexpr int NS = REF ? TG_NSTAT : 4;          // statistics this instance produces
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     __shared__ __align__(8) uint64_t wbar, bar_a, bar_b, bar_w;
     __shared__ uint32_t tmem_slot;
-    __shared__ double sred[4][NCW];
+    __shared__ double sred[NS][NCW];
     __shared__ float muS[NPART][A][128];
     if ((smem_u32(smem_raw) & 1023u) != 0u) __trap();
     float *Wsm = reinterpret_cast<float *>(smem_raw);
@@ -178,7 +184,7 @@ __global__ void __launch_bounds__(NPART * 128 + 32, 1) update_tc_kernel(const __
     for (int j = 0; j < A; ++j) c_wo[j] = c_bo[j] = 0.0f;
 #pragma unroll
     for (int o = 0; o < O; ++o) c_w0[o] = 0.0f;
-    double s_obj = 0.0, s_cnt = 0.0, s_ratio = 0.0, s_clip = 0.0;
+    double s_obj = 0.0, s_cnt = 0.0, s_ratio = 0.0, s_clip = 0.0, s_kl = 0.0;
 
     const int64_t N = a.N;
     const int64_t NB = (N + 127) / 128;
@@ -266,7 +272,7 @@ __global__ void __launch_bounds__(NPART * 128 + 32, 1) update_tc_kernel(const __
     } else {
     // ===== compute warps =====
     // software prefetch of a tile's per-sample inputs
-    float xn[O], an[A], advn = 0.f, olpn = 0.f;
+    float xn[O], an[A], advn = 0.f, olpn = 0.f, lrn = 0.f;
     bool vn = false;
     auto prefetch = [&](int64_t tile) {
         vn = false;
@@ -282,6 +288,7 @@ __global__ void __launch_bounds__(NPART * 128 + 32, 1) update_tc_kernel(const __
                 for (int j2 = 0; j2 < A; ++j2) an[j2] = a.act[((int64_t)t * A + j2) * N + n];
                 advn = a.adv[(int64_t)t * N + n];
                 olpn = a.oldlp[(int64_t)t * N + n];
+                if (REF) lrn = a.reflp[(int64_t)t * N + n];
             }
         }
     };
@@ -342,7 +349,7 @@ __global__ void __launch_bounds__(NPART * 128 + 32, 1) update_tc_kernel(const __
     for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
         float x[O], av[A];
         const bool valid = vn;
-        const float adv = advn, olp = olpn;
+        const float adv = advn, olp = olpn, lr = lrn;
 #pragma unroll
         for (int o = 0; o < O; ++o) x[o] = valid ? xn[o] : 0.0f;
 #pragma unroll
@@ -452,10 +459,20 @@ __global__ void __launch_bounds__(NPART * 128 + 32, 1) update_tc_kernel(const __
                 eo = expf(olp);
                 dlp -= a.kl_scale * eo;
             }
+            float dkl = 0.0f;
+            if (REF) {                          // k3 KL to the reference policy
+                const float u = lr - lp, em = expm1f(u);
+                dkl = em - u;
+                dlp += a.ref_coef * em;
+            }
 #pragma unroll
             for (int j = 0; j < A; ++j) dmu[j] = dlp * (av[j] - mu[j]) * a.inv_var[j];
             if (hf == 0) {       // one of the threads of a sample keeps the statistics
                 s_obj += (double)fminf(s1, s2) * a.scale + (double)a.kl_scale * eo * (olp - lp);
+                if (REF) {
+                    s_obj -= (double)a.ref_coef * dkl;
+                    s_kl += dkl;
+                }
                 s_cnt += 1.0; s_ratio += ratio; s_clip += in_range ? 0.0 : 1.0;
 #pragma unroll
                 for (int j = 0; j < A; ++j) c_bo[j] += dmu[j];
@@ -553,17 +570,17 @@ __global__ void __launch_bounds__(NPART * 128 + 32, 1) update_tc_kernel(const __
     }
     // dbo and the statistics: warp shuffle, then a fixed-order sum over the warps
     {
-        double v[4] = {s_obj, s_cnt, s_ratio, s_clip};
+        double v[TG_NSTAT] = {s_obj, s_cnt, s_ratio, s_clip, s_kl};
 #pragma unroll
-        for (int k = 0; k < 4; ++k) {
+        for (int k = 0; k < NS; ++k) {
             for (int off = 16; off > 0; off >>= 1) v[k] += __shfl_down_sync(0xffffffffu, v[k], off);
             if (lane == 0 && warp < NCW) sred[k][warp] = v[k];
         }
         __syncthreads();
-        if (threadIdx.x < 4 && a.spart) {
+        if (threadIdx.x < NS && a.spart) {
             double t = 0.0;
             for (int w = 0; w < NCW; ++w) t += sred[threadIdx.x][w];
-            a.spart[(int64_t)blockIdx.x * 4 + threadIdx.x] = t;
+            a.spart[(int64_t)blockIdx.x * TG_SPART_LD + threadIdx.x] = t;
         }
         __syncthreads();
 #pragma unroll
@@ -585,13 +602,19 @@ __global__ void __launch_bounds__(NPART * 128 + 32, 1) update_tc_kernel(const __
     if (threadIdx.x < 32) tmem_dealloc(tmem, 512);
 }
 
-template <int O, int A>
-static int launch_update_tc(const UpdTcArgs &a, int grid, size_t smem, cudaStream_t st) {
-    void (*kern)(const UpdTcArgs) = a.lay.act == TG_ACT_RELU ? update_tc_kernel<O, A, true> : update_tc_kernel<O, A, false>;
+template <int O, int A, bool REF>
+static int launch_update_tc_ref(const UpdTcArgs &a, int grid, size_t smem, cudaStream_t st) {
+    void (*kern)(const UpdTcArgs) =
+        a.lay.act == TG_ACT_RELU ? update_tc_kernel<O, A, true, REF> : update_tc_kernel<O, A, false, REF>;
     TG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     kern<<<grid, NPART * 128 + 32, smem, st>>>(a);
     TG_CUDA(cudaGetLastError());
     return TG_OK;
+}
+
+template <int O, int A>
+static int launch_update_tc(const UpdTcArgs &a, int grid, size_t smem, cudaStream_t st) {
+    return a.reflp ? launch_update_tc_ref<O, A, true>(a, grid, smem, st) : launch_update_tc_ref<O, A, false>(a, grid, smem, st);
 }
 
 bool tg_update_tc_eligible(const tg_mlp_cfg *mlp) {
@@ -602,21 +625,21 @@ bool tg_update_tc_eligible(const tg_mlp_cfg *mlp) {
 
 int tg_update_tc_grid(const tg_ctx *ctx) { return ctx->sm_count; }
 
-// Launch the tensor-core update kernel.  gpart [grid][n_params] must be zeroed; spart [grid][4].
+// Launch the tensor-core update kernel.  gpart [grid][n_params] must be zeroed; spart [grid][TG_SPART_LD].
 int tg_policy_grad_tc(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N, int T, const float *obs, const float *act,
-                      const float *adv, const float *old_logp, const int32_t *len, const float *params,
-                      const float *inv_sd, const float *inv_var, float log_norm, float eps_clip, float scale,
-                      float kl_scale, float *gpart, double *spart, int grid, cudaStream_t st) {
+                      const float *adv, const float *old_logp, const float *ref_logp, const int32_t *len,
+                      const float *params, const float *inv_sd, const float *inv_var, float log_norm, float eps_clip,
+                      float scale, float kl_scale, float ref_coef, float *gpart, double *spart, int grid, cudaStream_t st) {
     UpdTcArgs a;
     memset(&a, 0, sizeof(a));
     int rc = tg_build_tc_layout(mlp, &a.lay, true);
     if (rc) return rc;
     rc = tg_pack_weights_tc(ctx, a.lay, params, st);
     if (rc) return rc;
-    a.N = N; a.T = T; a.obs = obs; a.act = act; a.adv = adv; a.oldlp = old_logp; a.len = len;
+    a.N = N; a.T = T; a.obs = obs; a.act = act; a.adv = adv; a.oldlp = old_logp; a.reflp = ref_logp; a.len = len;
     a.packed = ctx->packed_tc;
     for (int j = 0; j < TG_MAX_ACT; ++j) { a.inv_sd[j] = inv_sd[j]; a.inv_var[j] = inv_var[j]; }
-    a.log_norm = log_norm; a.eps_clip = eps_clip; a.scale = scale; a.kl_scale = kl_scale;
+    a.log_norm = log_norm; a.eps_clip = eps_clip; a.scale = scale; a.kl_scale = kl_scale; a.ref_coef = ref_coef;
     a.gpart = gpart; a.spart = spart;
     rc = tg_len_order(ctx, N, T, len, st);
     if (rc) return rc;

@@ -63,11 +63,14 @@ struct TcwArgs {
     float inv_sd[TG_MAX_ACT], inv_var[TG_MAX_ACT], log_norm;
     float eps_clip, scale, kl_scale;
     float *gpart;                         // [grid][n_params], accumulated (+=) across launches
-    double *spart;                        // [grid][4], accumulated
+    double *spart;                        // [grid][TG_SPART_LD], accumulated
     // forward-only mode (tg_policy_forward_traj: critic values over a rollout ppo.py:93-94, old log-probs
     // ppo.py:142-143 / grpo.py:118-119): kernel A stops after the output layer and writes these; no kernel B
     int forward_only;
     float *out_mu, *out_logp;
+    // GRPO's KL term (REF instances): log-prob under a frozen reference policy and its coefficient beta * scale
+    const float *reflp;
+    float ref_coef;
 };
 
 bool tg_update_tcw_shape_built(const tg_mlp_cfg *mlp);
@@ -190,7 +193,9 @@ TG_D void tcw_reload32(const unsigned char *arr, int s, int cbk, uint32_t tm_hi,
 // NP = 2 keeps the CTA at 10 warps = 3 per SM sub-partition, i.e. 168 registers per thread and no spills; with
 // NP = 4 (18 warps, 96 registers) the epilogues spilled ~0.8 KB per thread into an L1 that the 222 KB of shared
 // memory leave almost no room for, and the serial step chain paid the L2 latency of every reload.
-template <int O, int A, bool RELU, int W, int NP>
+// REF: with GRPO's KL term to a reference policy (a.reflp).  A template flag, not a branch: at W = 256 the epilogues
+// run at the 96-register cap, and a runtime branch added ~30 B of spills to the instances without the term.
+template <int O, int A, bool RELU, int W, int NP, bool REF>
 __global__ void __launch_bounds__(NP * 128 + 64, 1) update_tcw_fwdbwd_kernel(const __grid_constant__ TcwArgs a) {
     constexpr int HW = W / NP, NCH = HW / 32, OKP = (O + 1 + 7) / 8 * 8, KH = W / 128;
     constexpr int XKP = (O + 1 + A + 7) / 8 * 8;      // rows of Y = [x, 1, dmu, 0..] handed to kernel B
@@ -199,18 +204,19 @@ __global__ void __launch_bounds__(NP * 128 + 64, 1) update_tcw_fwdbwd_kernel(con
     constexpr int NKC = W / 32;                       // K chunks per direction
     constexpr uint32_t CB = (uint32_t)W * 128u;       // chunk bytes
     constexpr uint32_t TM_D = 0u, TM_AHI = (uint32_t)W, TM_ALO = (uint32_t)W + 128u;
+    constexpr int NS = REF ? TG_NSTAT : 4;            // statistics this instance produces
     if (a.k_begin + blockIdx.x >= a.tstart[a.T]) return;      // no live tile for this CTA in this batch (CTA-uniform)
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     __shared__ __align__(8) uint64_t wbar, bar_d, bar_k0, full_bar[TCW_STAGES], empty_bar[TCW_STAGES];
     __shared__ uint32_t tmem_slot;
     __shared__ float muS[NP][A][128];
     __shared__ float dmuS[A][128];
-    __shared__ double sred[4][16];
-    // objective / count / ratio / clip statistics of sample row e, accumulated over the CTA's tiles by the part-0
-    // thread of that row (shared memory instead of 8 registers per thread: the epilogues run at the 96-register cap)
-    __shared__ double statS[4][128];
+    __shared__ double sred[NS][16];
+    // objective / count / ratio / clip / KL statistics of sample row e, accumulated over the CTA's tiles by the part-0
+    // thread of that row (shared memory instead of 10 registers per thread: the epilogues run at the 96-register cap)
+    __shared__ double statS[NS][128];
     if ((smem_u32(smem_raw) & 1023u) != 0u) __trap();
-    for (int i = threadIdx.x; i < 4 * 128; i += blockDim.x) statS[i / 128][i % 128] = 0.0;
+    for (int i = threadIdx.x; i < NS * 128; i += blockDim.x) statS[i / 128][i % 128] = 0.0;
     unsigned char *ring = smem_raw;
     float *Rsm = reinterpret_cast<float *>(smem_raw + TCW_STAGES * CB);
     unsigned char *O_hi = reinterpret_cast<unsigned char *>(Rsm + a.lay.resident);
@@ -452,7 +458,7 @@ __global__ void __launch_bounds__(NP * 128 + 64, 1) update_tcw_fwdbwd_kernel(con
             finish_A(H1s, false);
             // the per-sample scalars of the objective (action, advantage / regression target, old log-prob): gathered
             // HERE, in the shadow of the forward GEMM, so that they do not occupy registers during epilogue 1
-            float av[A], adv = 0.f, olp = 0.f;
+            float av[A], adv = 0.f, olp = 0.f, lr = 0.f;
             int64_t n_own = 0;
 #pragma unroll
             for (int jj = 0; jj < A; ++jj) av[jj] = 0.0f;
@@ -471,6 +477,7 @@ __global__ void __launch_bounds__(NP * 128 + 64, 1) update_tcw_fwdbwd_kernel(con
                     for (int jj = 0; jj < A; ++jj) av[jj] = __ldg(a.act + ((int64_t)t * A + jj) * N + n);
                     adv = __ldg(a.adv + (int64_t)t * N + n);
                     olp = __ldg(a.oldlp + (int64_t)t * N + n);
+                    if (REF) lr = __ldg(a.reflp + (int64_t)t * N + n);
                 }
             }
             mbar_wait(&bar_d, ph_d);
@@ -549,6 +556,13 @@ __global__ void __launch_bounds__(NP * 128 + 64, 1) update_tcw_fwdbwd_kernel(con
                     if (a.kl_scale != 0.0f) {
                         eo = expf(olp);
                         dlp -= a.kl_scale * eo;
+                    }
+                    if (REF) {                      // k3 KL to the reference policy
+                        const float u = lr - lp, em = expm1f(u);
+                        const float dkl = em - u;
+                        dlp += a.ref_coef * em;
+                        statS[0][e] -= (double)a.ref_coef * dkl;
+                        statS[NS - 1][e] += dkl;
                     }
 #pragma unroll
                     for (int jj = 0; jj < A; ++jj) dmu[jj] = dlp * (av[jj] - mu[jj]) * a.inv_var[jj];
@@ -629,19 +643,19 @@ __global__ void __launch_bounds__(NP * 128 + 64, 1) update_tcw_fwdbwd_kernel(con
         float *gp = a.gpart + (int64_t)blockIdx.x * a.lay.n_params;
         const int64_t f2 = a.lay.flat_w[2];
         {
-            double v[4];
+            double v[NS];
 #pragma unroll
-            for (int kq = 0; kq < 4; ++kq) v[kq] = part == 0 ? statS[kq][e] : 0.0;
+            for (int kq = 0; kq < NS; ++kq) v[kq] = part == 0 ? statS[kq][e] : 0.0;
 #pragma unroll
-            for (int kq = 0; kq < 4; ++kq) {
+            for (int kq = 0; kq < NS; ++kq) {
                 for (int off = 16; off > 0; off >>= 1) v[kq] += __shfl_down_sync(0xffffffffu, v[kq], off);
                 if (lane == 0) sred[kq][warp] = v[kq];
             }
             asm volatile("bar.sync 8, %0;" ::"n"(NCT) : "memory");
-            if (threadIdx.x < 4 && a.spart) {
+            if (threadIdx.x < NS && a.spart) {
                 double tt = 0.0;
                 for (int w = 0; w < NP * 4; ++w) tt += sred[threadIdx.x][w];
-                a.spart[(int64_t)blockIdx.x * 4 + threadIdx.x] += tt;
+                a.spart[(int64_t)blockIdx.x * TG_SPART_LD + threadIdx.x] += tt;
             }
             asm volatile("bar.sync 8, %0;" ::"n"(NCT) : "memory");
 #pragma unroll
@@ -1001,8 +1015,10 @@ template <int O, int A, int W, int NP>
 static int launch_tcw_np(const TcwArgs &a0, int grid, int64_t total_upper, int64_t batch_tiles, cudaStream_t st) {
     constexpr int OKP = (O + 1 + 7) / 8 * 8;
     const size_t smemA = (size_t)TCW_STAGES * W * 128 + (size_t)a0.lay.resident * 4 + 2 * (size_t)128 * OKP * 4;
-    void (*kA)(const TcwArgs) = a0.lay.act == TG_ACT_RELU ? update_tcw_fwdbwd_kernel<O, A, true, W, NP>
-                                                          : update_tcw_fwdbwd_kernel<O, A, false, W, NP>;
+    void (*kA)(const TcwArgs) = a0.reflp ? (a0.lay.act == TG_ACT_RELU ? update_tcw_fwdbwd_kernel<O, A, true, W, NP, true>
+                                                                       : update_tcw_fwdbwd_kernel<O, A, false, W, NP, true>)
+                                         : (a0.lay.act == TG_ACT_RELU ? update_tcw_fwdbwd_kernel<O, A, true, W, NP, false>
+                                                                       : update_tcw_fwdbwd_kernel<O, A, false, W, NP, false>);
     // converter warps of kernel B: measured on B200 (profiles/README_r2.md) 8 / 12 / 16 warps = 293 / 267 / 241 us per
     // launch at W = 256 and 12 <= 16 at W = 128 (22 warps: no further gain, r2p)
     constexpr int NCV = W == 256 ? 16 : 12;
@@ -1037,12 +1053,12 @@ static int launch_tcw(const TcwArgs &a0, int grid, int64_t total_upper, int64_t 
     return launch_tcw_np<O, A, W, (W == 256 ? 4 : 2)>(a0, grid, total_upper, batch_tiles, st);
 }
 
-// gpart [sm_count][n_params] and spart [sm_count][4] must be zeroed by the caller.
+// gpart [sm_count][n_params] and spart [sm_count][TG_SPART_LD] must be zeroed by the caller.
 int tg_policy_grad_tcw(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N, int T, const float *obs, const float *act,
                        const float *adv, const float *old_logp, const float *target, const int32_t *len, const float *params,
                        const float *inv_sd, const float *inv_var, float log_norm, float eps_clip, float scale,
                        float kl_scale, float *gpart, double *spart, int grid, cudaStream_t st, float *out_mu,
-                       float *out_logp) {
+                       float *out_logp, const float *ref_logp, float ref_coef) {
     TcwArgs a;
     memset(&a, 0, sizeof(a));
     tg_build_tcw_layout(mlp, &a.lay, true);
@@ -1072,12 +1088,12 @@ int tg_policy_grad_tcw(tg_ctx *ctx, const tg_mlp_cfg *mlp, int64_t N, int T, con
     a.sc.base = reinterpret_cast<unsigned char *>(ctx->scratch) + tstart_bytes;
     tcw_tstart_kernel<<<1, 32, 0, st>>>(T, ctx->cnt, tstart);
     TG_CUDA(cudaGetLastError());
-    a.N = N; a.T = T; a.obs = obs; a.act = act; a.adv = adv; a.oldlp = old_logp; a.target = target;
+    a.N = N; a.T = T; a.obs = obs; a.act = act; a.adv = adv; a.oldlp = old_logp; a.target = target; a.reflp = ref_logp;
     a.perm = ctx->perm; a.cnt = ctx->cnt; a.tstart = tstart;
     a.packed = ctx->packed_tc;
     a.params = params;
     for (int j = 0; j < TG_MAX_ACT; ++j) { a.inv_sd[j] = inv_sd ? inv_sd[j] : 1.0f; a.inv_var[j] = inv_var ? inv_var[j] : 1.0f; }
-    a.log_norm = log_norm; a.eps_clip = eps_clip; a.scale = scale; a.kl_scale = kl_scale;
+    a.log_norm = log_norm; a.eps_clip = eps_clip; a.scale = scale; a.kl_scale = kl_scale; a.ref_coef = ref_coef;
     a.gpart = gpart; a.spart = spart;
     a.out_mu = out_mu; a.out_logp = out_logp;
     a.forward_only = (out_mu != nullptr || out_logp != nullptr) ? 1 : 0;

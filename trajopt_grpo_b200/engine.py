@@ -295,8 +295,12 @@ def advantage_ppo_normalize(T, length, sums, adv, rtg):
 
 
 def policy_grad(dims, activation, params, cov_diag, obs, act, adv, old_logp, length, eps_clip, scale, kl_scale=0.0,
-                out_grad=None):
-    """tg_policy_grad -> (grad [n_params], stats [4] = objective, n_valid, sum ratio, n_clipped)."""
+                out_grad=None, ref_logp=None, ref_scale=0.0):
+    """tg_policy_grad -> (grad [n_params], stats [4] = objective, n_valid, sum ratio, n_clipped).
+
+    With `ref_logp` [T,N] (log-probs of `act` under a frozen reference policy): tg_policy_grad_ref, GRPO's k3 KL
+    penalty -ref_scale * sum(exp(u) - u - 1), u = ref_logp - logp, added to the objective (ref_scale = beta * scale),
+    and stats [5] = objective, n_valid, sum ratio, n_clipped, sum(exp(u) - u - 1)."""
     lib = L.load()
     T, O, N = obs.shape
     A = act.shape[1]
@@ -306,15 +310,24 @@ def policy_grad(dims, activation, params, cov_diag, obs, act, adv, old_logp, len
     _need(old_logp, torch.float32, "old_logp", (T, N))
     _need(length, torch.int32, "len", (N,))
     _need(params, torch.float32, "params")
+    if ref_logp is not None:
+        _need(ref_logp, torch.float32, "ref_logp", (T, N))
     dev = obs.device
     mcfg = L.mlp_cfg(dims, activation)
     grad = torch.empty_like(params) if out_grad is None else out_grad
-    stats = torch.empty((4,), dtype=torch.float32, device=dev)
+    stats = torch.empty((4 if ref_logp is None else 5,), dtype=torch.float32, device=dev)
     with torch.cuda.device(dev):
         ws = _workspace("grad", lib.tg_policy_grad_workspace_bytes(L.ctx(dev), C.byref(mcfg)), dev)
-        rc = lib.tg_policy_grad(L.ctx(dev), C.byref(mcfg), N, T, L.ptr(obs), L.ptr(act), L.ptr(adv), L.ptr(old_logp),
-                                L.ptr(length), L.ptr(params), L.cov_array(cov_diag), float(eps_clip), float(scale),
-                                float(kl_scale), L.ptr(grad), L.ptr(stats), L.ptr(ws), L.stream_ptr())
+        if ref_logp is None:
+            rc = lib.tg_policy_grad(L.ctx(dev), C.byref(mcfg), N, T, L.ptr(obs), L.ptr(act), L.ptr(adv),
+                                    L.ptr(old_logp), L.ptr(length), L.ptr(params), L.cov_array(cov_diag),
+                                    float(eps_clip), float(scale), float(kl_scale), L.ptr(grad), L.ptr(stats),
+                                    L.ptr(ws), L.stream_ptr())
+        else:
+            rc = lib.tg_policy_grad_ref(L.ctx(dev), C.byref(mcfg), N, T, L.ptr(obs), L.ptr(act), L.ptr(adv),
+                                        L.ptr(old_logp), L.ptr(ref_logp), L.ptr(length), L.ptr(params),
+                                        L.cov_array(cov_diag), float(eps_clip), float(scale), float(kl_scale),
+                                        float(ref_scale), L.ptr(grad), L.ptr(stats), L.ptr(ws), L.stream_ptr())
     L.check(rc, "tg_policy_grad")
     _count(3 if length_order.held else 5)          # pack, [order_keys, order_count,] update, grad_reduce
     return grad, stats
