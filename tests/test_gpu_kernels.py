@@ -171,6 +171,34 @@ def test_rollout_philox_equals_explicit_noise(E, golden_dir):
         assert torch.equal(a[k], b[k]), k
 
 
+@pytest.mark.parametrize("hidden", [[32, 32], [64, 64], [128, 128], [256, 256]],
+                         ids=["fp32", "tc64", "tc128", "tc256"])
+def test_rollout_kernels_philox_and_without_logp(E, hidden):
+    """Each of the four rollout kernels (FP32 pipe, tensor cores at width 64, 128 and 256) draws in-kernel Philox
+    noise exactly as tg_noise_fill materialises it, and leaves its other outputs bit-identical when it writes no
+    log-probs (PPO.learn_streamed rolls out without them)."""
+    kind, T, N, A = 3, 60, 300, 4
+    rng = np.random.default_rng(17)
+    dims = [R.OBS_DIM[kind]] + hidden + [A]
+    Ws = [(rng.standard_normal((dims[i + 1], dims[i])) / np.sqrt(dims[i])).astype(np.float32) for i in range(len(dims) - 1)]
+    bs = [(0.1 * rng.standard_normal(dims[i + 1])).astype(np.float32) for i in range(len(dims) - 1)]
+    params, init = dev(_flat(Ws, bs)), dev(R.reset_states(kind, N, rng).T.copy(), torch.float32)
+
+    def run(**kw):
+        out = E.rollout(kind, T, R.DEFAULT_DT[kind], dims, "ReLU", params, [0.3] * A, init, env_offset=5, **kw)
+        torch.cuda.synchronize()
+        return out
+
+    a = run(noise=E.noise_fill(99, N, T, A, env_offset=5))
+    b = run(seed=99)
+    c = run(seed=99, want_logp=False)
+    for k in ("obs", "act", "rew", "logp", "len", "ret"):
+        assert torch.equal(a[k], b[k]), k
+    assert c["logp"] is None
+    for k in ("obs", "act", "rew", "len", "ret"):
+        assert torch.equal(b[k], c[k]), k
+
+
 @pytest.mark.parametrize("hidden,kind", [([64, 64], 1), ([128, 128], 2), ([256, 256], 3), ([128, 128, 128, 128], 0),
                                          ([40, 24], 2), ([], 1)])
 def test_rollout_matches_oracle_all_tile_configs(E, hidden, kind):

@@ -10,6 +10,8 @@
 // where `s` is advanced in place, `bal` is the Pendulum balanced-step counter; WRAPPED = the action is
 // already the wrapped control (Env._dynamics' argument) instead of the raw policy sample.
 #pragma once
+#include <type_traits>
+
 #include "tg_common.cuh"
 
 struct EnvParams {
@@ -23,6 +25,18 @@ struct EnvParams {
     //   Pendulum: k[0] = 1 / (mass * length**2), k[1] = mass * gravity * length
     double k[5];
 };
+// validates `env` and derives its EnvParams (tg_rollout.cu)
+int tg_fill_env_params(const tg_env_cfg *env, EnvParams *p);
+
+// Calls f(std::integral_constant<int, KIND>()) for the env kind of a validated tg_env_cfg.
+template <typename F> auto tg_with_env_kind(int kind, F &&f) {
+    switch (kind) {
+        case TG_ENV_CARTPOLE: return f(std::integral_constant<int, TG_ENV_CARTPOLE>());
+        case TG_ENV_PENDULUM: return f(std::integral_constant<int, TG_ENV_PENDULUM>());
+        case TG_ENV_QUADPOLE2D: return f(std::integral_constant<int, TG_ENV_QUADPOLE2D>());
+        default: return f(std::integral_constant<int, TG_ENV_QUADPOLE>());
+    }
+}
 
 template <typename R> struct Mth;
 template <> struct Mth<float> {

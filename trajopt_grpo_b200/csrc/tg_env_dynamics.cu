@@ -3,8 +3,6 @@
 // pendulum_env.py:48-75, quadrotor_env.py:417-528, 1044-1130).  Reward and termination are discarded.
 #include "tg_env.cuh"
 
-int tg_fill_env_params(const tg_env_cfg *env, EnvParams *p);   // tg_rollout.cu
-
 template <int KIND, typename R>
 __global__ void env_dynamics_kernel(EnvParams p, int64_t N, const R *__restrict__ state, const float *__restrict__ control,
                                     R *__restrict__ next) {
@@ -46,10 +44,7 @@ extern "C" int tg_env_dynamics(tg_ctx *ctx, const tg_env_cfg *env, int precision
     if (rc) return rc;
     TG_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = (cudaStream_t)stream;
-    switch (env->kind) {
-        case TG_ENV_CARTPOLE: return launch<TG_ENV_CARTPOLE>(precision, p, N, state, control, next_state, st);
-        case TG_ENV_PENDULUM: return launch<TG_ENV_PENDULUM>(precision, p, N, state, control, next_state, st);
-        case TG_ENV_QUADPOLE2D: return launch<TG_ENV_QUADPOLE2D>(precision, p, N, state, control, next_state, st);
-        default: return launch<TG_ENV_QUADPOLE>(precision, p, N, state, control, next_state, st);
-    }
+    return tg_with_env_kind(env->kind, [&](auto kind) {
+        return launch<decltype(kind)::value>(precision, p, N, state, control, next_state, st);
+    });
 }

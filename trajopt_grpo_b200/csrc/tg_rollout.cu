@@ -16,36 +16,15 @@
 //     done, then the CTA only zero-fills the remaining rows.
 #include <math.h>
 
-#include "tg_env.cuh"
 #include "tg_mlp.cuh"
+#include "tg_rollout.cuh"
 #include "tg_umma.cuh"
 
-// tg_rollout_tc256.cu
-bool tg_tc256_eligible(const tg_mlp_cfg *mlp);
-int tg_rollout_tc256(tg_ctx *ctx, const tg_env_cfg *env, const EnvParams &ep, const tg_mlp_cfg *mlp, int precision,
-                     int64_t N, const void *init_state, const float *params, const float *sd, float log_norm,
-                     const float *noise, uint64_t seed, int64_t env_offset, float *out_obs, float *out_act, float *out_rew,
-                     float *out_logp, int32_t *out_len, float *out_ret, cudaStream_t st);
-
-struct RolloutArgs {
-    EnvParams env;
-    tg_mlp_layout lay;
-    int64_t N;
-    const void *init_state;
-    const float *packed;
-    const float *noise;
-    uint64_t seed;
-    int64_t env_offset;
-    float sd[TG_MAX_ACT], log_norm;
-    float *obs, *act, *rew, *logp, *ret;
-    int32_t *len;
-};
-
 template <int KIND, typename R, int CFG, bool WG>
-__global__ void __launch_bounds__(TileCfg<CFG>::NT) rollout_kernel(const __grid_constant__ RolloutArgs a) {
-    using E = Env<KIND>;
+__global__ void __launch_bounds__(TileCfg<CFG>::NT) rollout_kernel(const __grid_constant__ RolloutArgs<tg_mlp_layout> a) {
+    using Ev = RolloutEnv<KIND, R>;
     constexpr int B = TileCfg<CFG>::B, NT = TileCfg<CFG>::NT, LDX = B + 4;
-    constexpr int S = E::S, A = E::A;
+    constexpr int S = Ev::S, A = Ev::A;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ __align__(8) uint64_t wbar;
     float *Ws = reinterpret_cast<float *>(smem_raw);
@@ -55,34 +34,19 @@ __global__ void __launch_bounds__(TileCfg<CFG>::NT) rollout_kernel(const __grid_
     const float *W = WG ? a.packed : Ws;
     if (!WG) stage_weights_tma(Ws, a.packed, a.lay.total, &wbar);
 
-    const int T = a.env.max_steps;
-    const int64_t N = a.N;
+    const int T = a.io.env.max_steps;
     const int64_t n = (int64_t)blockIdx.x * B + threadIdx.x;
     const bool owner = threadIdx.x < B;
-    const bool real_env = owner && n < N;
-    bool alive = real_env;
-    R s[S];
-    int steps = 0, bal = 0;
-    float ret = 0.0f;
-    if (real_env) {
-        const R *init = reinterpret_cast<const R *>(a.init_state);
-#pragma unroll
-        for (int i = 0; i < S; ++i) s[i] = init[(int64_t)i * N + n];
-    } else {
-#pragma unroll
-        for (int i = 0; i < S; ++i) s[i] = (R)0;
-    }
+    Ev ev(a.io, n, owner && n < a.io.N, true);      // only owner threads hold an env
     const int nl = a.lay.n_layers;
     int t = 0;
     for (; t < T; ++t) {
-        // 1. publish the observation (stored BEFORE acting, rollout_worker.py:53)
+        // 1. publish the observation
         if (owner) {
+            float x[S];
+            ev.observe(a.io, t, x);
 #pragma unroll
-            for (int i = 0; i < S; ++i) {
-                const float o = alive ? (float)s[i] : 0.0f;
-                Xa[i * LDX + threadIdx.x] = o;
-                if (real_env) a.obs[((int64_t)t * S + i) * N + n] = o;
-            }
+            for (int i = 0; i < S; ++i) Xa[i * LDX + threadIdx.x] = x[i];
         }
         __syncthreads();
         // 2. hidden layers (ping-pong Xa <-> Xb)
@@ -96,72 +60,26 @@ __global__ void __launch_bounds__(TileCfg<CFG>::NT) rollout_kernel(const __grid_
         float mu[A];
         tile_output_layer<CFG, A, WG>(W + a.lay.L[nl - 1].wt, W + a.lay.L[nl - 1].bias, xin, P, a.lay.L[nl - 1].K, mu);
         // 4. sample, step the env, write the trajectory rows
-        if (owner) {
-            float act[A], lp = 0.0f, rw = 0.0f;
-            if (alive) {
-                float eps[4];
-                if (a.noise != nullptr) {
-#pragma unroll
-                    for (int j = 0; j < A; ++j) eps[j] = a.noise[((int64_t)t * A + j) * N + n];
-                } else {
-                    philox_normal4(a.seed, (uint64_t)(a.env_offset + n), (uint32_t)t, eps);
-                }
-                float m2 = 0.0f;
-#pragma unroll
-                for (int j = 0; j < A; ++j) {
-                    act[j] = mu[j] + a.sd[j] * eps[j];          // MultivariateNormal.rsample
-                    const float z = (act[j] - mu[j]) / a.sd[j];
-                    m2 += z * z;
-                }
-                lp = -0.5f * m2 - a.log_norm;
-                R r;
-                const bool done = E::template step<R>(s, act, a.env, steps, bal, r);
-                rw = (float)r;
-                ret += rw;
-                steps += 1;
-                alive = !done;
-            } else {
-#pragma unroll
-                for (int j = 0; j < A; ++j) act[j] = 0.0f;
-            }
-            if (real_env) {
-#pragma unroll
-                for (int j = 0; j < A; ++j) a.act[((int64_t)t * A + j) * N + n] = act[j];
-                a.rew[(int64_t)t * N + n] = rw;
-                if (a.logp) a.logp[(int64_t)t * N + n] = lp;
-            }
-        }
+        if (owner) ev.act(a.io, t, mu);
         // 5. tile-wide early exit; also the barrier that protects Xa/Xb/P reuse
-        if (!__syncthreads_or(alive ? 1 : 0)) { ++t; break; }
+        if (!__syncthreads_or(ev.alive ? 1 : 0)) { ++t; break; }
     }
-    // zero-fill the rows after every env of the tile finished (rollout_worker.py:64-68 padding)
-    if (real_env) {
-        for (; t < T; ++t) {
-#pragma unroll
-            for (int i = 0; i < S; ++i) a.obs[((int64_t)t * S + i) * N + n] = 0.0f;
-#pragma unroll
-            for (int j = 0; j < A; ++j) a.act[((int64_t)t * A + j) * N + n] = 0.0f;
-            a.rew[(int64_t)t * N + n] = 0.0f;
-            if (a.logp) a.logp[(int64_t)t * N + n] = 0.0f;
-        }
-        a.len[n] = steps;
-        if (a.ret) a.ret[n] = ret;
-    }
+    ev.finish(a.io, t);
 }
 
 template <int KIND, typename R, int CFG, bool WG>
-static int launch_rollout(const RolloutArgs &a, size_t smem, cudaStream_t st) {
+static int launch_rollout(const RolloutArgs<tg_mlp_layout> &a, size_t smem, cudaStream_t st) {
     constexpr int B = TileCfg<CFG>::B, NT = TileCfg<CFG>::NT;
     auto kern = rollout_kernel<KIND, R, CFG, WG>;
     TG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const unsigned grid = (unsigned)((a.N + B - 1) / B);
+    const unsigned grid = (unsigned)((a.io.N + B - 1) / B);
     kern<<<grid, NT, smem, st>>>(a);
     TG_CUDA(cudaGetLastError());
     return TG_OK;
 }
 
 template <int KIND, typename R>
-static int dispatch_cfg(const RolloutArgs &a, size_t smem, bool wg, cudaStream_t st) {
+static int dispatch_cfg(const RolloutArgs<tg_mlp_layout> &a, size_t smem, bool wg, cudaStream_t st) {
     if (wg) {
         switch (a.lay.cfg) {
             case 0: return launch_rollout<KIND, R, 0, true>(a, smem, st);
@@ -176,12 +94,6 @@ static int dispatch_cfg(const RolloutArgs &a, size_t smem, bool wg, cudaStream_t
     }
 }
 
-template <int KIND>
-static int dispatch_prec(int precision, const RolloutArgs &a, size_t smem, bool wg, cudaStream_t st) {
-    return precision == TG_PREC_F64 ? dispatch_cfg<KIND, double>(a, smem, wg, st)
-                                    : dispatch_cfg<KIND, float>(a, smem, wg, st);
-}
-
 // ---------------------------------------------------------------------------
 // Tensor-core variant (TG_MATH_AUTO / TG_MATH_3XTF32, eligible policies: tg_tc_eligible).
 // 128 threads, thread i = env i of the tile = TMEM lane i.  Per step each thread evaluates
@@ -192,25 +104,11 @@ static int dispatch_prec(int precision, const RolloutArgs &a, size_t smem, bool 
 // comes back from TMEM with tcgen05.ld -- each thread receives exactly its env's row --
 // and bias/activation/output layer/sampling/dynamics continue in registers.
 // ---------------------------------------------------------------------------
-struct RolloutTcArgs {
-    EnvParams env;
-    tg_tc_layout lay;
-    int64_t N;
-    const void *init_state;
-    const float *packed;
-    const float *noise;
-    uint64_t seed;
-    int64_t env_offset;
-    float sd[TG_MAX_ACT], log_norm;
-    float *obs, *act, *rew, *logp, *ret;
-    int32_t *len;
-};
-
 // RELU: the activation is known at compile time (no per-element branch); otherwise a.lay.act
 template <int KIND, typename R, bool RELU>
-__global__ void __launch_bounds__(128) rollout_tc_kernel(const __grid_constant__ RolloutTcArgs a) {
-    using E = Env<KIND>;
-    constexpr int S = E::S, A = E::A, W = TC_W, O4 = (S + 1 + 3) / 4 * 4;
+__global__ void __launch_bounds__(128) rollout_tc_kernel(const __grid_constant__ RolloutArgs<tg_tc_layout> a) {
+    using Ev = RolloutEnv<KIND, R>;
+    constexpr int S = Ev::S, A = Ev::A, W = TC_W, O4 = (S + 1 + 3) / 4 * 4;
     // 1024-byte alignment comes from the declaration (no integer pointer arithmetic, so the
     // compiler keeps every access below in the shared address space: LDS/STS, not generic LD)
     extern __shared__ __align__(1024) unsigned char smem_raw[];
@@ -238,33 +136,16 @@ __global__ void __launch_bounds__(128) rollout_tc_kernel(const __grid_constant__
     // this thread's row of the [128][W] activation operand in the core-matrix layout
     const uint32_t row_off = (uint32_t)(threadIdx.x >> 3) * (uint32_t)(W / 4) * 128u + (uint32_t)(threadIdx.x & 7) * 16u;
 
-    const int T = a.env.max_steps;
-    const int64_t N = a.N;
+    const int T = a.io.env.max_steps;
     const int64_t n = (int64_t)blockIdx.x * 128 + threadIdx.x;
-    const bool real_env = n < N;
-    bool alive = real_env;
-    R s[S];
-    int steps = 0, bal = 0;
-    float ret = 0.0f;
-    if (real_env) {
-        const R *init = reinterpret_cast<const R *>(a.init_state);
-#pragma unroll
-        for (int i = 0; i < S; ++i) s[i] = init[(int64_t)i * N + n];
-    } else {
-#pragma unroll
-        for (int i = 0; i < S; ++i) s[i] = (R)0;
-    }
+    Ev ev(a.io, n, n < a.io.N, true);
     const int nh = a.lay.nh, act_kind = RELU ? TG_ACT_RELU : a.lay.act;
     const float *w1 = Wsm + a.lay.w1;
     uint32_t phase = 0;
     int t = 0;
     for (; t < T; ++t) {
         float x[S];
-#pragma unroll
-        for (int i = 0; i < S; ++i) {
-            x[i] = alive ? (float)s[i] : 0.0f;
-            if (real_env) a.obs[((int64_t)t * S + i) * N + n] = x[i];
-        }
+        ev.observe(a.io, t, x);
         // first Linear on the FP32 pipe (K = obs dim is tiny): h = act(W1 x + b1)
         float h[W];
 #pragma unroll
@@ -336,53 +217,10 @@ __global__ void __launch_bounds__(128) rollout_tc_kernel(const __grid_constant__
                 mu[j] = acc;
             }
         }
-        float act[A], lp = 0.0f, rw = 0.0f;
-        if (alive) {
-            float eps[4];
-            if (a.noise != nullptr) {
-#pragma unroll
-                for (int j = 0; j < A; ++j) eps[j] = a.noise[((int64_t)t * A + j) * N + n];
-            } else {
-                philox_normal4(a.seed, (uint64_t)(a.env_offset + n), (uint32_t)t, eps);
-            }
-            float m2 = 0.0f;
-#pragma unroll
-            for (int j = 0; j < A; ++j) {
-                act[j] = mu[j] + a.sd[j] * eps[j];
-                const float z = (act[j] - mu[j]) / a.sd[j];
-                m2 += z * z;
-            }
-            lp = -0.5f * m2 - a.log_norm;
-            R r;
-            const bool done = E::template step<R>(s, act, a.env, steps, bal, r);
-            rw = (float)r;
-            ret += rw;
-            steps += 1;
-            alive = !done;
-        } else {
-#pragma unroll
-            for (int j = 0; j < A; ++j) act[j] = 0.0f;
-        }
-        if (real_env) {
-#pragma unroll
-            for (int j = 0; j < A; ++j) a.act[((int64_t)t * A + j) * N + n] = act[j];
-            a.rew[(int64_t)t * N + n] = rw;
-            if (a.logp) a.logp[(int64_t)t * N + n] = lp;
-        }
-        if (!__syncthreads_or(alive ? 1 : 0)) { ++t; break; }
+        ev.act(a.io, t, mu);
+        if (!__syncthreads_or(ev.alive ? 1 : 0)) { ++t; break; }
     }
-    if (real_env) {
-        for (; t < T; ++t) {
-#pragma unroll
-            for (int i = 0; i < S; ++i) a.obs[((int64_t)t * S + i) * N + n] = 0.0f;
-#pragma unroll
-            for (int j = 0; j < A; ++j) a.act[((int64_t)t * A + j) * N + n] = 0.0f;
-            a.rew[(int64_t)t * N + n] = 0.0f;
-            if (a.logp) a.logp[(int64_t)t * N + n] = 0.0f;
-        }
-        a.len[n] = steps;
-        if (a.ret) a.ret[n] = ret;
-    }
+    ev.finish(a.io, t);
     tc_fence_before();
     __syncthreads();
     if (threadIdx.x < 32) tmem_dealloc(tmem, 64);
@@ -400,9 +238,9 @@ __global__ void __launch_bounds__(128) rollout_tc_kernel(const __grid_constant__
 // output-layer dot product meet in shared memory (fixed order -> deterministic).
 // ---------------------------------------------------------------------------
 template <int KIND, typename R, bool RELU, int W>
-__global__ void __launch_bounds__(256, 1) rollout_tc2_kernel(const __grid_constant__ RolloutTcArgs a) {
-    using E = Env<KIND>;
-    constexpr int S = E::S, A = E::A, HW = W / 2, O4 = (S + 1 + 3) / 4 * 4;
+__global__ void __launch_bounds__(256, 1) rollout_tc2_kernel(const __grid_constant__ RolloutArgs<tg_tc_layout> a) {
+    using Ev = RolloutEnv<KIND, R>;
+    constexpr int S = Ev::S, A = Ev::A, HW = W / 2, O4 = (S + 1 + 3) / 4 * 4;
     constexpr uint32_t TM_D = 0u, TM_AHI = (uint32_t)W, TM_ALO = 2u * (uint32_t)W;
     constexpr uint32_t TM_COLS = 512u;
     extern __shared__ __align__(1024) unsigned char smem_raw[];
@@ -429,34 +267,16 @@ __global__ void __launch_bounds__(256, 1) rollout_tc2_kernel(const __grid_consta
     const int c0 = hf * HW;                       // first column of this thread's half
     const uint32_t my_tm = tmem + ((uint32_t)(q * 32) << 16);
 
-    const int T = a.env.max_steps;
-    const int64_t N = a.N;
+    const int T = a.io.env.max_steps;
     const int64_t n = (int64_t)blockIdx.x * 128 + e;
-    const bool real_env = n < N;
-    const bool writer = real_env && hf == 0;
-    bool alive = real_env;
-    R s[S];
-    int steps = 0, bal = 0;
-    float ret = 0.0f;
-    if (real_env) {
-        const R *init = reinterpret_cast<const R *>(a.init_state);
-#pragma unroll
-        for (int i = 0; i < S; ++i) s[i] = init[(int64_t)i * N + n];
-    } else {
-#pragma unroll
-        for (int i = 0; i < S; ++i) s[i] = (R)0;
-    }
+    Ev ev(a.io, n, n < a.io.N, hf == 0);          // both threads step the env, the hf == 0 one records it
     const int nh = a.lay.nh, act_kind = RELU ? TG_ACT_RELU : a.lay.act;
     const float *w1 = Wsm + a.lay.w1 + (size_t)c0 * O4;
     uint32_t phase = 0;
     int t = 0;
     for (; t < T; ++t) {
         float x[S];
-#pragma unroll
-        for (int i = 0; i < S; ++i) {
-            x[i] = alive ? (float)s[i] : 0.0f;
-            if (writer) a.obs[((int64_t)t * S + i) * N + n] = x[i];
-        }
+        ev.observe(a.io, t, x);
         // first Linear on the FP32 pipe, this thread's HW neurons: h = act(W1 x + b1)
         float h[HW];
 #pragma unroll
@@ -547,82 +367,28 @@ __global__ void __launch_bounds__(256, 1) rollout_tc2_kernel(const __grid_consta
 #pragma unroll
             for (int j = 0; j < A; ++j) mu[j] = (bo[j] + muS[0][j][e]) + muS[1][j][e];
         }
-        float act[A], lp = 0.0f, rw = 0.0f;
-        if (alive) {
-            float eps[4];
-            if (a.noise != nullptr) {
-#pragma unroll
-                for (int j = 0; j < A; ++j) eps[j] = a.noise[((int64_t)t * A + j) * N + n];
-            } else {
-                philox_normal4(a.seed, (uint64_t)(a.env_offset + n), (uint32_t)t, eps);
-            }
-            float m2 = 0.0f;
-#pragma unroll
-            for (int j = 0; j < A; ++j) {
-                act[j] = mu[j] + a.sd[j] * eps[j];
-                const float z = (act[j] - mu[j]) / a.sd[j];
-                m2 += z * z;
-            }
-            lp = -0.5f * m2 - a.log_norm;
-            R r;
-            const bool done = E::template step<R>(s, act, a.env, steps, bal, r);
-            rw = (float)r;
-            ret += rw;
-            steps += 1;
-            alive = !done;
-        } else {
-#pragma unroll
-            for (int j = 0; j < A; ++j) act[j] = 0.0f;
-        }
-        if (writer) {
-#pragma unroll
-            for (int j = 0; j < A; ++j) a.act[((int64_t)t * A + j) * N + n] = act[j];
-            a.rew[(int64_t)t * N + n] = rw;
-            if (a.logp) a.logp[(int64_t)t * N + n] = lp;
-        }
-        if (!__syncthreads_or(alive ? 1 : 0)) { ++t; break; }
+        ev.act(a.io, t, mu);
+        if (!__syncthreads_or(ev.alive ? 1 : 0)) { ++t; break; }
     }
-    if (writer) {
-        for (; t < T; ++t) {
-#pragma unroll
-            for (int i = 0; i < S; ++i) a.obs[((int64_t)t * S + i) * N + n] = 0.0f;
-#pragma unroll
-            for (int j = 0; j < A; ++j) a.act[((int64_t)t * A + j) * N + n] = 0.0f;
-            a.rew[(int64_t)t * N + n] = 0.0f;
-            if (a.logp) a.logp[(int64_t)t * N + n] = 0.0f;
-        }
-        a.len[n] = steps;
-        if (a.ret) a.ret[n] = ret;
-    }
+    ev.finish(a.io, t);
     tc_fence_before();
     __syncthreads();
     if (threadIdx.x < 32) tmem_dealloc(tmem, TM_COLS);
 }
 
-template <int KIND, int W>
-static int launch_rollout_tc2(int precision, const RolloutTcArgs &a, cudaStream_t st) {
-    const size_t smem = ((size_t)a.lay.total * 4 + 1023) / 1024 * 1024;
-    const unsigned grid = (unsigned)((a.N + 127) / 128);
-    void (*kern)(const RolloutTcArgs);
-    const bool relu = a.lay.act == TG_ACT_RELU;
-    if (precision == TG_PREC_F64) kern = relu ? rollout_tc2_kernel<KIND, double, true, W> : rollout_tc2_kernel<KIND, double, false, W>;
-    else kern = relu ? rollout_tc2_kernel<KIND, float, true, W> : rollout_tc2_kernel<KIND, float, false, W>;
+// width 64: rollout_tc_kernel; width 128: rollout_tc2_kernel
+static int launch_rollout_tc(int kind, int precision, const RolloutArgs<tg_tc_layout> &a, cudaStream_t st) {
+    const bool w128 = a.lay.W == 128;
+    const size_t wbytes = ((size_t)a.lay.total * 4 + 1023) / 1024 * 1024;
+    const size_t smem = w128 ? wbytes : 1024 + wbytes + 2 * 128 * TC_W * 4;
+    auto kern = tg_with_env_kind(kind, [&](auto k) {
+        return tg_with_prec_relu(precision, a.lay.act, [&](auto r, auto relu) {
+            return w128 ? rollout_tc2_kernel<decltype(k)::value, decltype(r), decltype(relu)::value, 128>
+                        : rollout_tc_kernel<decltype(k)::value, decltype(r), decltype(relu)::value>;
+        });
+    });
     TG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<grid, 256, smem, st>>>(a);
-    TG_CUDA(cudaGetLastError());
-    return TG_OK;
-}
-
-template <int KIND>
-static int launch_rollout_tc(int precision, const RolloutTcArgs &a, cudaStream_t st) {
-    const size_t smem = 1024 + ((size_t)a.lay.total * 4 + 1023) / 1024 * 1024 + 2 * 128 * TC_W * 4;
-    const unsigned grid = (unsigned)((a.N + 127) / 128);
-    void (*kern)(const RolloutTcArgs);
-    const bool relu = a.lay.act == TG_ACT_RELU;
-    if (precision == TG_PREC_F64) kern = relu ? rollout_tc_kernel<KIND, double, true> : rollout_tc_kernel<KIND, double, false>;
-    else kern = relu ? rollout_tc_kernel<KIND, float, true> : rollout_tc_kernel<KIND, float, false>;
-    TG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<grid, 128, smem, st>>>(a);
+    kern<<<(unsigned)((a.io.N + 127) / 128), w128 ? 256 : 128, smem, st>>>(a);
     TG_CUDA(cudaGetLastError());
     return TG_OK;
 }
@@ -651,7 +417,6 @@ int tg_fill_env_params(const tg_env_cfg *env, EnvParams *p) {
     }
     return TG_OK;
 }
-static int fill_env_params(const tg_env_cfg *env, EnvParams *p) { return tg_fill_env_params(env, p); }
 
 extern "C" int tg_rollout(tg_ctx *ctx, const tg_env_cfg *env, const tg_mlp_cfg *mlp, int precision, int64_t N,
                           const void *init_state, const float *params, const float *cov_diag, const float *noise,
@@ -662,9 +427,9 @@ extern "C" int tg_rollout(tg_ctx *ctx, const tg_env_cfg *env, const tg_mlp_cfg *
                TG_ERR_ARG, "tg_rollout: null argument");
     TG_REQUIRE(N > 0, TG_ERR_SHAPE, "tg_rollout: N must be positive");
     TG_REQUIRE(precision == TG_PREC_F32 || precision == TG_PREC_F64, TG_ERR_ARG, "bad precision %d", precision);
-    RolloutArgs a;
-    memset(&a, 0, sizeof(a));
-    int rc = fill_env_params(env, &a.env);
+    RolloutIo io;
+    memset(&io, 0, sizeof(io));
+    int rc = tg_fill_env_params(env, &io.env);
     if (rc) return rc;
     int O, A;
     tg_env_dims(env->kind, &O, &A);
@@ -672,58 +437,43 @@ extern "C" int tg_rollout(tg_ctx *ctx, const tg_env_cfg *env, const tg_mlp_cfg *
                mlp->n_layers, TG_MAX_LAYERS);
     TG_REQUIRE(mlp->dims[0] == O && mlp->dims[mlp->n_layers] == A, TG_ERR_SHAPE,
                "policy dims (%d -> %d) do not match env obs/act dims (%d/%d)", mlp->dims[0], mlp->dims[mlp->n_layers], O, A);
-    rc = tg_gauss_consts(cov_diag, A, a.sd, nullptr, nullptr, &a.log_norm);
+    rc = tg_gauss_consts(cov_diag, A, io.sd, nullptr, nullptr, &io.log_norm);
     if (rc) return rc;
+    io.N = N;
+    io.init_state = init_state;
+    io.noise = noise;
+    io.seed = seed;
+    io.env_offset = env_offset;
+    io.obs = out_obs; io.act = out_act; io.rew = out_rew; io.logp = out_logp; io.len = out_len; io.ret = out_ret;
     cudaStream_t st = (cudaStream_t)stream;
     TG_CUDA(cudaSetDevice(ctx->device));
     // ---- tensor-core paths (3xTF32 tcgen05) for eligible policies
     if (tg_tc256_eligible(mlp) && ctx->math_mode != TG_MATH_FP32)      // 256-wide: weights streamed from L2
-        return tg_rollout_tc256(ctx, env, a.env, mlp, precision, N, init_state, params, a.sd, a.log_norm, noise, seed,
-                                env_offset, out_obs, out_act, out_rew, out_logp, out_len, out_ret, st);
+        return tg_rollout_tc256(ctx, mlp, precision, env->kind, params, io, st);
     const bool tc_ok = tg_tc_eligible(mlp);
     TG_REQUIRE(ctx->math_mode != TG_MATH_3XTF32 || tc_ok, TG_ERR_UNSUPPORTED,
                "TG_MATH_3XTF32 requested but the policy shape is not eligible (>= 2 hidden layers of equal width 64 or 128)");
     if (tc_ok && ctx->math_mode != TG_MATH_FP32) {
-        RolloutTcArgs b;
+        RolloutArgs<tg_tc_layout> b;
         memset(&b, 0, sizeof(b));
-        b.env = a.env;
+        b.io = io;
         rc = tg_build_tc_layout(mlp, &b.lay);
         if (rc) return rc;
         rc = tg_pack_weights_tc(ctx, b.lay, params, st);
         if (rc) return rc;
-        b.N = N; b.init_state = init_state; b.packed = ctx->packed_tc; b.noise = noise; b.seed = seed;
-        b.env_offset = env_offset;
-        memcpy(b.sd, a.sd, sizeof(b.sd));
-        b.log_norm = a.log_norm;
-        b.obs = out_obs; b.act = out_act; b.rew = out_rew; b.logp = out_logp; b.len = out_len; b.ret = out_ret;
+        b.packed = ctx->packed_tc;
         TG_REQUIRE(((size_t)b.lay.total * 4 + 1023) / 1024 * 1024 + 4096 <= (size_t)ctx->smem_optin, TG_ERR_UNSUPPORTED,
                    "staged tensor-core weights need %zu B of shared memory", (size_t)b.lay.total * 4);
-        if (b.lay.W == 128) {
-            switch (env->kind) {
-                case TG_ENV_CARTPOLE: return launch_rollout_tc2<TG_ENV_CARTPOLE, 128>(precision, b, st);
-                case TG_ENV_PENDULUM: return launch_rollout_tc2<TG_ENV_PENDULUM, 128>(precision, b, st);
-                case TG_ENV_QUADPOLE2D: return launch_rollout_tc2<TG_ENV_QUADPOLE2D, 128>(precision, b, st);
-                default: return launch_rollout_tc2<TG_ENV_QUADPOLE, 128>(precision, b, st);
-            }
-        }
-        switch (env->kind) {
-            case TG_ENV_CARTPOLE: return launch_rollout_tc<TG_ENV_CARTPOLE>(precision, b, st);
-            case TG_ENV_PENDULUM: return launch_rollout_tc<TG_ENV_PENDULUM>(precision, b, st);
-            case TG_ENV_QUADPOLE2D: return launch_rollout_tc<TG_ENV_QUADPOLE2D>(precision, b, st);
-            default: return launch_rollout_tc<TG_ENV_QUADPOLE>(precision, b, st);
-        }
+        return launch_rollout_tc(env->kind, precision, b, st);
     }
+    RolloutArgs<tg_mlp_layout> a;
+    memset(&a, 0, sizeof(a));
+    a.io = io;
     rc = tg_build_layout(mlp, false, &a.lay);
     if (rc) return rc;
     rc = tg_pack_weights(ctx, a.lay, params, st);
     if (rc) return rc;
-    a.N = N;
-    a.init_state = init_state;
     a.packed = ctx->packed;
-    a.noise = noise;
-    a.seed = seed;
-    a.env_offset = env_offset;
-    a.obs = out_obs; a.act = out_act; a.rew = out_rew; a.logp = out_logp; a.len = out_len; a.ret = out_ret;
     const int B = a.lay.B, NT = a.lay.NT;
     const size_t act_bytes = (2 * (size_t)a.lay.kmax * (B + 4) + (size_t)(NT / B) * TG_MAX_ACT * B) * sizeof(float);
     size_t smem = act_bytes + (size_t)a.lay.total * sizeof(float);
@@ -732,12 +482,10 @@ extern "C" int tg_rollout(tg_ctx *ctx, const tg_env_cfg *env, const tg_mlp_cfg *
     const bool wg = smem > (size_t)ctx->smem_optin;
     if (wg) smem = act_bytes;
     TG_REQUIRE(smem <= (size_t)ctx->smem_optin, TG_ERR_UNSUPPORTED, "activation tiles need %zu B of shared memory", smem);
-    switch (env->kind) {
-        case TG_ENV_CARTPOLE: return dispatch_prec<TG_ENV_CARTPOLE>(precision, a, smem, wg, st);
-        case TG_ENV_PENDULUM: return dispatch_prec<TG_ENV_PENDULUM>(precision, a, smem, wg, st);
-        case TG_ENV_QUADPOLE2D: return dispatch_prec<TG_ENV_QUADPOLE2D>(precision, a, smem, wg, st);
-        default: return dispatch_prec<TG_ENV_QUADPOLE>(precision, a, smem, wg, st);
-    }
+    return tg_with_env_kind(env->kind, [&](auto kind) {
+        return precision == TG_PREC_F64 ? dispatch_cfg<decltype(kind)::value, double>(a, smem, wg, st)
+                                        : dispatch_cfg<decltype(kind)::value, float>(a, smem, wg, st);
+    });
 }
 
 // ---------------------------------------------------------------------------
@@ -812,24 +560,14 @@ extern "C" int tg_env_step(tg_ctx *ctx, const tg_env_cfg *env, int precision, in
     TG_REQUIRE(N > 0, TG_ERR_SHAPE, "tg_env_step: N must be positive");
     TG_REQUIRE(precision == TG_PREC_F32 || precision == TG_PREC_F64, TG_ERR_ARG, "bad precision %d", precision);
     EnvParams p;
-    int rc = fill_env_params(env, &p);
+    int rc = tg_fill_env_params(env, &p);
     if (rc) return rc;
     TG_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = (cudaStream_t)stream;
-    switch (env->kind) {
-        case TG_ENV_CARTPOLE:
-            return launch_env_step<TG_ENV_CARTPOLE>(precision, p, N, state, raw_action, steps_done, bal_count,
-                                                    next_state, reward, done, bal_out, st);
-        case TG_ENV_PENDULUM:
-            return launch_env_step<TG_ENV_PENDULUM>(precision, p, N, state, raw_action, steps_done, bal_count,
-                                                    next_state, reward, done, bal_out, st);
-        case TG_ENV_QUADPOLE2D:
-            return launch_env_step<TG_ENV_QUADPOLE2D>(precision, p, N, state, raw_action, steps_done, bal_count,
+    return tg_with_env_kind(env->kind, [&](auto kind) {
+        return launch_env_step<decltype(kind)::value>(precision, p, N, state, raw_action, steps_done, bal_count,
                                                       next_state, reward, done, bal_out, st);
-        default:
-            return launch_env_step<TG_ENV_QUADPOLE>(precision, p, N, state, raw_action, steps_done, bal_count,
-                                                    next_state, reward, done, bal_out, st);
-    }
+    });
 }
 
 template <typename R>

@@ -23,8 +23,8 @@
 //     through shared memory; the part-0 thread samples the action, integrates the env, writes the rows.
 #include <math.h>
 
-#include "tg_env.cuh"
 #include "tg_mlp.cuh"
+#include "tg_rollout.cuh"
 #include "tg_umma.cuh"
 
 #define W256 256
@@ -32,20 +32,6 @@
 #define CHUNK_K 32
 #define CHUNK_FLOATS (W256 * CHUNK_K)           // 8192 floats = 32 KB
 #define N_CHUNKS (2 * W256 / CHUNK_K)           // 16: (hi, lo) x 8 K-chunks
-
-struct RolloutTc256Args {
-    EnvParams env;
-    TcwLayout lay;                               // built without the backward chunks
-    int64_t N;
-    const void *init_state;
-    const float *packed;
-    const float *noise;
-    uint64_t seed;
-    int64_t env_offset;
-    float sd[TG_MAX_ACT], log_norm;
-    float *obs, *act, *rew, *logp, *ret;
-    int32_t *len;
-};
 
 bool tg_tc256_eligible(const tg_mlp_cfg *mlp) {
     return mlp && mlp->n_layers == 3 && mlp->dims[1] == W256 && mlp->dims[2] == W256 && mlp->dims[0] >= 1 &&
@@ -58,9 +44,9 @@ bool tg_tc256_eligible(const tg_mlp_cfg *mlp) {
 #define BAR_K1 7
 
 template <int KIND, typename R, bool RELU>
-__global__ void __launch_bounds__(576, 1) rollout_tc256_kernel(const __grid_constant__ RolloutTc256Args a) {
-    using E = Env<KIND>;
-    constexpr int S = E::S, A = E::A, W = W256, HW = 64, OKP = (S + 1 + 7) / 8 * 8;
+__global__ void __launch_bounds__(576, 1) rollout_tc256_kernel(const __grid_constant__ RolloutArgs<TcwLayout> a) {
+    using Ev = RolloutEnv<KIND, R>;
+    constexpr int S = Ev::S, A = Ev::A, W = W256, HW = 64, OKP = (S + 1 + 7) / 8 * 8;
     constexpr uint32_t TM_D = 0u, TM_AHI = 256u, TM_ALO = 384u;
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     __shared__ __align__(8) uint64_t wbar, bar_d, bar_k0, full_bar[RING_STAGES], empty_bar[RING_STAGES];
@@ -94,8 +80,7 @@ __global__ void __launch_bounds__(576, 1) rollout_tc256_kernel(const __grid_cons
     tc_fence_after();
     const uint32_t tmem = tmem_slot;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int T = a.env.max_steps;
-    const int64_t N = a.N;
+    const int T = a.io.env.max_steps;
 
     if (warp == 16) {
         // ===== TMA producer: streams the 16 weight chunks of every step through the ring =====
@@ -185,33 +170,20 @@ __global__ void __launch_bounds__(576, 1) rollout_tc256_kernel(const __grid_cons
         const int c0 = part * HW;
         const uint32_t my_tm = tmem + ((uint32_t)(q * 32) << 16);
         const int64_t n = (int64_t)blockIdx.x * 128 + e;
-        const bool real_env = n < N;
-        const bool writer = real_env && part == 0;
         const int act_kind = RELU ? TG_ACT_RELU : a.lay.act;
         const float *b1 = Rsm + a.lay.b1 + c0, *wo = Rsm + a.lay.wo + c0, *bo = Rsm + a.lay.bo;
-        bool alive = writer;
-        R s[S];
-        int steps = 0, bal = 0;
-        float ret = 0.0f;
-        if (writer) {
-            const R *init = reinterpret_cast<const R *>(a.init_state);
-#pragma unroll
-            for (int i = 0; i < S; ++i) s[i] = init[(int64_t)i * N + n];
-        } else {
-#pragma unroll
-            for (int i = 0; i < S; ++i) s[i] = (R)0;
-        }
+        Ev ev(a.io, n, n < a.io.N && part == 0, true);      // only part 0 holds, steps and records the env
         uint32_t ph_d = 0, ph_k0 = 0;
         int t = 0;
         for (; t < T; ++t) {
             if (part == 0) {
+                float x[S];
+                ev.observe(a.io, t, x);
 #pragma unroll
                 for (int i = 0; i < S; ++i) {
-                    const float x = alive ? (float)s[i] : 0.0f;
-                    if (writer) a.obs[((int64_t)t * S + i) * N + n] = x;
-                    const float xh = tf32_hi(x);
+                    const float xh = tf32_hi(x[i]);
                     *reinterpret_cast<float *>(O_hi + core_offset(OKP, e, i)) = xh;
-                    *reinterpret_cast<float *>(O_lo + core_offset(OKP, e, i)) = x - xh;
+                    *reinterpret_cast<float *>(O_lo + core_offset(OKP, e, i)) = x[i] - xh;
                 }
             }
             fence_proxy_async();
@@ -286,95 +258,36 @@ __global__ void __launch_bounds__(576, 1) rollout_tc256_kernel(const __grid_cons
                 float mu[A];
 #pragma unroll
                 for (int j = 0; j < A; ++j) mu[j] = (((bo[j] + muS[0][j][e]) + muS[1][j][e]) + muS[2][j][e]) + muS[3][j][e];
-                float act[A], lp = 0.0f, rw = 0.0f;
-                if (alive) {
-                    float eps[4];
-                    if (a.noise != nullptr) {
-#pragma unroll
-                        for (int j = 0; j < A; ++j) eps[j] = a.noise[((int64_t)t * A + j) * N + n];
-                    } else {
-                        philox_normal4(a.seed, (uint64_t)(a.env_offset + n), (uint32_t)t, eps);
-                    }
-                    float m2 = 0.0f;
-#pragma unroll
-                    for (int j = 0; j < A; ++j) {
-                        act[j] = mu[j] + a.sd[j] * eps[j];
-                        const float z = (act[j] - mu[j]) / a.sd[j];
-                        m2 += z * z;
-                    }
-                    lp = -0.5f * m2 - a.log_norm;
-                    R r;
-                    const bool done = E::template step<R>(s, act, a.env, steps, bal, r);
-                    rw = (float)r;
-                    ret += rw;
-                    steps += 1;
-                    alive = !done;
-                } else {
-#pragma unroll
-                    for (int j = 0; j < A; ++j) act[j] = 0.0f;
-                }
-                if (writer) {
-#pragma unroll
-                    for (int j = 0; j < A; ++j) a.act[((int64_t)t * A + j) * N + n] = act[j];
-                    a.rew[(int64_t)t * N + n] = rw;
-                    if (a.logp) a.logp[(int64_t)t * N + n] = lp;
-                }
+                ev.act(a.io, t, mu);
             }
-            if (!__syncthreads_or(alive ? 1 : 0)) { ++t; break; }
+            if (!__syncthreads_or(ev.alive ? 1 : 0)) { ++t; break; }
         }
-        if (writer) {
-            for (; t < T; ++t) {
-#pragma unroll
-                for (int i = 0; i < S; ++i) a.obs[((int64_t)t * S + i) * N + n] = 0.0f;
-#pragma unroll
-                for (int j = 0; j < A; ++j) a.act[((int64_t)t * A + j) * N + n] = 0.0f;
-                a.rew[(int64_t)t * N + n] = 0.0f;
-                if (a.logp) a.logp[(int64_t)t * N + n] = 0.0f;
-            }
-            a.len[n] = steps;
-            if (a.ret) a.ret[n] = ret;
-        }
+        ev.finish(a.io, t);
     }
     tc_fence_before();
     __syncthreads();
     if (threadIdx.x < 32) tmem_dealloc(tmem, 512);
 }
 
-template <int KIND>
-static int launch_tc256(int precision, const RolloutTc256Args &a, size_t smem, cudaStream_t st) {
-    void (*kern)(const RolloutTc256Args);
-    const bool relu = a.lay.act == TG_ACT_RELU;
-    if (precision == TG_PREC_F64) kern = relu ? rollout_tc256_kernel<KIND, double, true> : rollout_tc256_kernel<KIND, double, false>;
-    else kern = relu ? rollout_tc256_kernel<KIND, float, true> : rollout_tc256_kernel<KIND, float, false>;
-    TG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const unsigned grid = (unsigned)((a.N + 127) / 128);
-    kern<<<grid, 576, smem, st>>>(a);
-    TG_CUDA(cudaGetLastError());
-    return TG_OK;
-}
-
-// Called by tg_rollout (tg_rollout.cu) for eligible 256-wide policies.
-int tg_rollout_tc256(tg_ctx *ctx, const tg_env_cfg *env, const EnvParams &ep, const tg_mlp_cfg *mlp, int precision,
-                     int64_t N, const void *init_state, const float *params, const float *sd, float log_norm,
-                     const float *noise, uint64_t seed, int64_t env_offset, float *out_obs, float *out_act, float *out_rew,
-                     float *out_logp, int32_t *out_len, float *out_ret, cudaStream_t st) {
-    RolloutTc256Args a;
+// Called by tg_rollout (tg_rollout.cu) for eligible 256-wide policies; io.init_state is `precision`.
+int tg_rollout_tc256(tg_ctx *ctx, const tg_mlp_cfg *mlp, int precision, int kind, const float *params, const RolloutIo &io,
+                     cudaStream_t st) {
+    RolloutArgs<TcwLayout> a;
     memset(&a, 0, sizeof(a));
-    a.env = ep;
-    tg_build_tcw_layout(mlp, &a.lay, false);
+    a.io = io;
+    tg_build_tcw_layout(mlp, &a.lay, false);      // without the backward chunks
     int rc = tg_pack_weights_tcw(ctx, a.lay, params, st);
     if (rc) return rc;
-    a.N = N; a.init_state = init_state; a.packed = ctx->packed_tc; a.noise = noise; a.seed = seed;
-    a.env_offset = env_offset;
-    memcpy(a.sd, sd, sizeof(a.sd));
-    a.log_norm = log_norm;
-    a.obs = out_obs; a.act = out_act; a.rew = out_rew; a.logp = out_logp; a.len = out_len; a.ret = out_ret;
+    a.packed = ctx->packed_tc;
     const size_t smem = (size_t)RING_STAGES * CHUNK_FLOATS * 4 + (size_t)a.lay.resident * 4 + 2 * (size_t)128 * a.lay.OKP * 4;
     TG_REQUIRE(smem + 12 * 1024 <= (size_t)ctx->smem_optin, TG_ERR_UNSUPPORTED, "tc256 rollout needs %zu B of shared memory", smem);
-    switch (env->kind) {
-        case TG_ENV_CARTPOLE: return launch_tc256<TG_ENV_CARTPOLE>(precision, a, smem, st);
-        case TG_ENV_PENDULUM: return launch_tc256<TG_ENV_PENDULUM>(precision, a, smem, st);
-        case TG_ENV_QUADPOLE2D: return launch_tc256<TG_ENV_QUADPOLE2D>(precision, a, smem, st);
-        default: return launch_tc256<TG_ENV_QUADPOLE>(precision, a, smem, st);
-    }
+    auto kern = tg_with_env_kind(kind, [&](auto k) {
+        return tg_with_prec_relu(precision, a.lay.act, [](auto r, auto relu) {
+            return rollout_tc256_kernel<decltype(k)::value, decltype(r), decltype(relu)::value>;
+        });
+    });
+    TG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<(unsigned)((io.N + 127) / 128), 576, smem, st>>>(a);
+    TG_CUDA(cudaGetLastError());
+    return TG_OK;
 }
